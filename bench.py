@@ -9,7 +9,9 @@ Workload (BASELINE.json configs[4], the configuration the multi-GPU metric is qu
 
   python bench.py --gpus N --steps K --warmup W          (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                   (the CPU restatement of the reference algorithm)
+  python bench.py ... --dump-outputs DIR                 (writes the image of the last timed step to DIR/image.npy)
 
+Writes nothing into the source tree: the synthetic scene assets are generated into a temporary directory.
 Prints ONE JSON line (rank 0).  `value` is device-timed with the scene resident in HBM; `e2e` goes through
 the C ABI with host buffers (scene upload H2D + image D2H inside the timed region).  At N = 1 the line also carries
 `configs`: BASELINE configs 1-4 (primitive / new-cbox / brdf / welcome-2018 at 144 k and 1 M triangles) measured in the
@@ -25,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                         # the source tree may be read-only; leave no __pycache__ in it
 
 WIDTH, HEIGHT = 1920, 1370
 SPP_TOTAL = 1024                                       # BASELINE.md §4 config 5: 256 / 1024 / 4096
@@ -124,13 +127,13 @@ def reference_traversal(st):
     return {"nodes_per_ray": nodes, "prims_per_ray": prims, "bytes_per_ray": 36.0 * nodes + 36.0 * prims}
 
 
-def run_reference(args):
+def run_reference(args, asset_root):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     import lumillyrender_b200 as lr
-    lr.ensure_assets(ROOT, bunny_tris=BUNNY_TRIS, need_ibl=False)
-    d = lr.Description(os.path.join(ROOT, "scenes", SCENE + ".toml"), asset_root=ROOT, resolution=(WIDTH, HEIGHT))
+    lr.ensure_assets(asset_root, bunny_tris=BUNNY_TRIS, need_ibl=False)
+    d = lr.Description(os.path.join(ROOT, "scenes", SCENE + ".toml"), asset_root=asset_root, resolution=(WIDTH, HEIGHT))
     from lumillyrender_b200.renderer import params_from_config
 
     def params_fn(spp):
@@ -196,22 +199,20 @@ def kernel_name(d):
     return "%s<%s, %s>" % ("render_pool_kernel" if pool else "render_persistent_kernel", integ, "tree" if tree else "flat")
 
 
-def run_configs(lr, torch, l2_peak, hbm_peak):
+def run_configs(lr, torch, l2_peak, hbm_peak, asset_root):
     """BASELINE configs 1-4 in the same run: device-timed render at the scene's own film size and spp (CUDA events on the
     launching stream, 3 repeats after a warm-up, L2 flushed between them), the byte model from one instrumented launch,
     and the CPU restatement on a bounded sample (~4 s) beside it."""
     from lumillyrender_b200.renderer import params_from_config
     out = []
-    roots = {0: ROOT, BUNNY_TRIS: ROOT}
+    roots = {0: asset_root, BUNNY_TRIS: asset_root}
     stream = torch.cuda.current_stream().cuda_stream
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-    tmp = None
     for label, name, (w, h), spp, tris in CONFIGS:
         if tris not in roots:
-            tmp = tmp or tempfile.mkdtemp(prefix="lumilly_bench_")
-            roots[tris] = lr.ensure_assets(os.path.join(tmp, "m%d" % tris), bunny_tris=tris, ibl_height=1600)
+            roots[tris] = lr.ensure_assets(os.path.join(asset_root, "m%d" % tris), bunny_tris=tris, ibl_height=1600)
         elif tris == BUNNY_TRIS:
-            lr.ensure_assets(ROOT, bunny_tris=BUNNY_TRIS, ibl_height=1600)
+            lr.ensure_assets(asset_root, bunny_tris=BUNNY_TRIS, ibl_height=1600)
         t0 = time.perf_counter()
         d = lr.Description(os.path.join(ROOT, "scenes", name + ".toml"), asset_root=roots[tris], resolution=(w, h))
         load_s = time.perf_counter() - t0
@@ -283,9 +284,6 @@ def run_configs(lr, torch, l2_peak, hbm_peak):
         s.close()
         d.close()
         del accum
-    if tmp:
-        import shutil
-        shutil.rmtree(tmp, ignore_errors=True)
     return out
 
 
@@ -297,11 +295,21 @@ def main():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the mean image of the last timed step (HxWx3 float32) to DIR/image.npy, for comparing builds")
     args = ap.parse_args()
-    if args.impl == "reference":
-        return run_reference(args)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU implementation only")
+    with tempfile.TemporaryDirectory(prefix="lumilly_bench_") as asset_root:
+        if args.impl == "reference":
+            return run_reference(args, asset_root)
+        run_b200(args, asset_root)
 
-    import numpy as np  # noqa: F401
+
+def run_b200(args, asset_root):
+    import numpy as np
     import torch
     import lumillyrender_b200 as lr
     from lumillyrender_b200.distributed import env_rank_world, render_sharded
@@ -317,12 +325,9 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     lr.init(local_rank)
-    if rank == 0:
-        lr.ensure_assets(ROOT, bunny_tris=BUNNY_TRIS, need_ibl=False)
-    if world > 1:
-        dist.barrier()
+    lr.ensure_assets(asset_root, bunny_tris=BUNNY_TRIS, need_ibl=False)     # every rank its own (deterministic) copy
     t0 = time.perf_counter()
-    d = lr.Description(os.path.join(ROOT, "scenes", SCENE + ".toml"), asset_root=ROOT, resolution=(WIDTH, HEIGHT))
+    d = lr.Description(os.path.join(ROOT, "scenes", SCENE + ".toml"), asset_root=asset_root, resolution=(WIDTH, HEIGHT))
     load_s = time.perf_counter() - t0
     s = d.scene()
     stream = torch.cuda.current_stream().cuda_stream
@@ -368,6 +373,10 @@ def main():
     total_s = float(total_ms.item()) * 1e-3
     rays, samples, launches = [float(x) for x in counts.tolist()]
     image_mean = float(accum.mean().item()) if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        # the last timed step's result as its caller receives it: the reduced, normalised image (seed 1000 + warmup + steps - 1)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "image.npy"), accum.cpu().numpy())
 
     # ---- e2e through the C ABI with host buffers: scene upload (H2D) + render + image download (D2H) per step
     host_img = torch.empty((HEIGHT, WIDTH, 3), dtype=torch.float32).pin_memory()
@@ -376,7 +385,7 @@ def main():
     import ctypes as C
     from lumillyrender_b200 import capi
     lib = capi.load_library()
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
     for i in range(1 + e2e_steps):
         barrier()
         t0 = time.perf_counter()
@@ -478,7 +487,7 @@ def main():
         if world == 1 and not args.no_configs:
             del accum, flush
             s.close()
-            line["configs"] = run_configs(lr, torch, l2_peak, hbm_peak)
+            line["configs"] = run_configs(lr, torch, l2_peak, hbm_peak, asset_root)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
