@@ -40,15 +40,52 @@ LR_DEV F3 operator-(F3 a, F3 b) { return f3(a.x - b.x, a.y - b.y, a.z - b.z); }
 LR_DEV F3 operator*(F3 a, float s) { return f3(a.x * s, a.y * s, a.z * s); }
 LR_DEV F3 operator*(float s, F3 a) { return f3(s * a.x, s * a.y, s * a.z); }
 LR_DEV F3 operator*(F3 a, F3 b) { return f3(a.x * b.x, a.y * b.y, a.z * b.z); }
-// IEEE quotient of a vector by a scalar.  In the one-path-per-lane kernel for pt-direct over a BVH the three divisions live in ONE
-// out-of-line function (LR_DIV_OUT_OF_LINE, set by build.py for that translation unit): ~20 inlined copies of 3 x 14 instructions
-// are a fifth of the kernel's code, and the kernel is instruction-fetch bound (A/B, profiles/r01_c_ab_s22.txt: +4.6 % on
-// sample.toml; the flat-only kernels are 3 % faster with the divisions inlined).
+// ------------------------------------------------------------------ exact quotients that avoid the general division
+// Under -prec-div=true every a / b is MUFU.RCP, five FFMA and an FCHK whose check sends the quotient to an out-of-line slow
+// path (__cuda_sm3x_div_rn_noftz_f32_slowpath) when an operand is outside the range the fast sequence handles.  A zero
+// dividend is outside that range (tools/div_probe.py on a B200: 242 cycles against 48 for a normal quotient,
+// profiles/r03_a_div_probe.txt), and the hot path divides zeros on every bounce: the ONB's cross(a, n) has one component
+// that is exactly +-0, two on an axis-aligned wall.  The helpers below give the IEEE
+// quotient bit for bit (tests/test_exact_quotients.py checks them exhaustively) without that slow path.
+//
+// div_zero_dividend: 0 / s for a nonzero, non-NaN s is by IEEE definition a zero whose sign is the XOR of the operands'
+// signs; the divide is handed a harmless dividend (s / s) in that case and its result is discarded.  Every other
+// combination (0 / 0, 0 / NaN, any nonzero dividend) is the real division.
+LR_DEV float div_zero_dividend(float a, float s) {
+  const bool z = a == 0.0f && fabsf(s) > 0.0f;
+  const float q = (z ? s : a) / s;
+  return z ? __uint_as_float((__float_as_uint(a) ^ __float_as_uint(s)) & 0x80000000u) : q;
+}
+// a / kPI correctly rounded in three operations (Markstein: y = RN(1 / b) and q0 = RN(a * y) within one ulp of a / b make
+// the residual r = a - b * q0 exact and RN(q0 + r * y) the correctly rounded quotient), for |a| >= 2^-95, where no step
+// underflows (exhaustively: the sequence is exact for every dividend with a biased exponent of 23 or more, inf / NaN
+// excepted).  A zero dividend gives a zero of its own sign; NaN, inf and tiny dividends take the real division, out of
+// line (the render never reaches it).
+constexpr float kPI_RCP = 0x1.45f306p-2f;                          // RN(1 / kPI)
+LR_COLD float div_cold(float a, float b) { return a / b; }
+LR_DEV float div_pi(float a) {
+  const unsigned e = (__float_as_uint(a) >> 23) & 0xffu;
+  if (e - 32u <= 254u - 32u) {
+    const float q0 = __fmul_rn(a, kPI_RCP);
+    const float r = __fmaf_rn(-kPI, q0, a);
+    return __fmaf_rn(r, kPI_RCP, q0);
+  }
+  return a == 0.0f ? a : div_cold(a, kPI);
+}
+
+// IEEE quotient of a vector by a scalar, each component through div_zero_dividend: zero components are common (the ONB's
+// cross product, axis-aligned normals and directions, black colour channels), and the guard is cheaper than the slow path
+// they would take (A/B, profiles/r03_a_ab.txt: sample.toml 36.4 -> 31.8 ms, welcome-2018 43.2 -> 40.9 ms; with the guard
+// in orthonormal_basis only, 32.6 / 44.4 ms).  In the one-path-per-lane kernel for pt-direct over a BVH the three
+// divisions live in ONE out-of-line function (LR_DIV_OUT_OF_LINE, set by build.py for that translation unit): ~20 inlined
+// copies of 3 x 14 instructions are a fifth of the kernel's code, and the kernel is instruction-fetch bound (A/B,
+// profiles/r01_c_ab_s22.txt: +4.6 % on sample.toml; the flat-only kernels are 3 % faster with the divisions inlined).
+LR_DEV F3 div3_inline(F3 a, float s) { return f3(div_zero_dividend(a.x, s), div_zero_dividend(a.y, s), div_zero_dividend(a.z, s)); }
 #ifdef LR_DIV_OUT_OF_LINE
-static __device__ __noinline__ F3 div3_call(F3 a, float s) { F3 r; r.x = a.x / s; r.y = a.y / s; r.z = a.z / s; return r; }
+static __device__ __noinline__ F3 div3_call(F3 a, float s) { return div3_inline(a, s); }
 LR_DEV F3 operator/(F3 a, float s) { return div3_call(a, s); }
 #else
-LR_DEV F3 operator/(F3 a, float s) { return f3(a.x / s, a.y / s, a.z / s); }
+LR_DEV F3 operator/(F3 a, float s) { return div3_inline(a, s); }
 #endif
 LR_DEV float dot(F3 a, F3 b) { return a.x * b.x + a.y * b.y + a.z * b.z; }
 LR_DEV F3 cross(F3 a, F3 b) { return f3(a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x); }
@@ -504,7 +541,7 @@ LR_DEV Surface surface_at(const DevScene& sc, F3 o, F3 d, float t, int id) {
 // ------------------------------------------------------------------ sampling utilities (util.rs)
 LR_DEV void orthonormal_basis(F3 n, F3& tangent, F3& binormal) {   // util.rs:12-21
   const F3 a = fabsf(n.x) > kEPS ? f3(0.0f, 1.0f, 0.0f) : f3(1.0f, 0.0f, 0.0f);
-  tangent = normalize(cross(a, n));
+  tangent = normalize(cross(a, n));                                // one component is +-0 whatever n is
   binormal = cross(n, tangent);
 }
 LR_DEV F3 reflect(F3 v, F3 normal) { return -v + normal * (dot(v, normal) * 2.0f); }   // util.rs:30-32
@@ -537,29 +574,33 @@ LR_DEV Mat load_mat(const DevScene& sc, int i) {
   return m;
 }
 
-// fmodf(x, m) for x >= 0 and a positive module m (the checker's 30 / 150 / 300), exactly: q = trunc(fl(x / m)) is the
-// true integer quotient or one above it (an IEEE quotient never rounds below an integer that the true quotient
-// reaches), so r = x - q*m, computed without rounding by one FMA, is the remainder or the remainder minus m, and
-// both that value and the corrected one are multiples of ulp(m) below 2^24 ulps, i.e. exactly representable.
-// Checked against fmod over random and adversarial inputs in tests/test_host_frontend.py (same IEEE operations).
+// fmodf(x, m) for x >= 0 and a positive module m (the checker's 30 / 150 / 300), exactly and without a division, given
+// m_rcp = RN(1 / m): q0 = trunc(RN(x * m_rcp)) is the integer quotient floor(x / m) or one off IN EITHER DIRECTION (the
+// product carries two roundings of at most half an ulp each, so it can land just below an integer the true quotient
+// reaches as well as just above it), r0 = x - q0*m by one FMA tells which (rounding is monotonic, so r0 < 0 and
+// r0 >= m are decided as for the exact value), and x - q*m with the corrected q is the remainder itself, exactly
+// representable (fmod is exact), so the last FMA does not round.  Beyond a quotient of 2^23 (and for NaN / inf) the
+// library routine.  Checked against fmod for every float32 x in tests/test_exact_quotients.py.
 LR_COLD float fmodf_cold(float x, float m) { return fmodf(x, m); }
-LR_DEV float fmod_pos(float x, float m) {
+LR_DEV float fmod_pos(float x, float m, float m_rcp) {
   if (!(x < m * 8388608.0f)) return fmodf_cold(x, m);                   // quotient beyond 2^23: the library routine (also NaN / inf)
-  const float q = truncf(x / m);
-  const float r = __fmaf_rn(-q, m, x);
-  return r < 0.0f ? r + m : r;
+  const float q0 = truncf(__fmul_rn(x, m_rcp));
+  const float r0 = __fmaf_rn(-q0, m, x);
+  const float q = r0 < 0.0f ? q0 - 1.0f : (r0 >= m ? q0 + 1.0f : q0);
+  return __fmaf_rn(-q, m, x);
 }
-LR_DEV float signed_mod(float base, float module) {                // lambert.rs:58-64  (base % module on |base|)
-  const float r = fmod_pos(fabsf(base), module);
+LR_DEV float signed_mod(float base, float module, float module_rcp) {   // lambert.rs:58-64  (base % module on |base|)
+  const float r = fmod_pos(fabsf(base), module, module_rcp);
   return base > 0.0f ? r : module - r;
 }
 LR_DEV float checker(float u, float v) {                           // lambert.rs:66-90 (grey value)
   const float lw = 2.0f, li = 150.0f, sw = 1.0f, si = 30.0f, cw = 150.0f, ci = 300.0f;
-  const float lu = signed_mod(u, li), lv = signed_mod(v, li);
+  const float li_rcp = 0x1.b4e81cp-8f, si_rcp = 0x1.111112p-5f, ci_rcp = 0x1.b4e81cp-9f;   // RN(1 / 150), RN(1 / 30), RN(1 / 300)
+  const float lu = signed_mod(u, li, li_rcp), lv = signed_mod(v, li, li_rcp);
   if (lu < lw || lv < lw) return 0.5f;
-  const float su = signed_mod(u, si), sv = signed_mod(v, si);
+  const float su = signed_mod(u, si, si_rcp), sv = signed_mod(v, si, si_rcp);
   if (su < sw || sv < sw) return 0.6f;
-  const float cu = signed_mod(u, ci), cv = signed_mod(v, ci);
+  const float cu = signed_mod(u, ci, ci_rcp), cv = signed_mod(v, ci, ci_rcp);
   if ((cu < cw || cv < cw) && !(cu < cw && cv < cw)) return 0.8f;
   return 1.0f;
 }
@@ -661,7 +702,8 @@ LR_GGX void ggx_sample(float roughness, F3 out_, F3 on, float xi2, float s1, flo
 LR_DEV F3 mat_brdf(const Mat& m, F3 out_, F3 in_, F3 n, F3 pos) {
   if (m.type == LR_MAT_LAMBERT) {                                  // lambert.rs:32-35
     const float c = checker(pos.x, pos.z);
-    return m.color * f3(c, c, c) / kPI;
+    const F3 cc = m.color * f3(c, c, c);
+    return f3(div_pi(cc.x), div_pi(cc.y), div_pi(cc.z));          // cc / kPI, exactly
   }
   if (m.type == LR_MAT_GGX) return ggx_brdf(m.color, m.param0, m.param1, out_, in_, n);
   return mat_brdf_other(m.type, m.color, m.param0, m.param1, out_, in_, n);
@@ -723,7 +765,7 @@ LR_DEV void mat_sample(const Mat& m, F3 out_, F3 n, Pcg& rng, F3& in_, float& pd
     const float r2s = sqrtf(xi2);
     const F3 s = f3(c1 * r2s, s1 * r2s, sqrtf(1.0f - xi2));
     in_ = u * s.x + v * s.y + on * s.z;
-    pdf = dot(in_, n) / kPI;
+    pdf = div_pi(dot(in_, n));                                     // dot(in_, n) / kPI, exactly
     return;
   }
   if (m.type == LR_MAT_GGX) {
