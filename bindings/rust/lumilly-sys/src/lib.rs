@@ -39,6 +39,7 @@ pub enum LrScene {}
 pub enum LrHostScene {}
 pub enum LrFilm {}
 pub enum LrMultiScene {}
+pub enum LrMultiFilm {}
 pub const LR_AOV_NORMAL: i32 = 0;
 pub const LR_AOV_DEPTH: i32 = 1;
 pub const LR_BVH_HOST: i32 = 0;
@@ -75,6 +76,13 @@ extern "C" {
     pub fn lr_film_save(film: *const LrFilm, path: *const c_char) -> c_int;
     pub fn lr_film_load(scene: *const LrScene, path: *const c_char, out: *mut *mut LrFilm) -> c_int;
     pub fn lr_film_destroy(film: *mut LrFilm);
+    pub fn lr_multi_film_create(ms: *mut LrMultiScene, params: *const LrRenderParams, want_sumsq: i32, out: *mut *mut LrMultiFilm) -> c_int;
+    pub fn lr_multi_film_render(film: *mut LrMultiFilm, spp_count: i32, stats: *mut LrStats) -> c_int;
+    pub fn lr_multi_film_info(film: *const LrMultiFilm, spp_done: *mut i32, crop_w: *mut i32, crop_h: *mut i32, has_sumsq: *mut i32) -> c_int;
+    pub fn lr_multi_film_read(film: *const LrMultiFilm, out_rgb: *mut f32, out_sumsq: *mut f32) -> c_int;
+    pub fn lr_multi_film_save(film: *const LrMultiFilm, path: *const c_char) -> c_int;
+    pub fn lr_multi_film_load(ms: *mut LrMultiScene, path: *const c_char, out: *mut *mut LrMultiFilm) -> c_int;
+    pub fn lr_multi_film_destroy(film: *mut LrMultiFilm);
     pub fn lr_trace_primary(scene: *const LrScene, u: f32, v: f32, ua: f32, va: f32, prim: *mut i32, t: *mut f32) -> c_int;
     pub fn lr_trace_rays(scene: *const LrScene, n: i64, origins: *const f32, directions: *const f32, prim: *mut i32, t: *mut f32, normal: *mut f32) -> c_int;
     pub fn lr_trace_rays_query(scene: *const LrScene, n: i64, origins: *const f32, directions: *const f32, query: i32, prim: *mut i32, t: *mut f32,

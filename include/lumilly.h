@@ -258,6 +258,27 @@ int lr_film_save(const LrFilm* film, const char* path);
 int lr_film_load(const LrScene* scene, const char* path, LrFilm** out);
 void lr_film_destroy(LrFilm* film);
 
+/* ---- the same film on the devices of an LrMultiScene.  The crop's 8x4 pixel tiles are dealt round-robin: shard k of
+ * n_devices owns the tiles t with t % n_devices == k and renders on devices[k].  Every pixel's samples are still added in
+ * sample order on one device, starting from the stored sum, so the image, the sums of squares and the ray count equal
+ * those of one lr_render with splits = 1, bit for bit, for ANY device count (lr_multi_render, which shards by sample
+ * index, cannot promise that).  lr_multi_film_render launches every device at once, each on its own stream, and returns
+ * when all are done (stats: totals, kernel_ms the slowest device's).  read / save gather the image on devices[0], each
+ * pixel from the device that owns it (peer reads over NVLink, staged copies where a peer cannot be mapped).
+ * params->splits must be 0 or 1 (it is always 1).  save writes the checkpoint format of lr_film_save, byte for byte
+ * what lr_film_save writes for the same state; lr_film_load resumes it on one device, and lr_multi_film_load resumes a
+ * checkpoint of either kind on any LrMultiScene (its header must say splits = 1).  Destroy the films of an LrMultiScene
+ * before the LrMultiScene.  Not re-entrant, like lr_multi_render: the calls switch the calling thread's CUDA device
+ * (restored on return) and the library's current device.                                                           */
+typedef struct LrMultiFilm LrMultiFilm;
+int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* params, int32_t want_sumsq, LrMultiFilm** out);
+int lr_multi_film_render(LrMultiFilm* film, int32_t spp_count, LrStats* stats /* nullable */);
+int lr_multi_film_info(const LrMultiFilm* film, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq);   /* each nullable */
+int lr_multi_film_read(const LrMultiFilm* film, float* out_rgb /* mean so far */, float* out_sumsq /* nullable */);
+int lr_multi_film_save(const LrMultiFilm* film, const char* path);
+int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out);
+void lr_multi_film_destroy(LrMultiFilm* film);
+
 /* ---- parity probe: nearest hit of the primary ray through every film pixel with the
  * sensor jitter fixed to (u,v) and the aperture sample fixed to (ua,va).
  * prim[i] = primitive id or -1, t[i] = Intersection.distance (bvh.rs:131-141).      */

@@ -5,7 +5,7 @@ The product is the C-ABI shared library (include/lumilly.h, built from csrc/ by 
 the thin host-side mirror used by the tests, bench.py and the CLI wrapper.  No CPU fallback exists.
 """
 from .capi import LumillyError, library_path, load_library  # noqa: F401
-from .renderer import (Description, Film, MultiScene, Scene, device_info, init, load_hdr, measure_hbm_read_gbs,  # noqa: F401
+from .renderer import (Description, Film, MultiFilm, MultiScene, Scene, device_info, init, load_hdr, measure_hbm_read_gbs,  # noqa: F401
                        measure_l2_read_gbs, save_hdr, save_png)
 from .assets import ensure_assets  # noqa: F401
 

@@ -112,6 +112,13 @@ SIGNATURES = {
     "lr_multi_scene_create": (C.c_int, [C.POINTER(LrSceneDesc), i32, _PI, C.POINTER(_VP)]),
     "lr_multi_render": (C.c_int, [_VP, C.POINTER(LrRenderParams), _PF, _PF, C.POINTER(LrStats)]),
     "lr_multi_scene_destroy": (None, [_VP]),
+    "lr_multi_film_create": (C.c_int, [_VP, C.POINTER(LrRenderParams), i32, C.POINTER(_VP)]),
+    "lr_multi_film_render": (C.c_int, [_VP, i32, C.POINTER(LrStats)]),
+    "lr_multi_film_info": (C.c_int, [_VP, _PI, _PI, _PI, _PI]),
+    "lr_multi_film_read": (C.c_int, [_VP, _PF, _PF]),
+    "lr_multi_film_save": (C.c_int, [_VP, C.c_char_p]),
+    "lr_multi_film_load": (C.c_int, [_VP, C.c_char_p, C.POINTER(_VP)]),
+    "lr_multi_film_destroy": (None, [_VP]),
     "lr_trace_primary": (C.c_int, [_VP, f32, f32, f32, f32, _PI, _PF]),
     "lr_trace_rays": (C.c_int, [_VP, i64, _PF, _PF, _PI, _PF, _PF]),
     "lr_trace_rays_query": (C.c_int, [_VP, i64, _PF, _PF, i32, _PI, _PF, _PF]),

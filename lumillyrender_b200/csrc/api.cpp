@@ -344,7 +344,11 @@ int lr_scene_bytes(const LrScene* s, uint64_t* h2d_bytes) {
   return LR_OK;
 }
 
-static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& dp) {
+// One part of a pixel-sharded film (lr_multi_film_*): shard `index` of `count` (device_scene.h: shard_of_tile).  Such a
+// render always runs one thread per pixel, adding its samples in order (splits = 1), whatever LR_SPLITS says.
+struct FilmShard { int index, count; };
+
+static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& dp, const FilmShard* shard = nullptr) {
   if (!s || !p) return fail(LR_ERR_INVALID, "null argument");
   if (p->integrator != LR_INTEGRATOR_PT && p->integrator != LR_INTEGRATOR_PT_DIRECT)
     return fail(LR_ERR_INVALID, "Unknown integrator type");            // main.rs:124
@@ -362,8 +366,8 @@ static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& 
     dp.crop_x = 0; dp.crop_y = 0; dp.crop_w = s->width; dp.crop_h = s->height;
   }
   dp.tiles_x = (dp.crop_w + 7) / 8; dp.tiles_y = (dp.crop_h + 3) / 4;
-  int splits = p->splits;
-  if (const char* e_splits = std::getenv("LR_SPLITS")) splits = std::atoi(e_splits);   // development knob
+  int splits = shard ? 1 : p->splits;
+  if (const char* e_splits = std::getenv("LR_SPLITS"); e_splits && !shard) splits = std::atoi(e_splits);   // development knob
   if (splits <= 0) {
     // auto: enough threads for ~2 full waves of 148 SMs x 2048 resident threads, >= 4 samples per thread
     const long long px_threads = (long long)dp.tiles_x * dp.tiles_y * 32;
@@ -375,6 +379,9 @@ static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& 
   const size_t px = (size_t)dp.crop_w * dp.crop_h;
   while (splits > 1 && px * 3 * sizeof(float) * splits > (1ull << 30)) splits--;
   dp.splits = splits;
+  dp.shard = shard ? shard->index : 0;
+  dp.n_shards = shard ? shard->count : 1;
+  dp.unit_tiles = shard_tile_count(dp.tiles_x * dp.tiles_y, dp.shard, dp.n_shards);
   // kernel organisation knobs (development / profiling only; defaults are the measured best, DESIGN.md §4)
   const char* e_di = std::getenv("LR_DEFER_ITERS");
   const char* e_dt = std::getenv("LR_DEFER_THRESH");
@@ -396,11 +403,23 @@ static int ensure_scratch(float** buf, size_t* have, size_t need) {
   return LR_OK;
 }
 
-int lr_render_accumulate_device(const LrScene* s, const LrRenderParams* p, float* d_sum, float* d_sumsq, void* cuda_stream) {
+// pixels of the crop inside the shard's tiles (the tiles on the right and bottom edges may be partly outside the crop)
+static uint64_t shard_pixels(const DevParams& dp) {
+  if (dp.n_shards == 1) return (uint64_t)dp.crop_w * dp.crop_h;
+  uint64_t n = 0;
+  for (int j = 0; j < dp.unit_tiles; j++) {
+    const int t = shard_tile(j, dp.shard, dp.n_shards), tx = t % dp.tiles_x, ty = t / dp.tiles_x;
+    n += (uint64_t)std::min(8, dp.crop_w - 8 * tx) * (uint64_t)std::min(4, dp.crop_h - 4 * ty);
+  }
+  return n;
+}
+
+// lr_render_accumulate_device for the whole crop (shard = nullptr) or for one shard of its tiles (lr_multi_film_render)
+static int accumulate(const LrScene* s, const LrRenderParams* p, float* d_sum, float* d_sumsq, void* cuda_stream, const FilmShard* shard) {
   if (!s) return fail(LR_ERR_INVALID, "null argument");
   const OnDevice on(s->device);
   DevParams dp;
-  if (int rc = resolve_params(s, p, dp)) return rc;
+  if (int rc = resolve_params(s, p, dp, shard)) return rc;
   if (!d_sum) return fail(LR_ERR_INVALID, "d_sum is null");
   if (int rc = ensure_device()) return rc;
   cudaStream_t st = (cudaStream_t)cuda_stream;
@@ -413,6 +432,7 @@ int lr_render_accumulate_device(const LrScene* s, const LrRenderParams* p, float
     if (cudaEventSynchronize(s->ev1) == cudaSuccess && cudaEventElapsedTime(&ms, s->ev0, s->ev1) == cudaSuccess) s->acc_kernel_ms += ms;
     s->ev_pending = false;
   }
+  if (dp.unit_tiles == 0) return LR_OK;                   // a shard without tiles (a crop smaller than the shard count)
   if (dp.splits > 1) {
     if (int rc = ensure_scratch(&s->d_partial, &s->partial_floats, n * dp.splits)) return rc;
     ksum = s->d_partial;
@@ -437,9 +457,13 @@ int lr_render_accumulate_device(const LrScene* s, const LrRenderParams* p, float
   }
   LR_CUDA(cudaEventRecord(s->ev1, st));
   s->ev_pending = true;
-  s->acc_samples += (uint64_t)dp.crop_w * dp.crop_h * (uint64_t)dp.spp_count;
+  s->acc_samples += shard_pixels(dp) * (uint64_t)dp.spp_count;
   s->last_splits = dp.splits;
   return LR_OK;
+}
+
+int lr_render_accumulate_device(const LrScene* s, const LrRenderParams* p, float* d_sum, float* d_sumsq, void* cuda_stream) {
+  return accumulate(s, p, d_sum, d_sumsq, cuda_stream, nullptr);
 }
 
 int lr_stats_fetch(const LrScene* s, void* cuda_stream, LrStats* stats) {
@@ -647,6 +671,16 @@ int multi_create(const LrSceneDesc* desc, int32_t n_devices, const int32_t* devi
   return LR_OK;
 }
 
+// statistics of several devices: totals, the slowest device's kernel time
+void add_device_stats(LrStats& total, const LrStats& st) {
+  total.rays += st.rays; total.samples += st.samples; total.nodes_visited += st.nodes_visited; total.tris_tested += st.tris_tested;
+  total.spheres_tested += st.spheres_tested; total.nonfinite_samples += st.nonfinite_samples; total.gate_retraces += st.gate_retraces;
+  total.flat_tris_tested += st.flat_tris_tested; total.flat_boxes_tested += st.flat_boxes_tested;
+  total.kernel_ms = std::max(total.kernel_ms, st.kernel_ms);
+  total.launches += st.launches;
+  total.splits = std::max(total.splits, st.splits);
+}
+
 int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float* out_sumsq, LrStats* stats) {
   if (!m || !p || !out_rgb) return fail(LR_ERR_INVALID, "null argument");
   if (p->spp_count <= 0 || p->spp_begin < 0) return fail(LR_ERR_INVALID, "spp range must be non-empty and non-negative");
@@ -736,12 +770,7 @@ int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float
       g_device = m->devices[i];
       LrStats st;
       if ((rc = lr_stats_fetch(m->scenes[i], m->streams[i], &st)) != LR_OK) break;
-      total.rays += st.rays; total.samples += st.samples; total.nodes_visited += st.nodes_visited; total.tris_tested += st.tris_tested;
-      total.spheres_tested += st.spheres_tested; total.nonfinite_samples += st.nonfinite_samples; total.gate_retraces += st.gate_retraces;
-      total.flat_tris_tested += st.flat_tris_tested; total.flat_boxes_tested += st.flat_boxes_tested;
-      total.kernel_ms = std::max(total.kernel_ms, st.kernel_ms);
-      total.launches += st.launches;
-      total.splits = std::max(total.splits, st.splits);
+      add_device_stats(total, st);
     }
     total.launches += out_sumsq ? 2 : 1;
   } while (0);
@@ -866,6 +895,57 @@ struct FilmHeader {                      // checkpoint file: this header, then c
   uint64_t seed;
 };
 
+// The checkpoint format, shared by LrFilm and LrMultiFilm: a film of either kind saves the same bytes for the same state
+// and loads the other's checkpoints.
+FilmHeader film_header(int film_w, int film_h, const LrRenderParams& p, int32_t crop_w, int32_t crop_h, int32_t spp_done, bool has_sumsq) {
+  FilmHeader h;
+  std::memset(&h, 0, sizeof(h));
+  std::memcpy(h.magic, kFilmMagic, 8);
+  h.film_w = film_w; h.film_h = film_h;
+  h.crop_x = p.crop_w > 0 ? p.crop_x : 0; h.crop_y = p.crop_w > 0 ? p.crop_y : 0; h.crop_w = crop_w; h.crop_h = crop_h;
+  h.integrator = p.integrator; h.depth = p.depth; h.depth_limit = p.depth_limit; h.no_direct_emitter = p.no_direct_emitter;
+  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = spp_done; h.has_sumsq = has_sumsq ? 1 : 0; h.seed = p.seed;
+  return h;
+}
+
+// `data`: the raw sums, then the sums of squares if the header says so
+int film_write(const char* path, const FilmHeader& h, const std::vector<float>& data) {
+  // written next to the target and renamed: a crash mid-write never leaves a torn checkpoint under `path`
+  const std::string tmp = std::string(path) + ".part";
+  FILE* fp = std::fopen(tmp.c_str(), "wb");
+  if (!fp) return fail(LR_ERR_IO, std::string("cannot write `") + tmp + "`");
+  const bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(data.data(), sizeof(float), data.size(), fp) == data.size();
+  const bool closed = std::fclose(fp) == 0;
+  if (!ok || !closed || std::rename(tmp.c_str(), path) != 0) { std::remove(tmp.c_str()); return fail(LR_ERR_IO, std::string("cannot write `") + path + "`"); }
+  return LR_OK;
+}
+
+// reads a checkpoint made for a film_w x film_h film: its header, its data (as film_write) and the parameters to resume with
+int film_read(const char* path, int film_w, int film_h, FilmHeader* hp, std::vector<float>* data, LrRenderParams* params) {
+  FILE* fp = std::fopen(path, "rb");
+  if (!fp) return fail(LR_ERR_IO, std::string("File `") + path + "` is not found.");
+  FilmHeader& h = *hp;
+  int rc = LR_OK;
+  do {
+    if (std::fread(&h, sizeof(h), 1, fp) != 1 || std::memcmp(h.magic, kFilmMagic, 8) != 0) { rc = fail(LR_ERR_PARSE, "not a film checkpoint"); break; }
+    if (h.film_w != film_w || h.film_h != film_h) { rc = fail(LR_ERR_INVALID, "the checkpoint was made for another film resolution"); break; }
+    if (h.crop_w <= 0 || h.crop_h <= 0 || h.crop_x < 0 || h.crop_y < 0 || h.crop_x + h.crop_w > film_w || h.crop_y + h.crop_h > film_h ||
+        h.spp_done < 0 || h.spp_begin < 0) { rc = fail(LR_ERR_PARSE, "corrupt film checkpoint header"); break; }
+    const size_t n = (size_t)h.crop_w * h.crop_h * 3;
+    data->resize(n * (h.has_sumsq ? 2 : 1));
+    if (std::fread(data->data(), sizeof(float), data->size(), fp) != data->size()) { rc = fail(LR_ERR_PARSE, "truncated film checkpoint"); break; }
+  } while (0);
+  std::fclose(fp);
+  if (rc != LR_OK) return rc;
+  LrRenderParams& p = *params;
+  std::memset(&p, 0, sizeof(p));
+  p.integrator = h.integrator; p.depth = h.depth; p.depth_limit = h.depth_limit; p.no_direct_emitter = h.no_direct_emitter;
+  p.splits = h.splits; p.spp_begin = h.spp_begin; p.seed = h.seed;
+  const bool whole = h.crop_x == 0 && h.crop_y == 0 && h.crop_w == film_w && h.crop_h == film_h;
+  if (!whole) { p.crop_x = h.crop_x; p.crop_y = h.crop_y; p.crop_w = h.crop_w; p.crop_h = h.crop_h; }
+  return LR_OK;
+}
+
 int film_alloc(const LrScene* s, const LrRenderParams* p, int want_sumsq, LrFilm** out) {
   if (!s) return fail(LR_ERR_INVALID, "null argument");
   const OnDevice on(s->device);
@@ -958,50 +1038,18 @@ static int film_save_body(const LrFilm* f, const char* path) {
   std::vector<float> host(n * (f->d_sumsq ? 2 : 1));
   LR_CUDA(cudaMemcpy(host.data(), f->d_sum, n * sizeof(float), cudaMemcpyDeviceToHost));
   if (f->d_sumsq) LR_CUDA(cudaMemcpy(host.data() + n, f->d_sumsq, n * sizeof(float), cudaMemcpyDeviceToHost));
-  FilmHeader h;
-  std::memset(&h, 0, sizeof(h));
-  std::memcpy(h.magic, kFilmMagic, 8);
-  const LrRenderParams& p = f->params;
-  h.film_w = f->scene->width; h.film_h = f->scene->height;
-  h.crop_x = p.crop_w > 0 ? p.crop_x : 0; h.crop_y = p.crop_w > 0 ? p.crop_y : 0; h.crop_w = f->crop_w; h.crop_h = f->crop_h;
-  h.integrator = p.integrator; h.depth = p.depth; h.depth_limit = p.depth_limit; h.no_direct_emitter = p.no_direct_emitter;
-  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = f->spp_done; h.has_sumsq = f->d_sumsq ? 1 : 0; h.seed = p.seed;
-  // written next to the target and renamed: a crash mid-write never leaves a torn checkpoint under `path`
-  const std::string tmp = std::string(path) + ".part";
-  FILE* fp = std::fopen(tmp.c_str(), "wb");
-  if (!fp) return fail(LR_ERR_IO, std::string("cannot write `") + tmp + "`");
-  const bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(host.data(), sizeof(float), host.size(), fp) == host.size();
-  const bool closed = std::fclose(fp) == 0;
-  if (!ok || !closed || std::rename(tmp.c_str(), path) != 0) { std::remove(tmp.c_str()); return fail(LR_ERR_IO, std::string("cannot write `") + path + "`"); }
-  return LR_OK;
+  return film_write(path, film_header(f->scene->width, f->scene->height, f->params, f->crop_w, f->crop_h, f->spp_done, f->d_sumsq != nullptr), host);
 }
 int lr_film_save(const LrFilm* f, const char* path) { LR_GUARDED(film_save_body(f, path)); }
 
 static int film_load_body(const LrScene* s, const char* path, LrFilm** out) {
   if (!s || !path || !out) return fail(LR_ERR_INVALID, "null argument");
   *out = nullptr;
-  FILE* fp = std::fopen(path, "rb");
-  if (!fp) return fail(LR_ERR_IO, std::string("File `") + path + "` is not found.");
   FilmHeader h;
   std::vector<float> host;
-  int rc = LR_OK;
-  do {
-    if (std::fread(&h, sizeof(h), 1, fp) != 1 || std::memcmp(h.magic, kFilmMagic, 8) != 0) { rc = fail(LR_ERR_PARSE, "not a film checkpoint"); break; }
-    if (h.film_w != s->width || h.film_h != s->height) { rc = fail(LR_ERR_INVALID, "the checkpoint was made for another film resolution"); break; }
-    if (h.crop_w <= 0 || h.crop_h <= 0 || h.crop_x < 0 || h.crop_y < 0 || h.crop_x + h.crop_w > s->width || h.crop_y + h.crop_h > s->height ||
-        h.spp_done < 0 || h.spp_begin < 0) { rc = fail(LR_ERR_PARSE, "corrupt film checkpoint header"); break; }
-    const size_t n = (size_t)h.crop_w * h.crop_h * 3;
-    host.resize(n * (h.has_sumsq ? 2 : 1));
-    if (std::fread(host.data(), sizeof(float), host.size(), fp) != host.size()) { rc = fail(LR_ERR_PARSE, "truncated film checkpoint"); break; }
-  } while (0);
-  std::fclose(fp);
-  if (rc != LR_OK) return rc;
   LrRenderParams p;
-  std::memset(&p, 0, sizeof(p));
-  p.integrator = h.integrator; p.depth = h.depth; p.depth_limit = h.depth_limit; p.no_direct_emitter = h.no_direct_emitter;
-  p.splits = h.splits; p.spp_begin = h.spp_begin; p.seed = h.seed;
-  const bool whole = h.crop_x == 0 && h.crop_y == 0 && h.crop_w == s->width && h.crop_h == s->height;
-  if (!whole) { p.crop_x = h.crop_x; p.crop_y = h.crop_y; p.crop_w = h.crop_w; p.crop_h = h.crop_h; }
+  int rc = film_read(path, s->width, s->height, &h, &host, &p);
+  if (rc != LR_OK) return rc;
   LrFilm* f = nullptr;
   if ((rc = film_alloc(s, &p, h.has_sumsq, &f)) != LR_OK) return rc;
   const size_t n = (size_t)h.crop_w * h.crop_h * 3;
@@ -1013,6 +1061,265 @@ static int film_load_body(const LrScene* s, const char* path, LrFilm** out) {
   return LR_OK;
 }
 int lr_film_load(const LrScene* s, const char* path, LrFilm** out) { LR_GUARDED(film_load_body(s, path, out)); }
+
+// ---------------------------------------------------------------- progressive / resumable rendering on several GPUs
+}  // extern "C"
+
+// A film of an LrMultiScene, sharded by pixel: shard k of n_shards (device_scene.h: shard_of_tile) renders on device
+// shard_device(k, n).  Every device keeps a crop-sized sum buffer but writes only the pixels of its own shards; the image
+// is gathered on devices[0], each pixel from the device that owns it.
+struct LrMultiFilm {
+  LrMultiScene* ms = nullptr;
+  LrRenderParams params{};               // as LrFilm's, with splits = 1
+  int32_t spp_done = 0;
+  int32_t crop_w = 0, crop_h = 0;
+  int n_shards = 1;
+  bool has_sumsq = false;
+  float* d_sum[kMaxPeers] = {};          // on ms->devices[i]
+  float* d_sumsq[kMaxPeers] = {};
+};
+
+namespace {
+
+int use_device(const LrMultiScene* m, int i) {
+  const cudaError_t e = cudaSetDevice(m->devices[i]);
+  if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+  g_device = m->devices[i];
+  return LR_OK;
+}
+
+// the end of every multi-film call: after a failure nothing of the call stays in flight; the calling thread and the library
+// are back on the multi scene's home device, as lr_multi_render leaves them
+int multi_finish(const LrMultiScene* m, int rc) {
+  const std::string err = g_error;
+  if (rc != LR_OK) for (int i = 0; i < m->n; i++) { cudaSetDevice(m->devices[i]); cudaDeviceSynchronize(); }
+  cudaSetDevice(m->home);
+  g_device = m->home;
+  g_error = err;
+  return rc;
+}
+
+void mfilm_free(LrMultiFilm* f) {
+  const LrMultiScene* m = f->ms;
+  int prev = 0;
+  cudaGetDevice(&prev);
+  for (int i = 0; i < m->n; i++) {
+    if (!f->d_sum[i] && !f->d_sumsq[i]) continue;
+    cudaSetDevice(m->devices[i]);
+    cudaDeviceSynchronize();
+    dev_free(f->d_sum[i]);
+    dev_free(f->d_sumsq[i]);
+  }
+  cudaSetDevice(prev);
+  delete f;
+}
+
+int mfilm_alloc(LrMultiScene* m, const LrRenderParams* p, int want_sumsq, LrMultiFilm** out) {
+  if (!m || !p || !out) return fail(LR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  // the bit-for-bit contract (every pixel's samples added in order from the stored sum) holds for one thread per pixel only
+  if (p->splits != 0 && p->splits != 1) return fail(LR_ERR_INVALID, "a multi-device film renders with splits = 1");
+  LrRenderParams probe = *p;
+  probe.spp_count = 1;
+  const FilmShard whole{0, 1};
+  DevParams dp;
+  if (int rc = resolve_params(m->scenes[0], &probe, dp, &whole)) return rc;
+  LrMultiFilm* f = new LrMultiFilm();
+  f->ms = m; f->params = *p; f->params.spp_count = 0; f->params.splits = 1;
+  f->crop_w = dp.crop_w; f->crop_h = dp.crop_h; f->has_sumsq = want_sumsq != 0;
+  f->n_shards = m->n;
+  // LR_FILM_SHARDS=S (development / tests): S shards over the devices, so that one GPU runs the interleaved kernels too
+  if (const char* e_shards = std::getenv("LR_FILM_SHARDS")) f->n_shards = std::max(1, std::atoi(e_shards));
+  const size_t bytes = (size_t)dp.crop_w * dp.crop_h * 3 * sizeof(float);
+  int rc = LR_OK;
+  for (int i = 0; i < m->n && rc == LR_OK; i++) {
+    if ((rc = use_device(m, i)) != LR_OK) break;
+    cudaError_t e = dev_alloc((void**)&f->d_sum[i], bytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(f->d_sum[i], 0, bytes, 0);
+    if (e == cudaSuccess && want_sumsq) e = dev_alloc((void**)&f->d_sumsq[i], bytes);
+    if (e == cudaSuccess && want_sumsq) e = cudaMemsetAsync(f->d_sumsq[i], 0, bytes, 0);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(0);       // the render streams do not order against the legacy stream
+    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film: ") + cudaGetErrorString(e));
+  }
+  if ((rc = multi_finish(m, rc)) != LR_OK) {
+    const std::string err = g_error;
+    mfilm_free(f);
+    g_error = err;
+    return rc;
+  }
+  *out = f;
+  return LR_OK;
+}
+
+int mfilm_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) {
+  if (!f) return fail(LR_ERR_INVALID, "null argument");
+  if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
+  LrMultiScene* m = f->ms;
+  LrRenderParams q = f->params;
+  q.spp_begin = f->params.spp_begin + f->spp_done;
+  q.spp_count = spp_count;
+  LrStats total;
+  std::memset(&total, 0, sizeof(total));
+  int rc = LR_OK;
+  do {
+    for (int i = 0; i < m->n && rc == LR_OK; i++) {          // drop the counters of earlier calls
+      LrStats dropped;
+      if ((rc = use_device(m, i)) == LR_OK) rc = lr_stats_fetch(m->scenes[i], m->streams[i], &dropped);
+    }
+    if (rc != LR_OK) break;
+    // launch: asynchronous on every device's own stream, so the devices render concurrently; a device with several shards
+    // renders them one after the other (disjoint pixels of the same buffer)
+    for (int k = 0; k < f->n_shards && rc == LR_OK; k++) {
+      const int i = shard_device(k, m->n);
+      const FilmShard shard{k, f->n_shards};
+      if ((rc = use_device(m, i)) == LR_OK) rc = accumulate(m->scenes[i], &q, f->d_sum[i], f->d_sumsq[i], m->streams[i], &shard);
+    }
+    if (rc != LR_OK) break;
+    // wait for every device; statistics are totals, kernel_ms the slowest device's
+    for (int i = 0; i < m->n && rc == LR_OK; i++) {
+      LrStats st;
+      if ((rc = use_device(m, i)) != LR_OK || (rc = lr_stats_fetch(m->scenes[i], m->streams[i], &st)) != LR_OK) break;
+      add_device_stats(total, st);
+    }
+  } while (0);
+  if ((rc = multi_finish(m, rc)) != LR_OK) return rc;
+  f->spp_done += spp_count;
+  if (stats) *stats = total;
+  return LR_OK;
+}
+
+// The film's crop on devices[0] into dst (device memory there): each pixel from the buffer of the device that owns it
+// (`bufs`: one per device), read over NVLink where devices[0] maps the peer and from a staged copy where it does not;
+// divided by `divisor` if it is > 0.  Asynchronous on devices[0]'s stream; the caller has made devices[0] current.
+int mfilm_gather(const LrMultiFilm* f, float* const* bufs, float* dst, float divisor) {
+  LrMultiScene* m = f->ms;
+  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
+  cudaStream_t st0 = m->streams[0];
+  size_t need_staged = 0;
+  for (int i = 1; i < m->n; i++) if (!m->mapped[i]) need_staged += n;
+  cudaError_t e = cudaSuccess;
+  if (need_staged > m->staged_floats) {
+    e = cudaStreamSynchronize(st0);                           // an earlier gather may still read the old staging buffer
+    if (e == cudaSuccess) {
+      dev_free(m->staged);
+      m->staged = nullptr; m->staged_floats = 0;
+      e = dev_alloc((void**)&m->staged, need_staged * sizeof(float));
+      if (e == cudaSuccess) m->staged_floats = need_staged;
+    }
+  }
+  PeerBuffers src;
+  src.count = m->n;
+  float* stage_next = m->staged;
+  for (int i = 0; i < m->n && e == cudaSuccess; i++) {
+    src.p[i] = bufs[i];
+    if (!m->mapped[i]) {
+      e = cudaMemcpyPeerAsync(stage_next, m->devices[0], bufs[i], m->devices[i], n * sizeof(float), st0);
+      src.p[i] = stage_next;
+      stage_next += n;
+    }
+  }
+  if (e == cudaSuccess) e = launch_gather_shards(dst, src, f->crop_w, f->crop_h, f->n_shards, divisor, st0);
+  if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("multi film gather: ") + cudaGetErrorString(e));
+  return LR_OK;
+}
+
+// the gathered sums (sums of squares after them if asked for) or the mean, to host memory
+int mfilm_download(const LrMultiFilm* f, float divisor, float* out, float* out_sumsq) {
+  const LrMultiScene* m = f->ms;
+  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
+  int rc = use_device(m, 0);
+  float* d_tmp = nullptr;
+  cudaError_t e = cudaSuccess;
+  if (rc == LR_OK) {
+    e = dev_alloc((void**)&d_tmp, n * sizeof(float));
+    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film: ") + cudaGetErrorString(e));
+  }
+  if (rc == LR_OK && (rc = mfilm_gather(f, f->d_sum, d_tmp, divisor)) == LR_OK) {
+    e = cudaMemcpyAsync(out, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, m->streams[0]);
+    if (e == cudaSuccess && out_sumsq && (rc = mfilm_gather(f, f->d_sumsq, d_tmp, 0.0f)) == LR_OK)
+      e = cudaMemcpyAsync(out_sumsq, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, m->streams[0]);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(m->streams[0]);
+    if (rc == LR_OK && e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film D2H: ") + cudaGetErrorString(e));
+  }
+  if (d_tmp) { if (rc != LR_OK) cudaStreamSynchronize(m->streams[0]); dev_free(d_tmp); }
+  return multi_finish(m, rc);
+}
+
+int mfilm_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) {
+  if (!f || !out_rgb) return fail(LR_ERR_INVALID, "null argument");
+  if (out_sumsq && !f->has_sumsq) return fail(LR_ERR_INVALID, "the film was created without sums of squares");
+  if (f->spp_done <= 0) return fail(LR_ERR_INVALID, "the film holds no samples yet");
+  return mfilm_download(f, (float)f->spp_done, out_rgb, out_sumsq);   // main.rs:104, as lr_film_read
+}
+
+int mfilm_save(const LrMultiFilm* f, const char* path) {
+  if (!f || !path) return fail(LR_ERR_INVALID, "null argument");
+  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
+  std::vector<float> host(n * (f->has_sumsq ? 2 : 1));
+  if (int rc = mfilm_download(f, 0.0f, host.data(), f->has_sumsq ? host.data() + n : nullptr)) return rc;
+  const LrScene* s0 = f->ms->scenes[0];
+  return film_write(path, film_header(s0->width, s0->height, f->params, f->crop_w, f->crop_h, f->spp_done, f->has_sumsq), host);
+}
+
+int mfilm_load(LrMultiScene* m, const char* path, LrMultiFilm** out) {
+  if (!m || !path || !out) return fail(LR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  FilmHeader h;
+  std::vector<float> host;
+  LrRenderParams p;
+  int rc = film_read(path, m->scenes[0]->width, m->scenes[0]->height, &h, &host, &p);
+  if (rc != LR_OK) return rc;
+  if (h.splits != 1) return fail(LR_ERR_INVALID, "the checkpoint was rendered with splits != 1; a multi-device film adds samples in order");
+  LrMultiFilm* f = nullptr;
+  if ((rc = mfilm_alloc(m, &p, h.has_sumsq, &f)) != LR_OK) return rc;
+  // the sums go to devices[0], and from there to every other device
+  const size_t bytes = (size_t)h.crop_w * h.crop_h * 3 * sizeof(float);
+  cudaStream_t st0 = m->streams[0];
+  rc = use_device(m, 0);
+  cudaError_t e = cudaSuccess;
+  if (rc == LR_OK) {
+    e = cudaMemcpyAsync(f->d_sum[0], host.data(), bytes, cudaMemcpyHostToDevice, st0);
+    if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyAsync(f->d_sumsq[0], host.data() + bytes / sizeof(float), bytes, cudaMemcpyHostToDevice, st0);
+    for (int i = 1; i < m->n && e == cudaSuccess; i++) {
+      e = cudaMemcpyPeerAsync(f->d_sum[i], m->devices[i], f->d_sum[0], m->devices[0], bytes, st0);
+      if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyPeerAsync(f->d_sumsq[i], m->devices[i], f->d_sumsq[0], m->devices[0], bytes, st0);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st0);
+    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film load: ") + cudaGetErrorString(e));
+  }
+  if ((rc = multi_finish(m, rc)) != LR_OK) {
+    const std::string err = g_error;
+    mfilm_free(f);
+    g_error = err;
+    return rc;
+  }
+  f->spp_done = h.spp_done;
+  *out = f;
+  return LR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* p, int32_t want_sumsq, LrMultiFilm** out) {
+  LR_GUARDED(mfilm_alloc(ms, p, want_sumsq, out));
+}
+int lr_multi_film_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(mfilm_render(f, spp_count, stats)); }
+int lr_multi_film_info(const LrMultiFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) {
+  if (!f) return fail(LR_ERR_INVALID, "null argument");
+  if (spp_done) *spp_done = f->spp_done;
+  if (crop_w) *crop_w = f->crop_w;
+  if (crop_h) *crop_h = f->crop_h;
+  if (has_sumsq) *has_sumsq = f->has_sumsq ? 1 : 0;
+  return LR_OK;
+}
+int lr_multi_film_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(mfilm_read(f, out_rgb, out_sumsq)); }
+int lr_multi_film_save(const LrMultiFilm* f, const char* path) { LR_GUARDED(mfilm_save(f, path)); }
+int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out) { LR_GUARDED(mfilm_load(ms, path, out)); }
+void lr_multi_film_destroy(LrMultiFilm* f) {
+  if (f) mfilm_free(f);
+}
 
 static int measure_read(uint64_t bytes, int iters, int warm, float* gbs) {
   if (!gbs || bytes < (1u << 20) || iters <= 0) return fail(LR_ERR_INVALID, "bad argument");

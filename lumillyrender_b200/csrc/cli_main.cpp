@@ -5,7 +5,8 @@
 // panics become a message on stderr and a non-zero exit status.
 //
 // Extra, optional arguments (not in the reference):  --spp N  --resolution WxH  --seed S  --device D
-//   --gpus N (render on devices D..D+N-1 of this box from this one process: lr_render_multi, samples sharded by index)
+//   --gpus N (render on devices D..D+N-1 of this box from this one process: lr_render_multi, samples sharded by index;
+//   with --progress an LrMultiFilm, pixels sharded by tile, whose checkpoints resume under any other --gpus)
 //   --assets DIR (root that mesh/IBL paths are resolved against; default: the current directory, like the reference)
 //   --progress N (render N samples per pixel at a time through an LrFilm and print the progress line main.rs:81-91 left
 //   commented out)  --checkpoint FILE (with --progress: the film is saved after every chunk, and an existing FILE is
@@ -67,7 +68,8 @@ int main(int argc, char** argv) {
   if (!scene_path) { std::fprintf(stderr, "Path for .toml must be specified.\n"); return 2; }   // main.rs:47-49
   if (aov && std::strcmp(aov, "normal") != 0 && std::strcmp(aov, "depth") != 0) { std::fprintf(stderr, "error: --aov normal|depth\n"); return 2; }
   if (checkpoint && progress <= 0) { std::fprintf(stderr, "error: --checkpoint needs --progress N\n"); return 2; }
-  if ((progress > 0 || aov) && gpus > 1) { std::fprintf(stderr, "error: --progress / --aov render on one GPU\n"); return 2; }
+  if (gpus > 8) { std::fprintf(stderr, "error: --gpus takes 1..8\n"); return 2; }
+  if (aov && gpus > 1) { std::fprintf(stderr, "error: --aov renders on one GPU\n"); return 2; }
   std::printf("loading: %s\n", scene_path);
 
   LrHostScene* hs = nullptr;
@@ -94,10 +96,9 @@ int main(int argc, char** argv) {
   p.depth = cfg.depth; p.depth_limit = cfg.depth_limit; p.no_direct_emitter = cfg.no_direct_emitter; p.seed = seed;
   std::vector<float> img((size_t)cfg.width * cfg.height * 3);
   LrStats st;
-  if (gpus > 1) {
-    if (gpus > 8) { std::fprintf(stderr, "error: --gpus takes 1..8\n"); return 2; }
-    int32_t devices[8];
-    for (int i = 0; i < gpus; i++) devices[i] = device + i;
+  int32_t devices[8];
+  for (int i = 0; i < gpus && i < 8; i++) devices[i] = device + i;
+  if (gpus > 1 && progress <= 0) {
     std::printf("gpus: %d (devices %d..%d, samples sharded by index, one peer-reading reduce)\n", gpus, device, device + gpus - 1);
     if (lr_render_multi(lr_host_scene_desc(hs), &p, gpus, devices, img.data(), nullptr, &st) != LR_OK) return die("rendering");
   } else if (aov) {
@@ -113,30 +114,40 @@ int main(int argc, char** argv) {
     }
     std::printf("aov: %s\n", aov);
   } else if (progress > 0) {
-    // the progress hook of main.rs:81-91 (chunks of samples instead of pixels), resumable through a checkpoint file
+    // the progress hook of main.rs:81-91 (chunks of samples instead of pixels), resumable through a checkpoint file; on
+    // several GPUs the film is sharded by pixel, and both film kinds write and read the same checkpoints
     p.splits = 1;                                             // samples are added in order: any cut of the range gives the same bits
     LrFilm* film = nullptr;
+    LrMultiScene* ms = nullptr;
+    LrMultiFilm* mfilm = nullptr;
+    if (gpus > 1) {
+      std::printf("gpus: %d (devices %d..%d, pixels sharded by tile)\n", gpus, device, device + gpus - 1);
+      if (lr_multi_scene_create(lr_host_scene_desc(hs), gpus, devices, &ms) != LR_OK) return die("uploading scene");
+    }
     struct stat sb;
     if (checkpoint && stat(checkpoint, &sb) == 0) {
-      if (lr_film_load(scene, checkpoint, &film) != LR_OK) return die("resuming the checkpoint");
-    } else if (lr_film_create(scene, &p, 0, &film) != LR_OK) return die("creating the film");
+      if ((ms ? lr_multi_film_load(ms, checkpoint, &mfilm) : lr_film_load(scene, checkpoint, &film)) != LR_OK) return die("resuming the checkpoint");
+    } else if ((ms ? lr_multi_film_create(ms, &p, 0, &mfilm) : lr_film_create(scene, &p, 0, &film)) != LR_OK) return die("creating the film");
     int32_t done = 0;
-    lr_film_info(film, &done, nullptr, nullptr, nullptr);
+    if (ms) lr_multi_film_info(mfilm, &done, nullptr, nullptr, nullptr);
+    else lr_film_info(film, &done, nullptr, nullptr, nullptr);
     if (done > 0) std::printf("resuming: %d of %d spp are in %s\n", done, cfg.samples, checkpoint);
     std::memset(&st, 0, sizeof(st));
     while (done < cfg.samples) {
       const int n = cfg.samples - done < progress ? cfg.samples - done : progress;
       LrStats part;
-      if (lr_film_render(film, n, &part) != LR_OK) return die("rendering");
+      if ((ms ? lr_multi_film_render(mfilm, n, &part) : lr_film_render(film, n, &part)) != LR_OK) return die("rendering");
       done += n;
       st.kernel_ms += part.kernel_ms; st.samples += part.samples; st.rays += part.rays; st.nonfinite_samples += part.nonfinite_samples;
-      if (checkpoint && lr_film_save(film, checkpoint) != LR_OK) return die("writing the checkpoint");
+      if (checkpoint && (ms ? lr_multi_film_save(mfilm, checkpoint) : lr_film_save(film, checkpoint)) != LR_OK) return die("writing the checkpoint");
       std::printf("\rprocessing... (%d/%d : %.0f%%) ", done, cfg.samples, 100.0 * done / cfg.samples);
       std::fflush(stdout);
     }
     std::printf("\n");
-    if (lr_film_read(film, img.data(), nullptr) != LR_OK) return die("reading the film");
+    if ((ms ? lr_multi_film_read(mfilm, img.data(), nullptr) : lr_film_read(film, img.data(), nullptr)) != LR_OK) return die("reading the film");
     lr_film_destroy(film);
+    lr_multi_film_destroy(mfilm);
+    lr_multi_scene_destroy(ms);
   } else if (lr_render(scene, &p, img.data(), nullptr, &st) != LR_OK) return die("rendering");
   if (!aov) std::printf("render: %.3f ms on the GPU, %.1f Msamples/s, %.1f Mrays/s, %llu non-finite samples\n", st.kernel_ms,
               st.samples / (st.kernel_ms * 1e3), st.rays / (st.kernel_ms * 1e3), (unsigned long long)st.nonfinite_samples);

@@ -52,9 +52,25 @@ struct DevParams {
   int crop_x, crop_y, crop_w, crop_h;
   int splits;
   int tiles_x, tiles_y;                  // 8x4 pixel tiles over the crop window
+  int shard, n_shards;                   // this launch renders the tiles t with shard_of_tile(t, n_shards) == shard (default 0 of 1)
+  int unit_tiles;                        // how many tiles that is: shard_tile_count(tiles_x * tiles_y, ...), set once on the host
   int defer_iters, defer_thresh;         // path vertices per phase A; suspended lanes that end it early (persistent.cuh)
   int organisation;                      // 0 = the build's measured best, 1 = one path per lane (persistent.cuh), 2 = pool (pool.cuh); BVH scenes only
 };
+
+// Pixel sharding of a film over several devices (lr_multi_film_*): the crop's 8x4 tiles are dealt round-robin, shard k of
+// S owns the tiles t with t % S == k, and shard k renders on device k % n_devices.  Round-robin balances the load without
+// knowing where the expensive pixels are.  Every pixel is rendered by exactly one shard, so its samples are still added
+// in sample order on one device and the image does not depend on S or on the device count.  The render kernels (decode_unit)
+// and the gather kernel (kernels.cu) both go through these functions.
+__host__ __device__ inline int shard_of_tile(int tile, int n_shards) { return tile % n_shards; }
+__host__ __device__ inline int shard_tile(int j, int shard, int n_shards) { return j * n_shards + shard; }   // j-th tile of the shard
+__host__ __device__ inline int shard_tile_count(int n_tiles, int shard, int n_shards) {
+  return shard < n_tiles ? (n_tiles - shard + n_shards - 1) / n_shards : 0;
+}
+__host__ __device__ inline int shard_device(int shard, int n_devices) { return shard % n_devices; }
+// work items of one render launch: one per (split, pixel slot of the shard's tiles)
+__host__ __device__ inline unsigned int render_units(const DevParams& p) { return (unsigned int)p.unit_tiles * 32u * (unsigned int)p.splits; }
 
 // device counter block (unsigned long long each)
 enum CounterSlot { C_RAYS = 0, C_NONFINITE = 1, C_NODES = 2, C_TRIS = 3, C_SPHERES = 4, C_RETRACE = 5, C_FLAT_TRIS = 6, C_NEXT_UNIT = 7, C_FLAT_BOXES = 8, C_COUNT = 9 };

@@ -1,6 +1,6 @@
 // kernels.cu — the small sm_100a kernels around the render kernel (which lives in persistent.cuh and is
-// instantiated in persistent_inst.cu): ordered reduction of spp splits, normalisation, the nearest-hit parity
-// probes, and the read-bandwidth microbenchmark.
+// instantiated in persistent_inst.cu): ordered reduction of spp splits, normalisation, the cross-device reduce and
+// gather, the nearest-hit parity probes, and the read-bandwidth microbenchmark.
 //
 // Compiled with -fmad=false (see device_path.cuh for the numerics contract).
 #include <algorithm>
@@ -34,6 +34,20 @@ __global__ void reduce_peers_kernel(float* __restrict__ dst, PeerBuffers src, si
   float acc = src.p[0][i];
   for (int k = 1; k < src.count; k++) acc = acc + src.p[k][i];
   dst[i] = divisor > 0.0f ? acc / divisor : acc;
+}
+
+// The image of a pixel-sharded film (lr_multi_film_*), on the first device: every device's buffer spans the whole crop but
+// holds only the pixels of its own shards (stale values or zeros elsewhere), so each pixel is taken from the device that
+// owns its tile, never summed across devices.  Divided by the sample count with the expression of scale_kernel, so the
+// bits equal lr_film_read's; divisor <= 0: the raw sums (sums of squares, checkpoints).
+__global__ void gather_shards_kernel(float* __restrict__ dst, const __grid_constant__ PeerBuffers src, int crop_w, int crop_h, int n_shards, float divisor) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (size_t)crop_w * crop_h * 3) return;
+  const int px = (int)(i / 3), lx = px % crop_w, ly = px / crop_w;
+  const int tiles_x = (crop_w + 7) / 8;
+  const int shard = shard_of_tile((ly >> 2) * tiles_x + (lx >> 3), n_shards);
+  const float v = src.p[shard_device(shard, src.count)][i];
+  dst[i] = divisor > 0.0f ? v / divisor : v;
 }
 
 // parity probe: nearest hit of the primary ray of every film pixel with fixed random numbers
@@ -181,6 +195,12 @@ cudaError_t launch_scale(float* dst, size_t n, float divisor, cudaStream_t strea
 
 cudaError_t launch_reduce_peers(float* dst, const PeerBuffers& src, size_t n, float divisor, cudaStream_t stream) {
   reduce_peers_kernel<<<(unsigned int)((n + 255) / 256), 256, 0, stream>>>(dst, src, n, divisor);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, float divisor, cudaStream_t stream) {
+  const size_t n = (size_t)crop_w * crop_h * 3;
+  gather_shards_kernel<<<(unsigned int)((n + 255) / 256), 256, 0, stream>>>(dst, src, crop_w, crop_h, n_shards, divisor);
   return cudaGetLastError();
 }
 

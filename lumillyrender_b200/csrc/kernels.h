@@ -20,6 +20,8 @@ cudaError_t launch_scale(float* dst, size_t n, float divisor, cudaStream_t strea
 constexpr int kMaxPeers = 8;
 struct PeerBuffers { const float* p[kMaxPeers]; int count; };
 cudaError_t launch_reduce_peers(float* dst, const PeerBuffers& src, size_t n, float divisor, cudaStream_t stream);
+// lr_multi_film: each pixel from the buffer of the device that owns its tile (shard_of_tile / shard_device), / divisor if > 0
+cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, float divisor, cudaStream_t stream);
 cudaError_t launch_primary(const DevScene& sc, float u, float v, float ua, float va, int* prim, float* t, cudaStream_t stream);
 cudaError_t launch_aov(const DevScene& sc, const DevParams& p, int kind, float* out, cudaStream_t stream);
 cudaError_t launch_rays(const DevScene& sc, long long n, const float* org, const float* dir, int* prim, float* t, float* nout,

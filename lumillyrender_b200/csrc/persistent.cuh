@@ -35,12 +35,12 @@ enum { F_DEPTH_MASK = 0xffff, F_ALLOW_EMISSION = 1 << 16, F_HAS_RAY = 1 << 17, F
 LR_DEV unsigned lanemask_lt() { unsigned m; asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m)); return m; }
 LR_DEV unsigned int warp_sum_u(unsigned int v) { return __reduce_add_sync(kFull, v); }
 
-// unit -> (split, crop-relative pixel): 8x4 pixel tiles lane by lane, so a warp starts on one tile
+// unit -> (split, crop-relative pixel): the shard's 8x4 pixel tiles lane by lane, so a warp starts on one tile
 LR_DEV bool decode_unit(const DevParams& p, unsigned int u, int& lx, int& ly, int& split) {
-  const unsigned int per_split = (unsigned int)p.tiles_x * p.tiles_y * 32u;
+  const unsigned int per_split = (unsigned int)p.unit_tiles * 32u;
   split = (int)(u / per_split);
   const unsigned int r = u % per_split;
-  const unsigned int tile = r >> 5, lane = r & 31u;
+  const unsigned int tile = (unsigned int)shard_tile((int)(r >> 5), p.shard, p.n_shards), lane = r & 31u;
   lx = (int)(tile % p.tiles_x) * 8 + (int)(lane & 7u);
   ly = (int)(tile / p.tiles_x) * 4 + (int)(lane >> 3);
   return lx < p.crop_w && ly < p.crop_h;
@@ -87,7 +87,7 @@ render_persistent_kernel(const __grid_constant__ DevScene sc, const __grid_const
   using namespace pk;
   constexpr int NR = INTEGRATOR == LR_INTEGRATOR_PT_DIRECT ? 2 : 1;     // rays a vertex can issue: extension (+ shadow)
   const int lane = (int)(threadIdx.x & 31);
-  const unsigned int n_units = (unsigned int)p.tiles_x * p.tiles_y * 32u * (unsigned int)p.splits;
+  const unsigned int n_units = render_units(p);
   const bool want_sumsq = out_sumsq != nullptr;
   // the flat list every ray gates and tests, staged into shared memory by the bulk-copy engine (device_path.cuh)
   __shared__ __align__(16) float4 flat_tab[kFlatListFloat4];
@@ -187,7 +187,7 @@ cudaError_t launch_persistent_one(const DevScene& sc, const DevParams& p, float*
   int nb = 0;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_persistent_kernel<INTEGRATOR, TREE, COUNT, BUILD>, kBlockThreads, 0) !=
           cudaSuccess || nb <= 0) nb = 4;
-  const long long units = (long long)p.tiles_x * p.tiles_y * 32 * p.splits;
+  const long long units = render_units(p);
   const long long want = (units + kBlockThreads - 1) / kBlockThreads;
   const unsigned int blocks = (unsigned int)std::max<long long>(1, std::min<long long>(want, (long long)nb * sm_count));
   render_persistent_kernel<INTEGRATOR, TREE, COUNT, BUILD><<<blocks, kBlockThreads, 0, stream>>>(sc, p, out_sum, out_sumsq, counters, next_unit);

@@ -122,7 +122,7 @@ render_pool_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ 
   const FlatList flat = stage_flat_list(sc, flat_tab, &flat_bar);
   extern __shared__ float pool_smem[];
   const int lane = (int)(threadIdx.x & 31);
-  const unsigned int n_units = (unsigned int)p.tiles_x * p.tiles_y * 32u * (unsigned int)p.splits;
+  const unsigned int n_units = render_units(p);
   const bool want_sumsq = out_sumsq != nullptr;
   float* const pool = pool_smem + (threadIdx.x >> 5) * warp_words<INTEGRATOR>(want_sumsq);
   int* const list = (int*)(pool + words_per_slot<INTEGRATOR>(want_sumsq) * NS);
@@ -315,7 +315,7 @@ cudaError_t launch_pool_one(const DevScene& sc, const DevParams& p, float* out_s
   int nb = 0;
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, kBlockThreads, smem) != cudaSuccess || nb <= 0) nb = 2;
   // a warp serves kSlots units at a time
-  const long long units = (long long)p.tiles_x * p.tiles_y * 32 * p.splits;
+  const long long units = render_units(p);
   const long long per_block = (long long)(kBlockThreads / 32) * pl::slots<INTEGRATOR>();
   const long long want = (units + per_block - 1) / per_block;
   const unsigned int blocks = (unsigned int)std::max<long long>(1, std::min<long long>(want, (long long)nb * sm_count));

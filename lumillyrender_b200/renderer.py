@@ -232,6 +232,14 @@ class MultiScene:
         check(self._lib.lr_multi_render(self._m, C.byref(p), _fptr(img), _fptr(sq) if sumsq else None, C.byref(st)))
         return img, sq, st.as_dict()
 
+    def film(self, sumsq=False, **kw):
+        """A resumable render on all the devices, sharded by pixel (lr_multi_film_*): see MultiFilm."""
+        return MultiFilm(self, params=kw.pop("params", None) or params_from_config(self.config, **kw), sumsq=sumsq)
+
+    def load_film(self, path):
+        """Resumes a checkpoint written by Film.save or MultiFilm.save on these devices."""
+        return MultiFilm(self, path=path)
+
     def close(self):
         if self._m:
             self._lib.lr_multi_scene_destroy(self._m)
@@ -244,25 +252,25 @@ class MultiScene:
             pass
 
 
-class Film:
-    """Per-pixel sums of a render in progress on the scene's device (lr_film_*): `render(n)` adds the next n sample
-    indices, `read()` gives the mean so far, `save(path)` / `Scene.load_film(path)` checkpoint and resume.  With
-    splits = 1 any cut of the sample range into `render` calls gives bit for bit the image of one `Scene.render`."""
+class _FilmBase:
+    """A render in progress behind one of the two film handles of the C ABI; `_API` is the prefix of its entry points
+    (lr_film_* or lr_multi_film_*), `owner` the handle they are created on."""
+    _API = None
 
-    def __init__(self, scene, params=None, sumsq=False, path=None):
+    def __init__(self, owner, params=None, sumsq=False, path=None):
         self._lib = capi.load_library()
-        self.scene = scene
+        self._fn = {n: getattr(self._lib, "%s_%s" % (self._API, n)) for n in ("create", "load", "render", "info", "read", "save", "destroy")}
         self._f = C.c_void_p()
         if path is not None:
-            check(self._lib.lr_film_load(scene._s, str(path).encode(), C.byref(self._f)))
+            check(self._fn["load"](owner, str(path).encode(), C.byref(self._f)))
         else:
-            check(self._lib.lr_film_create(scene._s, C.byref(params), 1 if sumsq else 0, C.byref(self._f)))
+            check(self._fn["create"](owner, C.byref(params), 1 if sumsq else 0, C.byref(self._f)))
         _, w, h, self.has_sumsq = self._info()
         self._shape = (h, w, 3)
 
     def _info(self):
         v = [C.c_int32() for _ in range(4)]
-        check(self._lib.lr_film_info(self._f, *[C.byref(x) for x in v]))
+        check(self._fn["info"](self._f, *[C.byref(x) for x in v]))
         return [x.value for x in v]
 
     @property
@@ -271,21 +279,21 @@ class Film:
 
     def render(self, spp):
         st = LrStats()
-        check(self._lib.lr_film_render(self._f, int(spp), C.byref(st)))
+        check(self._fn["render"](self._f, int(spp), C.byref(st)))
         return st.as_dict()
 
     def read(self, sumsq=False):
         img = np.empty(self._shape, dtype=np.float32)
         sq = np.empty(self._shape, dtype=np.float32) if sumsq else None
-        check(self._lib.lr_film_read(self._f, _fptr(img), _fptr(sq) if sumsq else None))
+        check(self._fn["read"](self._f, _fptr(img), _fptr(sq) if sumsq else None))
         return (img, sq) if sumsq else img
 
     def save(self, path):
-        check(self._lib.lr_film_save(self._f, str(path).encode()))
+        check(self._fn["save"](self._f, str(path).encode()))
 
     def close(self):
         if self._f:
-            self._lib.lr_film_destroy(self._f)
+            self._fn["destroy"](self._f)
             self._f = C.c_void_p()
 
     def __del__(self):
@@ -293,6 +301,28 @@ class Film:
             self.close()
         except Exception:
             pass
+
+
+class Film(_FilmBase):
+    """Per-pixel sums of a render in progress on the scene's device (lr_film_*): `render(n)` adds the next n sample
+    indices, `read()` gives the mean so far, `save(path)` / `Scene.load_film(path)` checkpoint and resume.  With
+    splits = 1 any cut of the sample range into `render` calls gives bit for bit the image of one `Scene.render`."""
+    _API = "lr_film"
+
+    def __init__(self, scene, params=None, sumsq=False, path=None):
+        self.scene = scene
+        super().__init__(scene._s, params, sumsq, path)
+
+
+class MultiFilm(_FilmBase):
+    """The same film on the devices of a MultiScene (lr_multi_film_*), sharded by 8x4 pixel tile: the image, sums of
+    squares and ray count are bit for bit those of `Scene.render(splits=1)` for any device count, and its checkpoints
+    are those of Film (either kind resumes the other's)."""
+    _API = "lr_multi_film"
+
+    def __init__(self, multi_scene, params=None, sumsq=False, path=None):
+        self.multi_scene = multi_scene
+        super().__init__(multi_scene._m, params, sumsq, path)
 
 
 def init(device=0):
