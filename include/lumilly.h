@@ -172,7 +172,7 @@ typedef struct LrStats {
   int32_t splits;              /* splits actually used                            */
 } LrStats;
 
-typedef struct LrScene LrScene;   /* opaque; owns device memory on the device that was current at lr_scene_create (lr_init).
+typedef struct LrScene LrScene;   /* opaque; owns device memory on the library's device (lr_init) at lr_scene_create.
                                      Every entry point that takes a scene (or a film of it) switches the calling thread to
                                      that device for the call and restores the caller's device on return.               */
 
@@ -213,9 +213,9 @@ int lr_stats_fetch(const LrScene* scene, void* cuda_stream, LrStats* stats);
    (peer access; staged copies where peer access is unavailable), adds them in list order and divides by
    spp_count.  out_rgb / out_sumsq / stats as lr_render (stats are totals, kernel_ms the slowest device's).
    1 <= n_devices <= 8, device ids distinct.  The result for a given device COUNT is bit-reproducible and
-   differs from other counts only by fp32 summation order.  Not re-entrant: it switches the calling thread's
-   CUDA device (restored on return) and the library's current device, so call it from one thread at a time
-   and not concurrently with other entry points. */
+   differs from other counts only by fp32 summation order.  It switches the calling thread's CUDA device as it
+   works and restores it on return; the library's device (lr_init) is untouched.  Not re-entrant: call it from
+   one thread at a time and not concurrently with other entry points. */
 /* The sample-range sharding rule, for any host that shards by itself (one process per GPU): part `part` of
    `n_parts` of the range [spp_begin, spp_begin + spp_count) — consecutive ranges that tile it exactly, sizes
    differing by <= 1, the larger ones first.  lr_render_multi and bench.py's ranks use this rule. */
@@ -268,8 +268,8 @@ void lr_film_destroy(LrFilm* film);
  * params->splits must be 0 or 1 (it is always 1).  save writes the checkpoint format of lr_film_save, byte for byte
  * what lr_film_save writes for the same state; lr_film_load resumes it on one device, and lr_multi_film_load resumes a
  * checkpoint of either kind on any LrMultiScene (its header must say splits = 1).  Destroy the films of an LrMultiScene
- * before the LrMultiScene.  Not re-entrant, like lr_multi_render: the calls switch the calling thread's CUDA device
- * (restored on return) and the library's current device.                                                           */
+ * before the LrMultiScene.  Not re-entrant, like lr_multi_render: the calls switch the calling thread's CUDA device as
+ * they work and restore it on return; the library's device (lr_init) is untouched.                                */
 typedef struct LrMultiFilm LrMultiFilm;
 int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* params, int32_t want_sumsq, LrMultiFilm** out);
 int lr_multi_film_render(LrMultiFilm* film, int32_t spp_count, LrStats* stats /* nullable */);

@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <system_error>
@@ -100,6 +101,21 @@ extern "C" {
 int lr_abi_version(void) { return LR_ABI_VERSION; }
 const char* lr_last_error(void) { return g_error.c_str(); }
 
+// What every device this library renders on is set up with (lr_init, lr_multi_scene_create): a memory pool that never trims.
+// Gives the device's SM count.
+static int setup_device(int device, int* sm_count) {
+  cudaDeviceProp prop;
+  const cudaError_t e = cudaGetDeviceProperties(&prop, device);
+  if (e != cudaSuccess) return fail(LR_ERR_NO_DEVICE, std::string("cudaGetDeviceProperties: ") + cudaGetErrorString(e));
+  *sm_count = std::max(prop.multiProcessorCount, 1);
+  cudaMemPool_t pool;
+  if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
+    unsigned long long keep = ~0ull;                    // never give freed blocks back to the driver
+    cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
+  }
+  return LR_OK;
+}
+
 int lr_init(int device) {
   int n = 0;
   cudaError_t e = cudaGetDeviceCount(&n);
@@ -109,18 +125,10 @@ int lr_init(int device) {
   if (device < 0 || device >= n) return fail(LR_ERR_INVALID, "device index out of range");
   e = cudaSetDevice(device);
   if (e != cudaSuccess) return fail(LR_ERR_NO_DEVICE, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
-  cudaDeviceProp prop;
-  e = cudaGetDeviceProperties(&prop, device);
-  if (e != cudaSuccess) return fail(LR_ERR_NO_DEVICE, std::string("cudaGetDeviceProperties: ") + cudaGetErrorString(e));
+  int sm_count = 0;
+  if (int rc = setup_device(device, &sm_count)) return rc;
   g_device = device;
-  g_sm_count = prop.multiProcessorCount;
-  {
-    cudaMemPool_t pool;
-    if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
-      unsigned long long keep = ~0ull;                    // never give freed blocks back to the driver
-      cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
-    }
-  }
+  g_sm_count = sm_count;
   return LR_OK;
 }
 
@@ -137,11 +145,9 @@ int lr_device_info(int* sm_count, int* l2_bytes, int* sm_clock_khz, char* name, 
   return LR_OK;
 }
 
-static int lr_scene_create_body(const LrSceneDesc* d, LrScene** out) {
-  if (!d || !out) return fail(LR_ERR_INVALID, "null argument");
-  *out = nullptr;
-  if (int rc = validate_desc(*d)) return rc;
-  if (int rc = ensure_device()) return rc;
+// the scene on `device` (with `sm_count` SMs); lr_scene_create passes the library's device
+static int scene_create(const LrSceneDesc* d, int device, int sm_count, LrScene** out) {
+  const OnDevice on(device);
 
   // ---- sizes.  Everything goes into ONE device block, packed on the host straight into a pinned staging arena and
   // uploaded with one copy (lr_scene_create is inside the timed region of an end-to-end render: 11 ms -> 4 ms).
@@ -190,7 +196,7 @@ static int lr_scene_create_body(const LrSceneDesc* d, LrScene** out) {
 
   struct SceneGuard { LrScene* s; ~SceneGuard() { if (s) lr_scene_destroy(s); } } guard{new LrScene()};   // released on success
   LrScene* s = guard.s;
-  s->device = g_device; s->sm_count = std::max(g_sm_count, 1);
+  s->device = device; s->sm_count = sm_count;
   cudaError_t e = cudaSuccess;
   DevScene& dv = s->dev;
   float area = 0.0f;
@@ -318,15 +324,21 @@ static int lr_scene_create_body(const LrSceneDesc* d, LrScene** out) {
   *out = s;
   return LR_OK;
 }
+
+static int lr_scene_create_body(const LrSceneDesc* d, LrScene** out) {
+  if (!d || !out) return fail(LR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  if (int rc = validate_desc(*d)) return rc;
+  if (int rc = ensure_device()) return rc;
+  return scene_create(d, g_device, g_sm_count, out);
+}
 int lr_scene_create(const LrSceneDesc* d, LrScene** out) { LR_GUARDED(lr_scene_create_body(d, out)); }
 
 void lr_scene_destroy(LrScene* s) {
   if (!s) return;
   // work of this handle may still be in flight on a caller stream the legacy stream does not order against
   if (s->ev_pending && s->ev1) cudaEventSynchronize(s->ev1);
-  int cur = -1;
-  const bool hop = cudaGetDevice(&cur) == cudaSuccess && cur != s->device && !s->allocs.empty();
-  if (hop) cudaSetDevice(s->device);                    // frees go to the owning device's stream
+  const OnDevice on(s->device);                         // frees go to the owning device's stream
   for (void* p : s->allocs) dev_free(p);                // one block: scene arrays + the counter words
   dev_free(s->d_film);
   dev_free(s->d_film_sq);
@@ -334,7 +346,6 @@ void lr_scene_destroy(LrScene* s) {
   dev_free(s->d_partial_sq);
   if (s->ev0) cudaEventDestroy(s->ev0);
   if (s->ev1) cudaEventDestroy(s->ev1);
-  if (hop) cudaSetDevice(cur);
   delete s;
 }
 
@@ -344,7 +355,7 @@ int lr_scene_bytes(const LrScene* s, uint64_t* h2d_bytes) {
   return LR_OK;
 }
 
-// One part of a pixel-sharded film (lr_multi_film_*): shard `index` of `count` (device_scene.h: shard_of_tile).  Such a
+// One shard of a sharded film (an LrMultiFilm): shard `index` of `count` (device_scene.h: shard_of_tile).  Such a
 // render always runs one thread per pixel, adding its samples in order (splits = 1), whatever LR_SPLITS says.
 struct FilmShard { int index, count; };
 
@@ -371,7 +382,7 @@ static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& 
   if (splits <= 0) {
     // auto: enough threads for ~2 full waves of 148 SMs x 2048 resident threads, >= 4 samples per thread
     const long long px_threads = (long long)dp.tiles_x * dp.tiles_y * 32;
-    const long long target = 2LL * std::max(g_sm_count, 1) * 2048;
+    const long long target = 2LL * s->sm_count * 2048;
     splits = (int)std::min<long long>((target + px_threads - 1) / px_threads, std::max(1, p->spp_count / 4));
   }
   splits = std::max(1, std::min(splits, p->spp_count));
@@ -414,14 +425,13 @@ static uint64_t shard_pixels(const DevParams& dp) {
   return n;
 }
 
-// lr_render_accumulate_device for the whole crop (shard = nullptr) or for one shard of its tiles (lr_multi_film_render)
+// lr_render_accumulate_device for the whole crop (shard = nullptr) or for one shard of its tiles (film_render)
 static int accumulate(const LrScene* s, const LrRenderParams* p, float* d_sum, float* d_sumsq, void* cuda_stream, const FilmShard* shard) {
   if (!s) return fail(LR_ERR_INVALID, "null argument");
   const OnDevice on(s->device);
   DevParams dp;
   if (int rc = resolve_params(s, p, dp, shard)) return rc;
   if (!d_sum) return fail(LR_ERR_INVALID, "d_sum is null");
-  if (int rc = ensure_device()) return rc;
   cudaStream_t st = (cudaStream_t)cuda_stream;
   const size_t n = (size_t)dp.crop_w * dp.crop_h * 3;
   float* ksum = d_sum; float* ksq = d_sumsq;
@@ -469,7 +479,6 @@ int lr_render_accumulate_device(const LrScene* s, const LrRenderParams* p, float
 int lr_stats_fetch(const LrScene* s, void* cuda_stream, LrStats* stats) {
   if (!s || !stats) return fail(LR_ERR_INVALID, "null argument");
   const OnDevice on(s->device);
-  if (!s || !stats) return fail(LR_ERR_INVALID, "null argument");
   cudaStream_t st = (cudaStream_t)cuda_stream;
   LR_CUDA(cudaStreamSynchronize(st));
   if (s->ev_pending) {
@@ -497,7 +506,6 @@ int lr_render(const LrScene* s, const LrRenderParams* p, float* out_rgb, float* 
   DevParams dp;
   if (int rc = resolve_params(s, p, dp)) return rc;
   if (!out_rgb) return fail(LR_ERR_INVALID, "out_rgb is null");
-  if (int rc = ensure_device()) return rc;
   const size_t n = (size_t)dp.crop_w * dp.crop_h * 3;
   // the film buffers live in the scene handle between calls (no cudaMalloc / cudaFree inside an end-to-end render)
   if (int rc = ensure_scratch(&s->d_film, &s->film_floats, n)) return rc;
@@ -524,15 +532,13 @@ int lr_render(const LrScene* s, const LrRenderParams* p, float* out_rgb, float* 
 }
 
 int lr_render_aov(const LrScene* s, const LrRenderParams* p, int32_t kind, float* out) {
-  if (!s) return fail(LR_ERR_INVALID, "null argument");
-  const OnDevice on(s->device);
   if (!s || !p || !out) return fail(LR_ERR_INVALID, "null argument");
+  const OnDevice on(s->device);
   if (kind != LR_AOV_NORMAL && kind != LR_AOV_DEPTH) return fail(LR_ERR_INVALID, "unknown AOV kind");
   LrRenderParams q = *p;
   q.integrator = LR_INTEGRATOR_PT;                      // not used by the AOVs
   DevParams dp;
   if (int rc = resolve_params(s, &q, dp)) return rc;
-  if (int rc = ensure_device()) return rc;
   const size_t n = (size_t)dp.crop_w * dp.crop_h * (kind == LR_AOV_NORMAL ? 3 : 1);
   float* d_out = nullptr;
   LR_CUDA(dev_alloc((void**)&d_out, n * sizeof(float)));
@@ -552,20 +558,20 @@ int lr_shard_range(int32_t spp_begin, int32_t spp_count, int32_t part, int32_t n
   return LR_OK;
 }
 
-// A copy of a device scene on the CURRENT device: the packed block travels device to device (NVLink) instead of being
-// packed and uploaded from the host again, and the array pointers are rebased into the new block.
-static int scene_clone(const LrScene* src, int src_device, int dst_device, LrScene** out) {
+// A copy of a device scene on `dst_device`, which the caller has made current: the packed block travels device to device
+// (NVLink) instead of being packed and uploaded from the host again, and the array pointers are rebased into the new block.
+static int scene_clone(const LrScene* src, int dst_device, int sm_count, LrScene** out) {
   *out = nullptr;
   if (src->allocs.size() != 1 || src->block_bytes == 0) return fail(LR_ERR_INVALID, "scene_clone: unexpected scene layout");
   LrScene* s = new LrScene();
-  s->device = dst_device; s->sm_count = std::max(g_sm_count, 1);       // lr_init(dst_device) ran just before
+  s->device = dst_device; s->sm_count = sm_count;
   char* block = nullptr;
   const char* from = (const char*)src->allocs[0];
   cudaError_t e = dev_alloc((void**)&block, src->block_bytes);
   if (e == cudaSuccess) {
     s->allocs.push_back(block);
     s->block_bytes = src->block_bytes;
-    e = cudaMemcpyPeerAsync(block, dst_device, from, src_device, src->h2d_bytes, 0);
+    e = cudaMemcpyPeerAsync(block, dst_device, from, src->device, src->h2d_bytes, 0);
   }
   const size_t o_counters = (const char*)src->d_counters - from;
   if (e == cudaSuccess) e = cudaMemsetAsync(block + o_counters, 0, C_COUNT * sizeof(unsigned long long), 0);
@@ -606,10 +612,34 @@ struct LrMultiScene {
   bool mapped[kMaxPeers] = {};
   float* staged = nullptr;                 // on devices[0]: copies of the film buffers it cannot map
   size_t staged_floats = 0;
-  int home = 0;
 };
 
 namespace {
+
+// OnDevice for a call that works on several devices: use(d) makes device d current, and on every way out the calling
+// thread's device is restored.  A call that fails (`rc`, the caller's status, is not LR_OK when the guard goes out of scope)
+// first synchronises every device it used, so nothing of the call stays in flight.
+struct OnDevices {
+  const int& rc;
+  int prev = -1;
+  int used[kMaxPeers] = {};
+  int n_used = 0;
+  explicit OnDevices(const int& status) : rc(status) {
+    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
+  }
+  ~OnDevices() {
+    if (rc != LR_OK) for (int i = 0; i < n_used; i++) { cudaSetDevice(used[i]); cudaDeviceSynchronize(); }
+    if (prev >= 0) cudaSetDevice(prev);
+  }
+  int use(int device) {
+    const cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+    if (std::find(used, used + n_used, device) == used + n_used && n_used < kMaxPeers) used[n_used++] = device;
+    return LR_OK;
+  }
+  OnDevices(const OnDevices&) = delete;
+  OnDevices& operator=(const OnDevices&) = delete;
+};
 
 // device i's stream-ordered pool grants `reader` access (plain cudaDeviceEnablePeerAccess covers cudaMalloc memory only)
 bool map_peer(int reader, int owner) {
@@ -641,30 +671,28 @@ int multi_create(const LrSceneDesc* desc, int32_t n_devices, const int32_t* devi
     if (devices[i] < 0 || devices[i] >= n_visible) return fail(LR_ERR_INVALID, "device index out of range");
     for (int j = 0; j < i; j++) if (devices[j] == devices[i]) return fail(LR_ERR_INVALID, "device listed twice");
   }
-  int prev_device = 0;
-  cudaGetDevice(&prev_device);
+  if (int rc = validate_desc(*desc)) return rc;
   LrMultiScene* m = new LrMultiScene();
   m->n = n_devices;
-  m->home = g_device >= 0 ? g_device : devices[0];
   for (int i = 0; i < n_devices; i++) m->devices[i] = devices[i];
   int rc = LR_OK;
-  // scenes first: the first device gets the scene from the host, the others a device-to-device copy of its packed block
-  for (int i = 0; i < n_devices && rc == LR_OK; i++) {
-    if ((rc = lr_init(devices[i])) != LR_OK) break;          // cudaSetDevice + the non-trimming memory pool
-    if ((rc = i == 0 ? lr_scene_create(desc, &m->scenes[0]) : scene_clone(m->scenes[0], devices[0], devices[i], &m->scenes[i])) != LR_OK) break;
-    cudaError_t e = cudaStreamCreateWithFlags(&m->streams[i], cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->done[i], cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(0);      // the clone has landed
-    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("lr_multi_scene_create: ") + cudaGetErrorString(e));
+  {
+    OnDevices on(rc);
+    // scenes first: the first device gets the scene from the host, the others a device-to-device copy of its packed block
+    for (int i = 0; i < n_devices && rc == LR_OK; i++) {
+      int sm_count = 0;
+      if ((rc = on.use(devices[i])) != LR_OK || (rc = setup_device(devices[i], &sm_count)) != LR_OK) break;
+      if ((rc = i == 0 ? scene_create(desc, devices[0], sm_count, &m->scenes[0]) : scene_clone(m->scenes[0], devices[i], sm_count, &m->scenes[i])) != LR_OK) break;
+      cudaError_t e = cudaStreamCreateWithFlags(&m->streams[i], cudaStreamNonBlocking);
+      if (e == cudaSuccess) e = cudaEventCreateWithFlags(&m->done[i], cudaEventDisableTiming);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(0);      // the clone has landed
+      if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("lr_multi_scene_create: ") + cudaGetErrorString(e));
+    }
+    m->mapped[0] = true;
+    for (int i = 1; i < n_devices && rc == LR_OK; i++) m->mapped[i] = map_peer(devices[0], devices[i]);
   }
-  m->mapped[0] = true;
-  for (int i = 1; i < n_devices && rc == LR_OK; i++) m->mapped[i] = map_peer(devices[0], devices[i]);
-  cudaSetDevice(m->home >= 0 && m->home < n_visible ? m->home : prev_device);
-  g_device = m->home;
   if (rc != LR_OK) {
-    const std::string err = g_error;
     lr_multi_scene_destroy(m);
-    g_error = err;
     return rc;
   }
   *out = m;
@@ -679,6 +707,35 @@ void add_device_stats(LrStats& total, const LrStats& st) {
   total.kernel_ms = std::max(total.kernel_ms, st.kernel_ms);
   total.launches += st.launches;
   total.splits = std::max(total.splits, st.splits);
+}
+
+// What devices[0] of `m` reads of the per-device buffers bufs[0..count), n floats each on m->devices[i]: the buffer itself
+// where devices[0] maps device i (always for i = 0), otherwise a copy staged into m->staged, which only grows.  Asynchronous
+// on `stream`, a stream of devices[0], which the caller has made current.  One buffer needs no LrMultiScene (m may be null).
+cudaError_t peer_buffers(LrMultiScene* m, int count, float* const* bufs, size_t n, cudaStream_t stream, PeerBuffers* src) {
+  size_t need = 0;
+  for (int i = 1; i < count; i++) if (!m->mapped[i]) need += n;
+  cudaError_t e = cudaSuccess;
+  if (need > 0 && need > m->staged_floats) {
+    e = cudaStreamSynchronize(stream);                         // an earlier call may still read the old staging buffer
+    if (e == cudaSuccess) {
+      dev_free(m->staged);
+      m->staged = nullptr; m->staged_floats = 0;
+      e = dev_alloc((void**)&m->staged, need * sizeof(float));
+      if (e == cudaSuccess) m->staged_floats = need;
+    }
+  }
+  src->count = count;
+  float* stage_next = need > 0 ? m->staged : nullptr;
+  for (int i = 0; i < count && e == cudaSuccess; i++) {
+    src->p[i] = bufs[i];
+    if (i > 0 && !m->mapped[i]) {
+      e = cudaMemcpyPeerAsync(stage_next, m->devices[0], bufs[i], m->devices[i], n * sizeof(float), stream);
+      src->p[i] = stage_next;
+      stage_next += n;
+    }
+  }
+  return e;
 }
 
 int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float* out_sumsq, LrStats* stats) {
@@ -699,12 +756,11 @@ int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float
   int rc = LR_OK;
   LrStats total;
   std::memset(&total, 0, sizeof(total));
+  OnDevices on(rc);
   do {
     // ---- launch: asynchronous on every device's own stream, so the devices render concurrently
     for (int i = 0; i < n_devices && rc == LR_OK; i++) {
-      cudaError_t e = cudaSetDevice(m->devices[i]);
-      if (e != cudaSuccess) { rc = fail(LR_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e)); break; }
-      g_device = m->devices[i];
+      if ((rc = on.use(m->devices[i])) != LR_OK) break;
       const LrScene* s = m->scenes[i];
       parts[i] = *p;
       if ((rc = lr_shard_range(p->spp_begin, p->spp_count, i, n_devices, &parts[i].spp_begin, &parts[i].spp_count)) != LR_OK) break;
@@ -715,7 +771,7 @@ int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float
       n = (size_t)dp.crop_w * dp.crop_h * 3;
       if ((rc = ensure_scratch(&s->d_film, &s->film_floats, n)) != LR_OK) break;
       if (out_sumsq && (rc = ensure_scratch(&s->d_film_sq, &s->film_sq_floats, n)) != LR_OK) break;
-      e = cudaMemsetAsync(s->d_film, 0, n * sizeof(float), m->streams[i]);
+      cudaError_t e = cudaMemsetAsync(s->d_film, 0, n * sizeof(float), m->streams[i]);
       if (e == cudaSuccess && out_sumsq) e = cudaMemsetAsync(s->d_film_sq, 0, n * sizeof(float), m->streams[i]);
       if (e != cudaSuccess) { rc = fail(LR_ERR_CUDA, std::string("lr_multi_render set-up: ") + cudaGetErrorString(e)); break; }
       if (parts[i].spp_count > 0 &&
@@ -728,58 +784,32 @@ int multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, float
 
     // ---- reduce + normalise on devices[0]: one kernel reads every device's sums (peer access over NVLink; a staged copy
     // where a peer cannot be mapped), adds them in list order and divides by spp (main.rs:104)
-    cudaError_t e = cudaSetDevice(m->devices[0]);
-    g_device = m->devices[0];
+    if ((rc = on.use(m->devices[0])) != LR_OK) break;
     cudaStream_t st0 = m->streams[0];
-    PeerBuffers sum_src, sq_src;
-    sum_src.count = sq_src.count = n_devices;
-    size_t need_staged = 0;
-    for (int i = 1; i < n_devices; i++) if (!m->mapped[i]) need_staged += n * (out_sumsq ? 2 : 1);
-    if (e == cudaSuccess && need_staged > m->staged_floats) {
-      dev_free(m->staged);
-      m->staged = nullptr; m->staged_floats = 0;
-      e = dev_alloc((void**)&m->staged, need_staged * sizeof(float));
-      if (e == cudaSuccess) m->staged_floats = need_staged;
+    cudaError_t e = cudaSuccess;
+    for (int i = 1; i < n_devices && e == cudaSuccess; i++) e = cudaStreamWaitEvent(st0, m->done[i], 0);   // device i's render
+    for (int sq = 0; sq < (out_sumsq ? 2 : 1) && e == cudaSuccess; sq++) {
+      float* bufs[kMaxPeers];
+      for (int i = 0; i < n_devices; i++) bufs[i] = sq ? m->scenes[i]->d_film_sq : m->scenes[i]->d_film;
+      PeerBuffers src;
+      e = peer_buffers(m, n_devices, bufs, n, st0, &src);
+      if (e == cudaSuccess) e = launch_reduce_peers(bufs[0], src, n, sq ? 0.0f : (float)p->spp_count, st0);   // main.rs:104
+      if (e == cudaSuccess) e = cudaMemcpyAsync(sq ? out_sumsq : out_rgb, bufs[0], n * sizeof(float), cudaMemcpyDeviceToHost, st0);
     }
-    float* stage_next = m->staged;
-    for (int i = 0; i < n_devices && e == cudaSuccess; i++) {
-      if (i > 0) e = cudaStreamWaitEvent(st0, m->done[i], 0);     // devices[0]'s stream waits for device i's render
-      if (e != cudaSuccess) break;
-      sum_src.p[i] = m->scenes[i]->d_film;
-      sq_src.p[i] = out_sumsq ? m->scenes[i]->d_film_sq : nullptr;
-      if (!m->mapped[i]) {
-        e = cudaMemcpyPeerAsync(stage_next, m->devices[0], m->scenes[i]->d_film, m->devices[i], n * sizeof(float), st0);
-        sum_src.p[i] = stage_next; stage_next += n;
-        if (e == cudaSuccess && out_sumsq) {
-          e = cudaMemcpyPeerAsync(stage_next, m->devices[0], m->scenes[i]->d_film_sq, m->devices[i], n * sizeof(float), st0);
-          sq_src.p[i] = stage_next; stage_next += n;
-        }
-      }
-    }
-    if (e == cudaSuccess) e = launch_reduce_peers(m->scenes[0]->d_film, sum_src, n, (float)p->spp_count, st0);   // main.rs:104
-    if (e == cudaSuccess && out_sumsq) e = launch_reduce_peers(m->scenes[0]->d_film_sq, sq_src, n, 0.0f, st0);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out_rgb, m->scenes[0]->d_film, n * sizeof(float), cudaMemcpyDeviceToHost, st0);
-    if (e == cudaSuccess && out_sumsq) e = cudaMemcpyAsync(out_sumsq, m->scenes[0]->d_film_sq, n * sizeof(float), cudaMemcpyDeviceToHost, st0);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st0);
     if (e != cudaSuccess) { rc = fail(LR_ERR_CUDA, std::string("lr_multi_render reduce: ") + cudaGetErrorString(e)); break; }
     lap("render+d2h");
 
     // ---- statistics: totals over the devices, the slowest device's kernel time
     for (int i = 0; i < n_devices && rc == LR_OK; i++) {
-      if (cudaSetDevice(m->devices[i]) != cudaSuccess) { rc = fail(LR_ERR_CUDA, "cudaSetDevice failed"); break; }
-      g_device = m->devices[i];
       LrStats st;
       if ((rc = lr_stats_fetch(m->scenes[i], m->streams[i], &st)) != LR_OK) break;
       add_device_stats(total, st);
     }
     total.launches += out_sumsq ? 2 : 1;
   } while (0);
-  const std::string err = g_error;
-  if (rc != LR_OK) for (int i = 0; i < n_devices; i++) { cudaSetDevice(m->devices[i]); cudaDeviceSynchronize(); }   // nothing of this call stays in flight
-  cudaSetDevice(m->home);
-  g_device = m->home;
   lap("stats");
-  if (rc != LR_OK) { g_error = err; return rc; }
+  if (rc != LR_OK) return rc;
   if (stats) *stats = total;
   return LR_OK;
 }
@@ -798,18 +828,15 @@ int lr_multi_render(LrMultiScene* m, const LrRenderParams* p, float* out_rgb, fl
 
 void lr_multi_scene_destroy(LrMultiScene* m) {
   if (!m) return;
-  int prev = 0;
-  cudaGetDevice(&prev);
   for (int i = 0; i < m->n; i++) {
     if (!m->scenes[i] && !m->streams[i] && !m->done[i]) continue;
-    cudaSetDevice(m->devices[i]);
+    const OnDevice on(m->devices[i]);
     cudaDeviceSynchronize();
     if (i == 0 && m->staged) dev_free(m->staged);
     lr_scene_destroy(m->scenes[i]);
     if (m->done[i]) cudaEventDestroy(m->done[i]);
     if (m->streams[i]) cudaStreamDestroy(m->streams[i]);
   }
-  cudaSetDevice(prev);
   delete m;
 }
 
@@ -821,17 +848,13 @@ int lr_render_multi(const LrSceneDesc* desc, const LrRenderParams* p, int32_t n_
   LrMultiScene* m = nullptr;
   if (int rc = lr_multi_scene_create(desc, n_devices, devices, &m)) return rc;
   const int rc = lr_multi_render(m, p, out_rgb, out_sumsq, stats);
-  const std::string err = g_error;
   lr_multi_scene_destroy(m);
-  g_error = err;
   return rc;
 }
 
 int lr_trace_primary(const LrScene* s, float u, float v, float ua, float va, int32_t* prim, float* t) {
-  if (!s) return fail(LR_ERR_INVALID, "null argument");
-  const OnDevice on(s->device);
   if (!s || !prim || !t) return fail(LR_ERR_INVALID, "null argument");
-  if (int rc = ensure_device()) return rc;
+  const OnDevice on(s->device);
   const size_t n = (size_t)s->width * s->height;
   int* d_prim = nullptr; float* d_t = nullptr;
   LR_CUDA(cudaMalloc((void**)&d_prim, n * sizeof(int)));
@@ -851,12 +874,10 @@ int lr_trace_rays(const LrScene* s, int64_t n, const float* origins, const float
 
 int lr_trace_rays_query(const LrScene* s, int64_t n, const float* origins, const float* directions, int32_t query, int32_t* prim, float* t,
                         float* normal) {
-  if (!s) return fail(LR_ERR_INVALID, "bad argument");
-  const OnDevice on(s->device);
   if (!s || !origins || !directions || !prim || !t || n < 0) return fail(LR_ERR_INVALID, "bad argument");
+  const OnDevice on(s->device);
   if (query != LR_QUERY_STRICT && query != LR_QUERY_RENDER) return fail(LR_ERR_INVALID, "unknown query kind");
   if (n == 0) return LR_OK;
-  if (int rc = ensure_device()) return rc;
   float *d_o = nullptr, *d_d = nullptr, *d_t = nullptr, *d_n = nullptr; int* d_p = nullptr;
   cudaError_t e = cudaMalloc((void**)&d_o, n * 3 * sizeof(float));
   if (e == cudaSuccess) e = cudaMalloc((void**)&d_d, n * 3 * sizeof(float));
@@ -877,14 +898,45 @@ int lr_trace_rays_query(const LrScene* s, int64_t n, const float* origins, const
 // ---------------------------------------------------------------- progressive / resumable rendering (main.rs:81-91)
 }  // extern "C"
 
-struct LrFilm {
-  const LrScene* scene = nullptr;
+// A film: the per-pixel sums (and sums of squares) of a render in progress, and how many sample indices they hold.  It is a
+// list of parts, one per device, each with crop-sized buffers on its scene's device.  The crop's 8x4 tiles are dealt over
+// n_shards shards (device_scene.h: shard_of_tile), shard k renders on part shard_device(k, n_parts), and read / save gather
+// the crop on part 0's device, each pixel from the part that owns it.  Both C handles are this film; what differs is fixed
+// at creation (film_of): an LrFilm is one part on the scene's device and the legacy stream and renders as lr_render does,
+// params->splits included; an LrMultiFilm has a part per device of its LrMultiScene, each on that device's stream, and is
+// sharded: one thread per pixel adds the samples in order (splits = 1), so the bits do not depend on the device count.
+struct Film {
+  struct Part {
+    const LrScene* scene = nullptr;
+    cudaStream_t stream = nullptr;
+    float* d_sum = nullptr;
+    float* d_sumsq = nullptr;
+  };
+  Part parts[kMaxPeers];
+  int n_parts = 1;
+  LrMultiScene* ms = nullptr;            // the peer mappings and staging the gather reads through (null: one part)
+  bool sharded = false;
+  int n_shards = 1;
   LrRenderParams params{};               // spp_begin = first sample index of the film, spp_count unused
   int32_t spp_done = 0;
   int32_t crop_w = 0, crop_h = 0;        // resolved window
-  float* d_sum = nullptr;
-  float* d_sumsq = nullptr;
+  bool has_sumsq = false;
+
+  Film() = default;
+  Film(const Film&) = delete;
+  Film& operator=(const Film&) = delete;
+  ~Film() {
+    for (int i = 0; i < n_parts; i++) {
+      if (!parts[i].d_sum && !parts[i].d_sumsq) continue;
+      const OnDevice on(parts[i].scene->device);
+      cudaDeviceSynchronize();
+      dev_free(parts[i].d_sum);
+      dev_free(parts[i].d_sumsq);
+    }
+  }
 };
+struct LrFilm : Film {};
+struct LrMultiFilm : Film {};
 
 namespace {
 constexpr char kFilmMagic[8] = {'L', 'R', 'F', 'I', 'L', 'M', '1', 0};
@@ -895,32 +947,8 @@ struct FilmHeader {                      // checkpoint file: this header, then c
   uint64_t seed;
 };
 
-// The checkpoint format, shared by LrFilm and LrMultiFilm: a film of either kind saves the same bytes for the same state
-// and loads the other's checkpoints.
-FilmHeader film_header(int film_w, int film_h, const LrRenderParams& p, int32_t crop_w, int32_t crop_h, int32_t spp_done, bool has_sumsq) {
-  FilmHeader h;
-  std::memset(&h, 0, sizeof(h));
-  std::memcpy(h.magic, kFilmMagic, 8);
-  h.film_w = film_w; h.film_h = film_h;
-  h.crop_x = p.crop_w > 0 ? p.crop_x : 0; h.crop_y = p.crop_w > 0 ? p.crop_y : 0; h.crop_w = crop_w; h.crop_h = crop_h;
-  h.integrator = p.integrator; h.depth = p.depth; h.depth_limit = p.depth_limit; h.no_direct_emitter = p.no_direct_emitter;
-  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = spp_done; h.has_sumsq = has_sumsq ? 1 : 0; h.seed = p.seed;
-  return h;
-}
-
-// `data`: the raw sums, then the sums of squares if the header says so
-int film_write(const char* path, const FilmHeader& h, const std::vector<float>& data) {
-  // written next to the target and renamed: a crash mid-write never leaves a torn checkpoint under `path`
-  const std::string tmp = std::string(path) + ".part";
-  FILE* fp = std::fopen(tmp.c_str(), "wb");
-  if (!fp) return fail(LR_ERR_IO, std::string("cannot write `") + tmp + "`");
-  const bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(data.data(), sizeof(float), data.size(), fp) == data.size();
-  const bool closed = std::fclose(fp) == 0;
-  if (!ok || !closed || std::rename(tmp.c_str(), path) != 0) { std::remove(tmp.c_str()); return fail(LR_ERR_IO, std::string("cannot write `") + path + "`"); }
-  return LR_OK;
-}
-
-// reads a checkpoint made for a film_w x film_h film: its header, its data (as film_write) and the parameters to resume with
+// reads a checkpoint made for a film_w x film_h film: its header, its data (the raw sums, then the sums of squares if the
+// header says so) and the parameters to resume with
 int film_read(const char* path, int film_w, int film_h, FilmHeader* hp, std::vector<float>* data, LrRenderParams* params) {
   FILE* fp = std::fopen(path, "rb");
   if (!fp) return fail(LR_ERR_IO, std::string("File `") + path + "` is not found.");
@@ -946,367 +974,185 @@ int film_read(const char* path, int film_w, int film_h, FilmHeader* hp, std::vec
   return LR_OK;
 }
 
-int film_alloc(const LrScene* s, const LrRenderParams* p, int want_sumsq, LrFilm** out) {
-  if (!s) return fail(LR_ERR_INVALID, "null argument");
-  const OnDevice on(s->device);
-  if (!s || !p || !out) return fail(LR_ERR_INVALID, "null argument");
-  *out = nullptr;
-  LrRenderParams probe = *p;
-  probe.spp_count = 1;
-  DevParams dp;
-  if (int rc = resolve_params(s, &probe, dp)) return rc;
-  if (int rc = ensure_device()) return rc;
+LrFilm* film_of(const LrScene* s) {
   LrFilm* f = new LrFilm();
-  f->scene = s; f->params = *p; f->params.spp_count = 0;
-  f->crop_w = dp.crop_w; f->crop_h = dp.crop_h;
-  const size_t bytes = (size_t)dp.crop_w * dp.crop_h * 3 * sizeof(float);
-  cudaError_t e = dev_alloc((void**)&f->d_sum, bytes);
-  if (e == cudaSuccess) e = cudaMemset(f->d_sum, 0, bytes);
-  if (e == cudaSuccess && want_sumsq) e = dev_alloc((void**)&f->d_sumsq, bytes);
-  if (e == cudaSuccess && want_sumsq) e = cudaMemset(f->d_sumsq, 0, bytes);
-  if (e != cudaSuccess) {
-    const std::string msg = std::string("film: ") + cudaGetErrorString(e);
-    lr_film_destroy(f);
-    return fail(LR_ERR_CUDA, msg);
-  }
-  *out = f;
-  return LR_OK;
-}
-}  // namespace
-
-extern "C" {
-
-int lr_film_create(const LrScene* s, const LrRenderParams* p, int32_t want_sumsq, LrFilm** out) { LR_GUARDED(film_alloc(s, p, want_sumsq, out)); }
-
-void lr_film_destroy(LrFilm* f) {
-  if (!f) return;
-  const OnDevice on(f->scene->device);
-  if (!f) return;
-  cudaDeviceSynchronize();
-  dev_free(f->d_sum);
-  dev_free(f->d_sumsq);
-  delete f;
+  f->parts[0].scene = s;
+  return f;
 }
 
-int lr_film_info(const LrFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) {
-  if (!f) return fail(LR_ERR_INVALID, "null argument");
-  if (spp_done) *spp_done = f->spp_done;
-  if (crop_w) *crop_w = f->crop_w;
-  if (crop_h) *crop_h = f->crop_h;
-  if (has_sumsq) *has_sumsq = f->d_sumsq ? 1 : 0;
-  return LR_OK;
-}
-
-int lr_film_render(LrFilm* f, int32_t spp_count, LrStats* stats) {
-  if (!f) return fail(LR_ERR_INVALID, "null argument");
-  if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
-  LrRenderParams q = f->params;
-  q.spp_begin = f->params.spp_begin + f->spp_done;
-  q.spp_count = spp_count;
-  LrStats dummy;
-  if (!stats) stats = &dummy;
-  if (int rc = lr_stats_fetch(f->scene, nullptr, stats)) return rc;       // drop counters of earlier calls
-  if (int rc = lr_render_accumulate_device(f->scene, &q, f->d_sum, f->d_sumsq, nullptr)) return rc;
-  if (int rc = lr_stats_fetch(f->scene, nullptr, stats)) return rc;       // synchronises: the samples are in the film
-  f->spp_done += spp_count;
-  return LR_OK;
-}
-
-int lr_film_read(const LrFilm* f, float* out_rgb, float* out_sumsq) {
-  if (!f) return fail(LR_ERR_INVALID, "null argument");
-  const OnDevice on(f->scene->device);
-  if (!f || !out_rgb) return fail(LR_ERR_INVALID, "null argument");
-  if (out_sumsq && !f->d_sumsq) return fail(LR_ERR_INVALID, "the film was created without sums of squares");
-  if (f->spp_done <= 0) return fail(LR_ERR_INVALID, "the film holds no samples yet");
-  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
-  float* d_tmp = nullptr;
-  LR_CUDA(dev_alloc((void**)&d_tmp, n * sizeof(float)));
-  cudaError_t e = cudaMemcpyAsync(d_tmp, f->d_sum, n * sizeof(float), cudaMemcpyDeviceToDevice, 0);
-  if (e == cudaSuccess) e = launch_scale(d_tmp, n, (float)f->spp_done, 0);            // main.rs:104
-  if (e == cudaSuccess) e = cudaMemcpy(out_rgb, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost);
-  if (e == cudaSuccess && out_sumsq) e = cudaMemcpy(out_sumsq, f->d_sumsq, n * sizeof(float), cudaMemcpyDeviceToHost);
-  dev_free(d_tmp);
-  if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("film read: ") + cudaGetErrorString(e));
-  return LR_OK;
-}
-
-static int film_save_body(const LrFilm* f, const char* path) {
-  if (!f) return fail(LR_ERR_INVALID, "null argument");
-  const OnDevice on(f->scene->device);
-  if (!f || !path) return fail(LR_ERR_INVALID, "null argument");
-  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
-  std::vector<float> host(n * (f->d_sumsq ? 2 : 1));
-  LR_CUDA(cudaMemcpy(host.data(), f->d_sum, n * sizeof(float), cudaMemcpyDeviceToHost));
-  if (f->d_sumsq) LR_CUDA(cudaMemcpy(host.data() + n, f->d_sumsq, n * sizeof(float), cudaMemcpyDeviceToHost));
-  return film_write(path, film_header(f->scene->width, f->scene->height, f->params, f->crop_w, f->crop_h, f->spp_done, f->d_sumsq != nullptr), host);
-}
-int lr_film_save(const LrFilm* f, const char* path) { LR_GUARDED(film_save_body(f, path)); }
-
-static int film_load_body(const LrScene* s, const char* path, LrFilm** out) {
-  if (!s || !path || !out) return fail(LR_ERR_INVALID, "null argument");
-  *out = nullptr;
-  FilmHeader h;
-  std::vector<float> host;
-  LrRenderParams p;
-  int rc = film_read(path, s->width, s->height, &h, &host, &p);
-  if (rc != LR_OK) return rc;
-  LrFilm* f = nullptr;
-  if ((rc = film_alloc(s, &p, h.has_sumsq, &f)) != LR_OK) return rc;
-  const size_t n = (size_t)h.crop_w * h.crop_h * 3;
-  cudaError_t e = cudaMemcpy(f->d_sum, host.data(), n * sizeof(float), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpy(f->d_sumsq, host.data() + n, n * sizeof(float), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) { lr_film_destroy(f); return fail(LR_ERR_CUDA, std::string("film load: ") + cudaGetErrorString(e)); }
-  f->spp_done = h.spp_done;
-  *out = f;
-  return LR_OK;
-}
-int lr_film_load(const LrScene* s, const char* path, LrFilm** out) { LR_GUARDED(film_load_body(s, path, out)); }
-
-// ---------------------------------------------------------------- progressive / resumable rendering on several GPUs
-}  // extern "C"
-
-// A film of an LrMultiScene, sharded by pixel: shard k of n_shards (device_scene.h: shard_of_tile) renders on device
-// shard_device(k, n).  Every device keeps a crop-sized sum buffer but writes only the pixels of its own shards; the image
-// is gathered on devices[0], each pixel from the device that owns it.
-struct LrMultiFilm {
-  LrMultiScene* ms = nullptr;
-  LrRenderParams params{};               // as LrFilm's, with splits = 1
-  int32_t spp_done = 0;
-  int32_t crop_w = 0, crop_h = 0;
-  int n_shards = 1;
-  bool has_sumsq = false;
-  float* d_sum[kMaxPeers] = {};          // on ms->devices[i]
-  float* d_sumsq[kMaxPeers] = {};
-};
-
-namespace {
-
-int use_device(const LrMultiScene* m, int i) {
-  const cudaError_t e = cudaSetDevice(m->devices[i]);
-  if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
-  g_device = m->devices[i];
-  return LR_OK;
-}
-
-// the end of every multi-film call: after a failure nothing of the call stays in flight; the calling thread and the library
-// are back on the multi scene's home device, as lr_multi_render leaves them
-int multi_finish(const LrMultiScene* m, int rc) {
-  const std::string err = g_error;
-  if (rc != LR_OK) for (int i = 0; i < m->n; i++) { cudaSetDevice(m->devices[i]); cudaDeviceSynchronize(); }
-  cudaSetDevice(m->home);
-  g_device = m->home;
-  g_error = err;
-  return rc;
-}
-
-void mfilm_free(LrMultiFilm* f) {
-  const LrMultiScene* m = f->ms;
-  int prev = 0;
-  cudaGetDevice(&prev);
-  for (int i = 0; i < m->n; i++) {
-    if (!f->d_sum[i] && !f->d_sumsq[i]) continue;
-    cudaSetDevice(m->devices[i]);
-    cudaDeviceSynchronize();
-    dev_free(f->d_sum[i]);
-    dev_free(f->d_sumsq[i]);
-  }
-  cudaSetDevice(prev);
-  delete f;
-}
-
-int mfilm_alloc(LrMultiScene* m, const LrRenderParams* p, int want_sumsq, LrMultiFilm** out) {
-  if (!m || !p || !out) return fail(LR_ERR_INVALID, "null argument");
-  *out = nullptr;
-  // the bit-for-bit contract (every pixel's samples added in order from the stored sum) holds for one thread per pixel only
-  if (p->splits != 0 && p->splits != 1) return fail(LR_ERR_INVALID, "a multi-device film renders with splits = 1");
-  LrRenderParams probe = *p;
-  probe.spp_count = 1;
-  const FilmShard whole{0, 1};
-  DevParams dp;
-  if (int rc = resolve_params(m->scenes[0], &probe, dp, &whole)) return rc;
+LrMultiFilm* film_of(LrMultiScene* m) {
   LrMultiFilm* f = new LrMultiFilm();
-  f->ms = m; f->params = *p; f->params.spp_count = 0; f->params.splits = 1;
-  f->crop_w = dp.crop_w; f->crop_h = dp.crop_h; f->has_sumsq = want_sumsq != 0;
+  f->n_parts = m->n;
+  for (int i = 0; i < m->n; i++) { f->parts[i].scene = m->scenes[i]; f->parts[i].stream = m->streams[i]; }
+  f->ms = m;
+  f->sharded = true;
   f->n_shards = m->n;
   // LR_FILM_SHARDS=S (development / tests): S shards over the devices, so that one GPU runs the interleaved kernels too
   if (const char* e_shards = std::getenv("LR_FILM_SHARDS")) f->n_shards = std::max(1, std::atoi(e_shards));
+  return f;
+}
+
+// the rest of a film's creation: its parameters, its window and zeroed buffers on every part
+int film_setup(Film* f, const LrRenderParams& p, int want_sumsq) {
+  // the bit-for-bit contract of a sharded film (every pixel's samples added in order from the stored sum) holds for one
+  // thread per pixel only
+  if (f->sharded && p.splits != 0 && p.splits != 1) return fail(LR_ERR_INVALID, "a multi-device film renders with splits = 1");
+  LrRenderParams probe = p;
+  probe.spp_count = 1;
+  DevParams dp;
+  if (int rc = resolve_params(f->parts[0].scene, &probe, dp)) return rc;
+  f->params = p; f->params.spp_count = 0;
+  if (f->sharded) f->params.splits = 1;
+  f->crop_w = dp.crop_w; f->crop_h = dp.crop_h; f->has_sumsq = want_sumsq != 0;
   const size_t bytes = (size_t)dp.crop_w * dp.crop_h * 3 * sizeof(float);
   int rc = LR_OK;
-  for (int i = 0; i < m->n && rc == LR_OK; i++) {
-    if ((rc = use_device(m, i)) != LR_OK) break;
-    cudaError_t e = dev_alloc((void**)&f->d_sum[i], bytes);
-    if (e == cudaSuccess) e = cudaMemsetAsync(f->d_sum[i], 0, bytes, 0);
-    if (e == cudaSuccess && want_sumsq) e = dev_alloc((void**)&f->d_sumsq[i], bytes);
-    if (e == cudaSuccess && want_sumsq) e = cudaMemsetAsync(f->d_sumsq[i], 0, bytes, 0);
+  OnDevices on(rc);
+  for (int i = 0; i < f->n_parts && rc == LR_OK; i++) {
+    Film::Part& part = f->parts[i];
+    if ((rc = on.use(part.scene->device)) != LR_OK) break;
+    cudaError_t e = dev_alloc((void**)&part.d_sum, bytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(part.d_sum, 0, bytes, 0);
+    if (e == cudaSuccess && want_sumsq) e = dev_alloc((void**)&part.d_sumsq, bytes);
+    if (e == cudaSuccess && want_sumsq) e = cudaMemsetAsync(part.d_sumsq, 0, bytes, 0);
     if (e == cudaSuccess) e = cudaStreamSynchronize(0);       // the render streams do not order against the legacy stream
-    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("film: ") + cudaGetErrorString(e));
   }
-  if ((rc = multi_finish(m, rc)) != LR_OK) {
-    const std::string err = g_error;
-    mfilm_free(f);
-    g_error = err;
-    return rc;
-  }
-  *out = f;
+  return rc;
+}
+
+// Owner: the LrScene of an LrFilm or the LrMultiScene of an LrMultiFilm
+template <class Owner, class Handle>
+int film_create(Owner* o, const LrRenderParams* p, int want_sumsq, Handle** out) {
+  if (!o || !p || !out) return fail(LR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  std::unique_ptr<Handle> f(film_of(o));
+  if (int rc = film_setup(f.get(), *p, want_sumsq)) return rc;
+  *out = f.release();
   return LR_OK;
 }
 
-int mfilm_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) {
+template <class Owner, class Handle>
+int film_load(Owner* o, const char* path, Handle** out) {
+  if (!o || !path || !out) return fail(LR_ERR_INVALID, "null argument");
+  *out = nullptr;
+  std::unique_ptr<Handle> f(film_of(o));
+  const Film::Part& p0 = f->parts[0];
+  FilmHeader h;
+  std::vector<float> host;
+  LrRenderParams p;
+  if (int rc = film_read(path, p0.scene->width, p0.scene->height, &h, &host, &p)) return rc;
+  if (f->sharded && h.splits != 1) return fail(LR_ERR_INVALID, "the checkpoint was rendered with splits != 1; a multi-device film adds samples in order");
+  if (int rc = film_setup(f.get(), p, h.has_sumsq)) return rc;
+  // the sums go to part 0, and from there to every other part
+  const size_t bytes = (size_t)h.crop_w * h.crop_h * 3 * sizeof(float);
+  int rc = LR_OK;
+  OnDevices on(rc);
+  if ((rc = on.use(p0.scene->device)) != LR_OK) return rc;
+  cudaError_t e = cudaMemcpyAsync(p0.d_sum, host.data(), bytes, cudaMemcpyHostToDevice, p0.stream);
+  if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyAsync(p0.d_sumsq, host.data() + bytes / sizeof(float), bytes, cudaMemcpyHostToDevice, p0.stream);
+  for (int i = 1; i < f->n_parts && e == cudaSuccess; i++) {
+    const Film::Part& part = f->parts[i];
+    e = cudaMemcpyPeerAsync(part.d_sum, part.scene->device, p0.d_sum, p0.scene->device, bytes, p0.stream);
+    if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyPeerAsync(part.d_sumsq, part.scene->device, p0.d_sumsq, p0.scene->device, bytes, p0.stream);
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(p0.stream);
+  if (e != cudaSuccess) return rc = fail(LR_ERR_CUDA, std::string("film load: ") + cudaGetErrorString(e));
+  f->spp_done = h.spp_done;
+  *out = f.release();
+  return LR_OK;
+}
+
+int film_render(Film* f, int32_t spp_count, LrStats* stats) {
   if (!f) return fail(LR_ERR_INVALID, "null argument");
   if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
-  LrMultiScene* m = f->ms;
   LrRenderParams q = f->params;
   q.spp_begin = f->params.spp_begin + f->spp_done;
   q.spp_count = spp_count;
   LrStats total;
   std::memset(&total, 0, sizeof(total));
   int rc = LR_OK;
-  do {
-    for (int i = 0; i < m->n && rc == LR_OK; i++) {          // drop the counters of earlier calls
-      LrStats dropped;
-      if ((rc = use_device(m, i)) == LR_OK) rc = lr_stats_fetch(m->scenes[i], m->streams[i], &dropped);
-    }
-    if (rc != LR_OK) break;
-    // launch: asynchronous on every device's own stream, so the devices render concurrently; a device with several shards
-    // renders them one after the other (disjoint pixels of the same buffer)
-    for (int k = 0; k < f->n_shards && rc == LR_OK; k++) {
-      const int i = shard_device(k, m->n);
-      const FilmShard shard{k, f->n_shards};
-      if ((rc = use_device(m, i)) == LR_OK) rc = accumulate(m->scenes[i], &q, f->d_sum[i], f->d_sumsq[i], m->streams[i], &shard);
-    }
-    if (rc != LR_OK) break;
-    // wait for every device; statistics are totals, kernel_ms the slowest device's
-    for (int i = 0; i < m->n && rc == LR_OK; i++) {
-      LrStats st;
-      if ((rc = use_device(m, i)) != LR_OK || (rc = lr_stats_fetch(m->scenes[i], m->streams[i], &st)) != LR_OK) break;
-      add_device_stats(total, st);
-    }
-  } while (0);
-  if ((rc = multi_finish(m, rc)) != LR_OK) return rc;
+  OnDevices on(rc);
+  for (int i = 0; i < f->n_parts && rc == LR_OK; i++) {     // drop the counters of earlier calls
+    LrStats dropped;
+    if ((rc = on.use(f->parts[i].scene->device)) == LR_OK) rc = lr_stats_fetch(f->parts[i].scene, f->parts[i].stream, &dropped);
+  }
+  // launch: asynchronous on every part's stream, so the devices render concurrently; a part with several shards renders
+  // them one after the other (disjoint pixels of the same buffer)
+  for (int k = 0; k < f->n_shards && rc == LR_OK; k++) {
+    const Film::Part& part = f->parts[shard_device(k, f->n_parts)];
+    const FilmShard shard{k, f->n_shards};
+    rc = accumulate(part.scene, &q, part.d_sum, part.d_sumsq, part.stream, f->sharded ? &shard : nullptr);
+  }
+  // wait for every part: the samples are in the film; statistics are totals, kernel_ms the slowest device's
+  for (int i = 0; i < f->n_parts && rc == LR_OK; i++) {
+    LrStats st;
+    if ((rc = lr_stats_fetch(f->parts[i].scene, f->parts[i].stream, &st)) == LR_OK) add_device_stats(total, st);
+  }
+  if (rc != LR_OK) return rc;
   f->spp_done += spp_count;
   if (stats) *stats = total;
   return LR_OK;
 }
 
-// The film's crop on devices[0] into dst (device memory there): each pixel from the buffer of the device that owns it
-// (`bufs`: one per device), read over NVLink where devices[0] maps the peer and from a staged copy where it does not;
-// divided by `divisor` if it is > 0.  Asynchronous on devices[0]'s stream; the caller has made devices[0] current.
-int mfilm_gather(const LrMultiFilm* f, float* const* bufs, float* dst, float divisor) {
-  LrMultiScene* m = f->ms;
+// The crop gathered on part 0's device, each pixel from the part that owns it (read over NVLink where that device maps the
+// part's device, from a staged copy where it does not), to host memory: the sums divided by `divisor` if it is > 0, and
+// the sums of squares too if out_sumsq is not null.
+int film_download(const Film* f, float divisor, float* out, float* out_sumsq) {
+  const Film::Part& p0 = f->parts[0];
   const size_t n = (size_t)f->crop_w * f->crop_h * 3;
-  cudaStream_t st0 = m->streams[0];
-  size_t need_staged = 0;
-  for (int i = 1; i < m->n; i++) if (!m->mapped[i]) need_staged += n;
-  cudaError_t e = cudaSuccess;
-  if (need_staged > m->staged_floats) {
-    e = cudaStreamSynchronize(st0);                           // an earlier gather may still read the old staging buffer
-    if (e == cudaSuccess) {
-      dev_free(m->staged);
-      m->staged = nullptr; m->staged_floats = 0;
-      e = dev_alloc((void**)&m->staged, need_staged * sizeof(float));
-      if (e == cudaSuccess) m->staged_floats = need_staged;
-    }
-  }
-  PeerBuffers src;
-  src.count = m->n;
-  float* stage_next = m->staged;
-  for (int i = 0; i < m->n && e == cudaSuccess; i++) {
-    src.p[i] = bufs[i];
-    if (!m->mapped[i]) {
-      e = cudaMemcpyPeerAsync(stage_next, m->devices[0], bufs[i], m->devices[i], n * sizeof(float), st0);
-      src.p[i] = stage_next;
-      stage_next += n;
-    }
-  }
-  if (e == cudaSuccess) e = launch_gather_shards(dst, src, f->crop_w, f->crop_h, f->n_shards, divisor, st0);
-  if (e != cudaSuccess) return fail(LR_ERR_CUDA, std::string("multi film gather: ") + cudaGetErrorString(e));
-  return LR_OK;
-}
-
-// the gathered sums (sums of squares after them if asked for) or the mean, to host memory
-int mfilm_download(const LrMultiFilm* f, float divisor, float* out, float* out_sumsq) {
-  const LrMultiScene* m = f->ms;
-  const size_t n = (size_t)f->crop_w * f->crop_h * 3;
-  int rc = use_device(m, 0);
+  int rc = LR_OK;
+  OnDevices on(rc);
+  if ((rc = on.use(p0.scene->device)) != LR_OK) return rc;
   float* d_tmp = nullptr;
-  cudaError_t e = cudaSuccess;
-  if (rc == LR_OK) {
-    e = dev_alloc((void**)&d_tmp, n * sizeof(float));
-    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film: ") + cudaGetErrorString(e));
+  cudaError_t e = dev_alloc((void**)&d_tmp, n * sizeof(float));
+  for (int sq = 0; sq < (out_sumsq ? 2 : 1) && e == cudaSuccess; sq++) {
+    float* bufs[kMaxPeers];
+    for (int i = 0; i < f->n_parts; i++) bufs[i] = sq ? f->parts[i].d_sumsq : f->parts[i].d_sum;
+    PeerBuffers src;
+    e = peer_buffers(f->ms, f->n_parts, bufs, n, p0.stream, &src);
+    if (e == cudaSuccess) e = launch_gather_shards(d_tmp, src, f->crop_w, f->crop_h, f->n_shards, sq ? 0.0f : divisor, p0.stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(sq ? out_sumsq : out, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, p0.stream);
   }
-  if (rc == LR_OK && (rc = mfilm_gather(f, f->d_sum, d_tmp, divisor)) == LR_OK) {
-    e = cudaMemcpyAsync(out, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, m->streams[0]);
-    if (e == cudaSuccess && out_sumsq && (rc = mfilm_gather(f, f->d_sumsq, d_tmp, 0.0f)) == LR_OK)
-      e = cudaMemcpyAsync(out_sumsq, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, m->streams[0]);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(m->streams[0]);
-    if (rc == LR_OK && e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film D2H: ") + cudaGetErrorString(e));
-  }
-  if (d_tmp) { if (rc != LR_OK) cudaStreamSynchronize(m->streams[0]); dev_free(d_tmp); }
-  return multi_finish(m, rc);
+  const cudaError_t done = cudaStreamSynchronize(p0.stream);   // before d_tmp goes back to the pool, on failure too
+  if (e == cudaSuccess) e = done;
+  dev_free(d_tmp);
+  if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("film read: ") + cudaGetErrorString(e));
+  return rc;
 }
 
-int mfilm_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) {
+int film_read_mean(const Film* f, float* out_rgb, float* out_sumsq) {
   if (!f || !out_rgb) return fail(LR_ERR_INVALID, "null argument");
   if (out_sumsq && !f->has_sumsq) return fail(LR_ERR_INVALID, "the film was created without sums of squares");
   if (f->spp_done <= 0) return fail(LR_ERR_INVALID, "the film holds no samples yet");
-  return mfilm_download(f, (float)f->spp_done, out_rgb, out_sumsq);   // main.rs:104, as lr_film_read
+  return film_download(f, (float)f->spp_done, out_rgb, out_sumsq);   // main.rs:104
 }
 
-int mfilm_save(const LrMultiFilm* f, const char* path) {
+// The checkpoint: a film saves the same bytes for the same state through either handle, and each handle loads the other's.
+int film_save(const Film* f, const char* path) {
   if (!f || !path) return fail(LR_ERR_INVALID, "null argument");
   const size_t n = (size_t)f->crop_w * f->crop_h * 3;
-  std::vector<float> host(n * (f->has_sumsq ? 2 : 1));
-  if (int rc = mfilm_download(f, 0.0f, host.data(), f->has_sumsq ? host.data() + n : nullptr)) return rc;
-  const LrScene* s0 = f->ms->scenes[0];
-  return film_write(path, film_header(s0->width, s0->height, f->params, f->crop_w, f->crop_h, f->spp_done, f->has_sumsq), host);
-}
-
-int mfilm_load(LrMultiScene* m, const char* path, LrMultiFilm** out) {
-  if (!m || !path || !out) return fail(LR_ERR_INVALID, "null argument");
-  *out = nullptr;
+  std::vector<float> data(n * (f->has_sumsq ? 2 : 1));
+  if (int rc = film_download(f, 0.0f, data.data(), f->has_sumsq ? data.data() + n : nullptr)) return rc;
+  const LrScene* s0 = f->parts[0].scene;
+  const LrRenderParams& p = f->params;
   FilmHeader h;
-  std::vector<float> host;
-  LrRenderParams p;
-  int rc = film_read(path, m->scenes[0]->width, m->scenes[0]->height, &h, &host, &p);
-  if (rc != LR_OK) return rc;
-  if (h.splits != 1) return fail(LR_ERR_INVALID, "the checkpoint was rendered with splits != 1; a multi-device film adds samples in order");
-  LrMultiFilm* f = nullptr;
-  if ((rc = mfilm_alloc(m, &p, h.has_sumsq, &f)) != LR_OK) return rc;
-  // the sums go to devices[0], and from there to every other device
-  const size_t bytes = (size_t)h.crop_w * h.crop_h * 3 * sizeof(float);
-  cudaStream_t st0 = m->streams[0];
-  rc = use_device(m, 0);
-  cudaError_t e = cudaSuccess;
-  if (rc == LR_OK) {
-    e = cudaMemcpyAsync(f->d_sum[0], host.data(), bytes, cudaMemcpyHostToDevice, st0);
-    if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyAsync(f->d_sumsq[0], host.data() + bytes / sizeof(float), bytes, cudaMemcpyHostToDevice, st0);
-    for (int i = 1; i < m->n && e == cudaSuccess; i++) {
-      e = cudaMemcpyPeerAsync(f->d_sum[i], m->devices[i], f->d_sum[0], m->devices[0], bytes, st0);
-      if (e == cudaSuccess && h.has_sumsq) e = cudaMemcpyPeerAsync(f->d_sumsq[i], m->devices[i], f->d_sumsq[0], m->devices[0], bytes, st0);
-    }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st0);
-    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("multi film load: ") + cudaGetErrorString(e));
-  }
-  if ((rc = multi_finish(m, rc)) != LR_OK) {
-    const std::string err = g_error;
-    mfilm_free(f);
-    g_error = err;
-    return rc;
-  }
-  f->spp_done = h.spp_done;
-  *out = f;
+  std::memset(&h, 0, sizeof(h));
+  std::memcpy(h.magic, kFilmMagic, 8);
+  h.film_w = s0->width; h.film_h = s0->height;
+  h.crop_x = p.crop_w > 0 ? p.crop_x : 0; h.crop_y = p.crop_w > 0 ? p.crop_y : 0; h.crop_w = f->crop_w; h.crop_h = f->crop_h;
+  h.integrator = p.integrator; h.depth = p.depth; h.depth_limit = p.depth_limit; h.no_direct_emitter = p.no_direct_emitter;
+  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = f->spp_done; h.has_sumsq = f->has_sumsq ? 1 : 0; h.seed = p.seed;
+  // written next to the target and renamed: a crash mid-write never leaves a torn checkpoint under `path`
+  const std::string tmp = std::string(path) + ".part";
+  FILE* fp = std::fopen(tmp.c_str(), "wb");
+  if (!fp) return fail(LR_ERR_IO, std::string("cannot write `") + tmp + "`");
+  const bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(data.data(), sizeof(float), data.size(), fp) == data.size();
+  const bool closed = std::fclose(fp) == 0;
+  if (!ok || !closed || std::rename(tmp.c_str(), path) != 0) { std::remove(tmp.c_str()); return fail(LR_ERR_IO, std::string("cannot write `") + path + "`"); }
   return LR_OK;
 }
 
-}  // namespace
-
-extern "C" {
-
-int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* p, int32_t want_sumsq, LrMultiFilm** out) {
-  LR_GUARDED(mfilm_alloc(ms, p, want_sumsq, out));
-}
-int lr_multi_film_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(mfilm_render(f, spp_count, stats)); }
-int lr_multi_film_info(const LrMultiFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) {
+int film_info(const Film* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) {
   if (!f) return fail(LR_ERR_INVALID, "null argument");
   if (spp_done) *spp_done = f->spp_done;
   if (crop_w) *crop_w = f->crop_w;
@@ -1314,12 +1160,25 @@ int lr_multi_film_info(const LrMultiFilm* f, int32_t* spp_done, int32_t* crop_w,
   if (has_sumsq) *has_sumsq = f->has_sumsq ? 1 : 0;
   return LR_OK;
 }
-int lr_multi_film_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(mfilm_read(f, out_rgb, out_sumsq)); }
-int lr_multi_film_save(const LrMultiFilm* f, const char* path) { LR_GUARDED(mfilm_save(f, path)); }
-int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out) { LR_GUARDED(mfilm_load(ms, path, out)); }
-void lr_multi_film_destroy(LrMultiFilm* f) {
-  if (f) mfilm_free(f);
-}
+}  // namespace
+
+extern "C" {
+
+int lr_film_create(const LrScene* s, const LrRenderParams* p, int32_t want_sumsq, LrFilm** out) { LR_GUARDED(film_create(s, p, want_sumsq, out)); }
+int lr_film_render(LrFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(film_render(f, spp_count, stats)); }
+int lr_film_info(const LrFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) { return film_info(f, spp_done, crop_w, crop_h, has_sumsq); }
+int lr_film_read(const LrFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(film_read_mean(f, out_rgb, out_sumsq)); }
+int lr_film_save(const LrFilm* f, const char* path) { LR_GUARDED(film_save(f, path)); }
+int lr_film_load(const LrScene* s, const char* path, LrFilm** out) { LR_GUARDED(film_load(s, path, out)); }
+void lr_film_destroy(LrFilm* f) { delete f; }
+
+int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* p, int32_t want_sumsq, LrMultiFilm** out) { LR_GUARDED(film_create(ms, p, want_sumsq, out)); }
+int lr_multi_film_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(film_render(f, spp_count, stats)); }
+int lr_multi_film_info(const LrMultiFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) { return film_info(f, spp_done, crop_w, crop_h, has_sumsq); }
+int lr_multi_film_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(film_read_mean(f, out_rgb, out_sumsq)); }
+int lr_multi_film_save(const LrMultiFilm* f, const char* path) { LR_GUARDED(film_save(f, path)); }
+int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out) { LR_GUARDED(film_load(ms, path, out)); }
+void lr_multi_film_destroy(LrMultiFilm* f) { delete f; }
 
 static int measure_read(uint64_t bytes, int iters, int warm, float* gbs) {
   if (!gbs || bytes < (1u << 20) || iters <= 0) return fail(LR_ERR_INVALID, "bad argument");

@@ -6,9 +6,9 @@
 //
 // Extra, optional arguments (not in the reference):  --spp N  --resolution WxH  --seed S  --device D
 //   --gpus N (render on devices D..D+N-1 of this box from this one process: lr_render_multi, samples sharded by index;
-//   with --progress an LrMultiFilm, pixels sharded by tile, whose checkpoints resume under any other --gpus)
+//   with --progress the film is sharded by pixel tile, and its checkpoints resume under any other --gpus)
 //   --assets DIR (root that mesh/IBL paths are resolved against; default: the current directory, like the reference)
-//   --progress N (render N samples per pixel at a time through an LrFilm and print the progress line main.rs:81-91 left
+//   --progress N (render N samples per pixel at a time through an LrMultiFilm and print the progress line main.rs:81-91 left
 //   commented out)  --checkpoint FILE (with --progress: the film is saved after every chunk, and an existing FILE is
 //   resumed — bit for bit the image of an uninterrupted run)  --aov normal|depth (Scene::normal / Scene::depth,
 //   scene.rs:48-62, instead of the radiance; depth is written normalised to its maximum)
@@ -88,8 +88,9 @@ int main(int argc, char** argv) {
   std::printf("polygons: %d\n", cfg.n_prims);                                   // description.rs:66
   std::printf("bvh construction: %gs\n", cfg.bvh_build_seconds);                 // description.rs:70-73
 
+  const bool film = progress > 0 && !aov;
   LrScene* scene = nullptr;
-  if (gpus <= 1 && lr_scene_create(lr_host_scene_desc(hs), &scene) != LR_OK) return die("uploading scene");
+  if (gpus <= 1 && !film && lr_scene_create(lr_host_scene_desc(hs), &scene) != LR_OK) return die("uploading scene");
   LrRenderParams p;
   std::memset(&p, 0, sizeof(p));
   p.integrator = cfg.integrator; p.spp_begin = 0; p.spp_count = cfg.samples;
@@ -97,7 +98,7 @@ int main(int argc, char** argv) {
   std::vector<float> img((size_t)cfg.width * cfg.height * 3);
   LrStats st;
   int32_t devices[8];
-  for (int i = 0; i < gpus && i < 8; i++) devices[i] = device + i;
+  for (int i = 0; i < 8; i++) devices[i] = device + i;
   if (gpus > 1 && progress <= 0) {
     std::printf("gpus: %d (devices %d..%d, samples sharded by index, one peer-reading reduce)\n", gpus, device, device + gpus - 1);
     if (lr_render_multi(lr_host_scene_desc(hs), &p, gpus, devices, img.data(), nullptr, &st) != LR_OK) return die("rendering");
@@ -113,39 +114,34 @@ int main(int argc, char** argv) {
       for (size_t i = 0; i < buf.size(); i++) img[3 * i] = img[3 * i + 1] = img[3 * i + 2] = mx > 0.0f ? buf[i] / mx : 0.0f;
     }
     std::printf("aov: %s\n", aov);
-  } else if (progress > 0) {
-    // the progress hook of main.rs:81-91 (chunks of samples instead of pixels), resumable through a checkpoint file; on
-    // several GPUs the film is sharded by pixel, and both film kinds write and read the same checkpoints
+  } else if (film) {
+    // the progress hook of main.rs:81-91 (chunks of samples instead of pixels), resumable through a checkpoint file; the
+    // film is sharded by pixel over the devices, so its image and its checkpoints do not depend on --gpus
     p.splits = 1;                                             // samples are added in order: any cut of the range gives the same bits
-    LrFilm* film = nullptr;
     LrMultiScene* ms = nullptr;
     LrMultiFilm* mfilm = nullptr;
-    if (gpus > 1) {
-      std::printf("gpus: %d (devices %d..%d, pixels sharded by tile)\n", gpus, device, device + gpus - 1);
-      if (lr_multi_scene_create(lr_host_scene_desc(hs), gpus, devices, &ms) != LR_OK) return die("uploading scene");
-    }
+    if (gpus > 1) std::printf("gpus: %d (devices %d..%d, pixels sharded by tile)\n", gpus, device, device + gpus - 1);
+    if (lr_multi_scene_create(lr_host_scene_desc(hs), gpus > 1 ? gpus : 1, devices, &ms) != LR_OK) return die("uploading scene");
     struct stat sb;
     if (checkpoint && stat(checkpoint, &sb) == 0) {
-      if ((ms ? lr_multi_film_load(ms, checkpoint, &mfilm) : lr_film_load(scene, checkpoint, &film)) != LR_OK) return die("resuming the checkpoint");
-    } else if ((ms ? lr_multi_film_create(ms, &p, 0, &mfilm) : lr_film_create(scene, &p, 0, &film)) != LR_OK) return die("creating the film");
+      if (lr_multi_film_load(ms, checkpoint, &mfilm) != LR_OK) return die("resuming the checkpoint");
+    } else if (lr_multi_film_create(ms, &p, 0, &mfilm) != LR_OK) return die("creating the film");
     int32_t done = 0;
-    if (ms) lr_multi_film_info(mfilm, &done, nullptr, nullptr, nullptr);
-    else lr_film_info(film, &done, nullptr, nullptr, nullptr);
+    lr_multi_film_info(mfilm, &done, nullptr, nullptr, nullptr);
     if (done > 0) std::printf("resuming: %d of %d spp are in %s\n", done, cfg.samples, checkpoint);
     std::memset(&st, 0, sizeof(st));
     while (done < cfg.samples) {
       const int n = cfg.samples - done < progress ? cfg.samples - done : progress;
       LrStats part;
-      if ((ms ? lr_multi_film_render(mfilm, n, &part) : lr_film_render(film, n, &part)) != LR_OK) return die("rendering");
+      if (lr_multi_film_render(mfilm, n, &part) != LR_OK) return die("rendering");
       done += n;
       st.kernel_ms += part.kernel_ms; st.samples += part.samples; st.rays += part.rays; st.nonfinite_samples += part.nonfinite_samples;
-      if (checkpoint && (ms ? lr_multi_film_save(mfilm, checkpoint) : lr_film_save(film, checkpoint)) != LR_OK) return die("writing the checkpoint");
+      if (checkpoint && lr_multi_film_save(mfilm, checkpoint) != LR_OK) return die("writing the checkpoint");
       std::printf("\rprocessing... (%d/%d : %.0f%%) ", done, cfg.samples, 100.0 * done / cfg.samples);
       std::fflush(stdout);
     }
     std::printf("\n");
-    if ((ms ? lr_multi_film_read(mfilm, img.data(), nullptr) : lr_film_read(film, img.data(), nullptr)) != LR_OK) return die("reading the film");
-    lr_film_destroy(film);
+    if (lr_multi_film_read(mfilm, img.data(), nullptr) != LR_OK) return die("reading the film");
     lr_multi_film_destroy(mfilm);
     lr_multi_scene_destroy(ms);
   } else if (lr_render(scene, &p, img.data(), nullptr, &st) != LR_OK) return die("rendering");

@@ -63,7 +63,7 @@ def test_cli_renders_and_writes_the_image(cli, tmp_path):
 
 @pytest.mark.gpu
 def test_cli_progress_checkpoint_resume_and_aov(cli, tmp_path):
-    """--progress renders in chunks through an LrFilm and prints the reference's abandoned progress line (main.rs:81-91);
+    """--progress renders in chunks through a film on the devices of --gpus (here one) and prints the reference's abandoned progress line (main.rs:81-91);
     an interrupted run (here: a first run asked for 4 of the 8 spp) resumed from its checkpoint writes byte for byte the
     PNG of an uninterrupted one; --aov writes Scene::normal / Scene::depth (scene.rs:48-62)."""
     scene = os.path.join(ROOT, "scenes", "primitive.toml")

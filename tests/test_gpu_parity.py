@@ -496,6 +496,20 @@ def test_resumable_render_equals_one_pass_bit_for_bit(scenes, lr, name, tmp_path
     assert np.array_equal(cf2.read(), ref[4:28, 8:48], equal_nan=True)
 
 
+@pytest.mark.parametrize("name", ["new-cbox", "sample"])
+def test_film_honours_splits(scenes, name):
+    """A film of one scene renders with the splits it was created with, as lr_render does: one call with splits = 4 gives
+    lr_render's image, sums of squares and ray count bit for bit."""
+    d, s, o = scenes(name)
+    ref, ref_sq, st = s.render(spp=8, seed=9, splits=4, sumsq=True)
+    film = s.film(sumsq=True, seed=9, splits=4)
+    fst = film.render(8)
+    img, sq = film.read(sumsq=True)
+    film.close()
+    assert st["splits"] == 4 and fst["splits"] == 4 and fst["rays"] == st["rays"] and fst["samples"] == st["samples"]
+    assert np.array_equal(img.view(np.uint32), ref.view(np.uint32)) and np.array_equal(sq.view(np.uint32), ref_sq.view(np.uint32))
+
+
 def test_film_error_paths(scenes, lr, tmp_path):
     from lumillyrender_b200.capi import LumillyError
     d, s, o = scenes("new-cbox")

@@ -224,6 +224,46 @@ def test_two_or_more_devices(scenes, lr, monkeypatch, no_peer, tmp_path):
         one.close()
 
 
+@pytest.mark.gpu
+def test_multi_device_calls_keep_the_callers_device(scenes, lr, tmp_path):
+    """Calls on a multi scene switch devices as they work, then give the calling thread its device back and leave the
+    library's device (lr_init) alone: after them a new scene still lands on the device the caller chose."""
+    torch = pytest.importorskip("torch")
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    _, _, ms = scenes("sample")                       # the multi scene lives on [0]
+    ck = str(tmp_path / "film.ck")
+    lr.init(1)
+    try:
+        def still_on_1(after):
+            assert torch.cuda.current_device() == 1, after
+        ms.render(spp=1, seed=3)
+        still_on_1("render")
+        film = ms.film(seed=3, splits=1)
+        still_on_1("film create")
+        film.render(1)
+        still_on_1("film render")
+        film.read()
+        still_on_1("film read")
+        film.save(ck)
+        still_on_1("film save")
+        film.close()
+        ms.load_film(ck).close()
+        still_on_1("film load")
+        # the pool never trims, so device 1's free memory shows where a new scene and its film buffers go: two buffers of
+        # 126 MB at 3840x2740, more than the earlier tests left in device 1's pool
+        w, h = 3840, 2740
+        big = load_scene(lr, "new-cbox", (w, h))
+        free = torch.cuda.mem_get_info(1)[0]
+        s1 = big.scene()
+        s1.render(spp=1, seed=3, sumsq=True)
+        assert free - torch.cuda.mem_get_info(1)[0] >= w * h * 3 * 4
+        still_on_1("a render of a new scene")
+        s1.close()
+    finally:
+        lr.init(0)
+
+
 @pytest.fixture(scope="module")
 def cli(lr, assets):
     from lumillyrender_b200 import build
