@@ -456,8 +456,8 @@ static int accumulate(const LrScene* s, const LrRenderParams* p, float* d_sum, f
     // the unit cursor lives in the last word of the counter block (reset on the stream before every launch)
     unsigned int* next_unit = reinterpret_cast<unsigned int*>(s->d_counters + C_NEXT_UNIT);
     LR_CUDA(cudaMemsetAsync(next_unit, 0, sizeof(unsigned long long), st));
-    LR_CUDA(launch_render_persistent(s->dev, dp, s->has_ggx, p->count_traversal != 0, ksum, d_sumsq ? ksq : nullptr, s->d_counters, next_unit,
-                                     std::max(s->sm_count, 1), st));
+    LR_CUDA(launch_render(s->dev, dp, s->has_ggx, p->count_traversal != 0, ksum, d_sumsq ? ksq : nullptr, s->d_counters, next_unit,
+                          std::max(s->sm_count, 1), st));
     s->acc_launches++;
   }
   if (dp.splits > 1) {
@@ -552,9 +552,9 @@ int lr_render_aov(const LrScene* s, const LrRenderParams* p, int32_t kind, float
 int lr_shard_range(int32_t spp_begin, int32_t spp_count, int32_t part, int32_t n_parts, int32_t* begin, int32_t* count) {
   if (!begin || !count) return fail(LR_ERR_INVALID, "null argument");
   if (n_parts <= 0 || part < 0 || part >= n_parts || spp_count < 0 || spp_begin < 0) return fail(LR_ERR_INVALID, "bad shard request");
-  const int per = spp_count / n_parts, rem = spp_count % n_parts;
-  *begin = spp_begin + part * per + std::min(part, rem);
-  *count = per + (part < rem ? 1 : 0);
+  const SampleRange r = range_part(spp_begin, spp_count, part, n_parts);
+  *begin = r.begin;
+  *count = r.count;
   return LR_OK;
 }
 

@@ -332,6 +332,11 @@ LR_DEV void flat_hits(const DevScene& sc, const FlatList fl, F3 o, F3 d, F3 inv,
   }
 }
 
+// Where a tree query starts culling, given the nearest hit t found before it (3e38: none): a primitive's computed t may
+// precede its box's computed entry, so boxes are culled a little beyond t
+LR_DEV float cull_distance(float t) { return t < 3.0e38f ? t * 1.0001f + 1e-4f : 3.0e38f; }
+constexpr int kTravDone = (int)0x80000000;       // end of a traversal stack: not a valid leaf code (first triangle would be 2^28 - 1)
+
 // conservative: can the ray reach the tree's bounds within [0, cull_t]?  (same padded-box form as the node test)
 LR_DEV bool bvh_bounds_hit(const DevScene& sc, F3 o, F3 inv, float cull_t) {
   const float ax = (sc.bvh_lo[0] - o.x) * inv.x, bx = (sc.bvh_hi[0] - o.x) * inv.x;
@@ -341,6 +346,8 @@ LR_DEV bool bvh_bounds_hit(const DevScene& sc, F3 o, F3 inv, float cull_t) {
   const float ex = fminf(fminf(fmaxf(ax, bx), fmaxf(ay, by)), fminf(fmaxf(az, bz), cull_t));
   return en <= ex;
 }
+// can a ray whose nearest hit so far is at t find a nearer one in the tree?  (the render query's test after the flat list)
+LR_DEV bool reaches_tree(const DevScene& sc, F3 o, F3 inv, float t) { return sc.n_nodes > 0 && bvh_bounds_hit(sc, o, inv, cull_distance(t)); }
 
 // BVH part of the STRICT nearest-hit query (probes, and the re-trace of the rare ray whose optimistic hit fails the gate):
 // "while-while" traversal (every lane first descends inner nodes until it holds a leaf or is done, the warp
@@ -351,14 +358,12 @@ LR_DEV bool bvh_bounds_hit(const DevScene& sc, F3 o, F3 inv, float cull_t) {
 // optimistic form below (trav_step: accept on the primitive test alone, gate the final nearest hit once).
 template <bool COUNT>
 LR_DEV void bvh_traverse(const DevScene& sc, F3 o, F3 d, F3 inv, float& best_t, int& best, TraceCounters& tc) {
-  // conservative cull distance: a primitive's computed t may precede its box's computed entry
-  float cull_t = best_t < 3.0e38f ? best_t * 1.0001f + 1e-4f : 3.0e38f;
-  constexpr int kDone = (int)0x80000000;       // not a valid leaf code (first triangle would be 2^28 - 1)
+  float cull_t = cull_distance(best_t);
   int stack[kStackDepth];
   int sp = 0;
-  stack[sp++] = kDone;
+  stack[sp++] = kTravDone;
   int cur = 0;
-  while (cur != kDone) {
+  while (cur != kTravDone) {
     while (cur >= 0) {
       const float4* np = sc.nodes + 4 * (size_t)cur;
       const float4 n0 = ldg4(np + 0), n1 = ldg4(np + 1), n2 = ldg4(np + 2), n3 = ldg4(np + 3);
@@ -388,7 +393,7 @@ LR_DEV void bvh_traverse(const DevScene& sc, F3 o, F3 d, F3 inv, float& best_t, 
         cur = stack[--sp];
       }
     }
-    if (cur != kDone) {
+    if (cur != kTravDone) {
       const int code = ~cur;
       const int first = code >> 3;
       const int count = (code & 7) + 1;
@@ -411,8 +416,8 @@ LR_DEV void bvh_traverse(const DevScene& sc, F3 o, F3 d, F3 inv, float& best_t, 
   }
 }
 
-// The optimistic form of the same query (accept on the primitive test, the caller gates the final nearest hit once with
-// bvh_hit_is_gated and falls back to the strict query if it fails: if the nearest candidate passes, it IS the gated nearest
+// The optimistic form of the same query (accept on the primitive test, finish_tree_query gates the final nearest hit once
+// with tri_gate and falls back to the strict query if it fails: if the nearest candidate passes, it IS the gated nearest
 // hit — the minimum over a superset that lies in the subset), organised as ONE loop whose every iteration advances a lane by at most
 // one inner node AND at most one triangle test: a leaf the descent reaches is moved to a one-entry leaf slot and the
 // descent goes on with the next stack entry while the slot's (<= 8) triangles are tested one per iteration.  In the
@@ -426,11 +431,10 @@ struct TravState {
   float best_t, cull_t;
   int best, cur, sp, leaf_first, leaf_left;
 };
-constexpr int kTravDone = (int)0x80000000;       // not a valid leaf code (first triangle would be 2^28 - 1)
 LR_DEV void trav_begin(TravState& s, int* stack, F3 o, F3 d, F3 inv, float best_t, int best) {
   s.o = o; s.d = d; s.inv = inv;
   s.best_t = best_t; s.best = best;
-  s.cull_t = best_t < 3.0e38f ? best_t * 1.0001f + 1e-4f : 3.0e38f;
+  s.cull_t = cull_distance(best_t);
   s.sp = 0;
   stack[s.sp++] = kTravDone;
   s.cur = 0;
@@ -499,8 +503,6 @@ LR_DEV void bvh_traverse_unified(const DevScene& sc, F3 o, F3 d, F3 inv, float& 
   best = s.best;
 }
 
-LR_DEV bool bvh_hit_is_gated(const DevScene& sc, F3 o, F3 inv, int id) { return tri_gate(sc, o, inv, id); }
-
 // Nearest hit: flat candidates first, then the BVH; among equal distances the lowest primitive id wins (the tie rule above).
 template <bool COUNT>
 LR_DEV void trace(const DevScene& sc, F3 o, F3 d, float& t_out, int& id_out, TraceCounters& tc) {
@@ -511,6 +513,25 @@ LR_DEV void trace(const DevScene& sc, F3 o, F3 d, float& t_out, int& id_out, Tra
   if (sc.n_nodes > 0) bvh_traverse<COUNT>(sc, o, d, inv, best_t, best, tc);
   t_out = best_t;
   id_out = best;
+}
+
+// strict nearest-hit query, out of line: only reached when the gate rejects an optimistic BVH hit (a few rays
+// per 10^8, LrStats.gate_retraces)
+template <bool COUNT>
+__device__ __noinline__ void trace_strict(const DevScene& sc, F3 o, F3 d, float* t, int* id, TraceCounters* tc) {
+  trace<COUNT>(sc, o, d, *t, *id, *tc);
+}
+
+// The tree part of the render query, for a ray whose nearest flat-list hit (t, id) is known and that reaches_tree: the
+// optimistic traversal, the nearest tree hit gated once, the strict query if the gate rejects it (counted in n_retrace).
+// The render kernels' BVH phase and the render-query probe (kernels.cu: rays_kernel<true>) both run this.
+template <bool COUNT>
+LR_DEV void finish_tree_query(const DevScene& sc, F3 o, F3 d, F3 inv, float& t, int& id, TraceCounters& tc, unsigned int& n_retrace) {
+  bvh_traverse_unified<COUNT>(sc, o, d, inv, t, id, tc);
+  if (id >= 0 && id < sc.n_bvh_tris && !tri_gate(sc, o, inv, id)) {
+    trace_strict<COUNT>(sc, o, d, &t, &id, &tc);
+    n_retrace++;
+  }
 }
 
 struct Surface {

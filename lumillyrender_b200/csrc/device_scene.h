@@ -55,7 +55,7 @@ struct DevParams {
   int shard, n_shards;                   // this launch renders the tiles t with shard_of_tile(t, n_shards) == shard (default 0 of 1)
   int unit_tiles;                        // how many tiles that is: shard_tile_count(tiles_x * tiles_y, ...), set once on the host
   int defer_iters, defer_thresh;         // path vertices per phase A; suspended lanes that end it early (persistent.cuh)
-  int organisation;                      // 0 = the build's measured best, 1 = one path per lane (persistent.cuh), 2 = pool (pool.cuh); BVH scenes only
+  int organisation;                      // BVH scenes only: 1 = one path per lane (persistent.cuh), otherwise the pool (pool.cuh)
 };
 
 // Pixel sharding of a film over several devices (lr_multi_film_*): the crop's 8x4 tiles are dealt round-robin, shard k of
@@ -69,6 +69,13 @@ __host__ __device__ inline int shard_tile_count(int n_tiles, int shard, int n_sh
   return shard < n_tiles ? (n_tiles - shard + n_shards - 1) / n_shards : 0;
 }
 __host__ __device__ inline int shard_device(int shard, int n_devices) { return shard % n_devices; }
+// A sample range [begin, begin + count) cut into n_parts consecutive ranges whose sizes differ by at most one: the range of
+// part `part`.  The devices of lr_render_multi (lr_shard_range) and the spp splits of one launch (path_vertex.inc) are cut so.
+struct SampleRange { int begin, count; };
+__host__ __device__ inline SampleRange range_part(int begin, int count, int part, int n_parts) {
+  const int per = count / n_parts, rem = count % n_parts;
+  return {begin + part * per + (part < rem ? part : rem), per + (part < rem ? 1 : 0)};
+}
 // work items of one render launch: one per (split, pixel slot of the shard's tiles)
 __host__ __device__ inline unsigned int render_units(const DevParams& p) { return (unsigned int)p.unit_tiles * 32u * (unsigned int)p.splits; }
 

@@ -1,4 +1,4 @@
-// kernels.cu — the small sm_100a kernels around the render kernel (which lives in persistent.cuh and is
+// kernels.cu — the small sm_100a kernels around the render kernel (which lives in persistent.cuh and pool.cuh and is
 // instantiated in persistent_inst.cu): ordered reduction of spp splits, normalisation, the cross-device reduce and
 // gather, the nearest-hit parity probes, and the read-bandwidth microbenchmark.
 //
@@ -74,9 +74,9 @@ primary_kernel(const __grid_constant__ DevScene sc, int tiles_x, int tiles_y, fl
   else { const Surface s = surface_at(sc, o, d, t, id); prim[i] = s.prim; tout[i] = t; }
 }
 
-// RENDER_QUERY = false: the strict query (the reference's gate on every candidate).  true: the query exactly as the render
-// kernels run it (path_vertex.inc + the BVH phase): flat list, tree-bounds test, optimistic traversal (trav_step), the
-// nearest tree hit gated once, strict re-trace if the gate rejects it — so a replay divergence can be pinned on a ray.
+// RENDER_QUERY = false: the strict query (the reference's gate on every candidate).  true: the render kernels' query through
+// their own code — flat_hits and reaches_tree (path_vertex.inc), then finish_tree_query (the BVH phase) — so a replay
+// divergence can be pinned on a ray.
 template <bool RENDER_QUERY>
 __global__ void __launch_bounds__(kBlockThreads)
 rays_kernel(const __grid_constant__ DevScene sc, long long n, const float* __restrict__ org, const float* __restrict__ dir,
@@ -92,10 +92,8 @@ rays_kernel(const __grid_constant__ DevScene sc, long long n, const float* __res
     t = 3.0e38f;
     id = -1;
     flat_hits<false>(sc, flat_list_global(sc), o, d, inv, t, id, tc);
-    if (sc.n_nodes > 0 && bvh_bounds_hit(sc, o, inv, t < 3.0e38f ? t * 1.0001f + 1e-4f : 3.0e38f)) {
-      bvh_traverse_unified<false>(sc, o, d, inv, t, id, tc);
-      if (id >= 0 && id < sc.n_bvh_tris && !bvh_hit_is_gated(sc, o, inv, id)) trace<false>(sc, o, d, t, id, tc);
-    }
+    unsigned int n_retrace = 0;
+    if (reaches_tree(sc, o, inv, t)) finish_tree_query<false>(sc, o, d, inv, t, id, tc, n_retrace);
   } else {
     trace<false>(sc, o, d, t, id, tc);
   }
@@ -171,14 +169,14 @@ __global__ void __launch_bounds__(256) read_bw_kernel(const float4* __restrict__
 }
 
 // ------------------------------------------------------------------ launchers
-cudaError_t launch_render_persistent(const DevScene& sc, const DevParams& p, bool has_ggx, bool count, float* out_sum, float* out_sumsq,
-                                     unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream) {
+cudaError_t launch_render(const DevScene& sc, const DevParams& p, bool has_ggx, bool count, float* out_sum, float* out_sumsq,
+                          unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream) {
   // the instrumented kernel exists in the (tree, GGX inline) units only: it is the most general code
   const bool tree = sc.n_nodes > 0 || count, ggx = has_ggx || count;
   using Fn = cudaError_t (*)(const DevScene&, const DevParams&, bool, float*, float*, unsigned long long*, unsigned int*, int, cudaStream_t);
   static const Fn table[2][2][2] = {
-      {{launch_persistent_i0_t0_g0, launch_persistent_i0_t0_g1}, {launch_persistent_i0_t1_g0, launch_persistent_i0_t1_g1}},
-      {{launch_persistent_i1_t0_g0, launch_persistent_i1_t0_g1}, {launch_persistent_i1_t1_g0, launch_persistent_i1_t1_g1}}};
+      {{launch_render_i0_t0_g0, launch_render_i0_t0_g1}, {launch_render_i0_t1_g0, launch_render_i0_t1_g1}},
+      {{launch_render_i1_t0_g0, launch_render_i1_t0_g1}, {launch_render_i1_t1_g0, launch_render_i1_t1_g1}}};
   return table[p.integrator == LR_INTEGRATOR_PT ? 0 : 1][tree ? 1 : 0][ggx ? 1 : 0](sc, p, count, out_sum, out_sumsq, counters, next_unit,
                                                                                    sm_count, stream);
 }

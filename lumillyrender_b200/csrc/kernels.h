@@ -3,16 +3,17 @@
 #include "device_scene.h"
 
 namespace lr {
-// the render kernel (persistent.cuh).  *next_unit must be 0 on `stream` before the launch.
-cudaError_t launch_render_persistent(const DevScene& sc, const DevParams& p, bool has_ggx, bool count, float* out_sum, float* out_sumsq,
-                                     unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream);
+// the render kernel in the organisation the scene runs (persistent.cuh or pool.cuh; instantiated per build in
+// persistent_inst.cu).  *next_unit must be 0 on `stream` before the launch.
+cudaError_t launch_render(const DevScene& sc, const DevParams& p, bool has_ggx, bool count, float* out_sum, float* out_sumsq,
+                          unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream);
 #define LR_DECL_INST(name)                                                                                              \
   cudaError_t name(const DevScene& sc, const DevParams& p, bool count, float* out_sum, float* out_sumsq,                \
                    unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream);
-LR_DECL_INST(launch_persistent_i0_t0_g0) LR_DECL_INST(launch_persistent_i0_t1_g0)
-LR_DECL_INST(launch_persistent_i1_t0_g0) LR_DECL_INST(launch_persistent_i1_t1_g0)
-LR_DECL_INST(launch_persistent_i0_t0_g1) LR_DECL_INST(launch_persistent_i0_t1_g1)
-LR_DECL_INST(launch_persistent_i1_t0_g1) LR_DECL_INST(launch_persistent_i1_t1_g1)
+LR_DECL_INST(launch_render_i0_t0_g0) LR_DECL_INST(launch_render_i0_t1_g0)
+LR_DECL_INST(launch_render_i1_t0_g0) LR_DECL_INST(launch_render_i1_t1_g0)
+LR_DECL_INST(launch_render_i0_t0_g1) LR_DECL_INST(launch_render_i0_t1_g1)
+LR_DECL_INST(launch_render_i1_t0_g1) LR_DECL_INST(launch_render_i1_t1_g1)
 #undef LR_DECL_INST
 cudaError_t launch_reduce_splits(float* dst, const float* partial, size_t n, int splits, cudaStream_t stream);
 cudaError_t launch_scale(float* dst, size_t n, float divisor, cudaStream_t stream);

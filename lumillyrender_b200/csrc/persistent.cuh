@@ -35,6 +35,31 @@ enum { F_DEPTH_MASK = 0xffff, F_ALLOW_EMISSION = 1 << 16, F_HAS_RAY = 1 << 17, F
 LR_DEV unsigned lanemask_lt() { unsigned m; asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m)); return m; }
 LR_DEV unsigned int warp_sum_u(unsigned int v) { return __reduce_add_sync(kFull, v); }
 
+// a render kernel's counters at its end: warp sums (left in the arguments), one atomic per counter and warp
+template <bool COUNT>
+LR_DEV void flush_counters(unsigned long long* counters, int lane, unsigned int& n_rays, unsigned int& n_nonfinite, unsigned int& n_retrace,
+                           TraceCounters& tc) {
+  n_rays = warp_sum_u(n_rays);
+  n_nonfinite = warp_sum_u(n_nonfinite);
+  n_retrace = warp_sum_u(n_retrace);
+  if (COUNT) {
+    tc.nodes = warp_sum_u(tc.nodes); tc.tris = warp_sum_u(tc.tris); tc.spheres = warp_sum_u(tc.spheres);
+    tc.flat_tris = warp_sum_u(tc.flat_tris); tc.flat_boxes = warp_sum_u(tc.flat_boxes);
+  }
+  if (lane == 0) {
+    if (n_rays) atomicAdd(counters + C_RAYS, (unsigned long long)n_rays);
+    if (n_nonfinite) atomicAdd(counters + C_NONFINITE, (unsigned long long)n_nonfinite);
+    if (n_retrace) atomicAdd(counters + C_RETRACE, (unsigned long long)n_retrace);
+    if (COUNT) {
+      atomicAdd(counters + C_NODES, (unsigned long long)tc.nodes);
+      atomicAdd(counters + C_TRIS, (unsigned long long)tc.tris);
+      atomicAdd(counters + C_SPHERES, (unsigned long long)tc.spheres);
+      atomicAdd(counters + C_FLAT_TRIS, (unsigned long long)tc.flat_tris);
+      atomicAdd(counters + C_FLAT_BOXES, (unsigned long long)tc.flat_boxes);
+    }
+  }
+}
+
 // unit -> (split, crop-relative pixel): the shard's 8x4 pixel tiles lane by lane, so a warp starts on one tile
 LR_DEV bool decode_unit(const DevParams& p, unsigned int u, int& lx, int& ly, int& split) {
   const unsigned int per_split = (unsigned int)p.unit_tiles * 32u;
@@ -44,13 +69,6 @@ LR_DEV bool decode_unit(const DevParams& p, unsigned int u, int& lx, int& ly, in
   lx = (int)(tile % p.tiles_x) * 8 + (int)(lane & 7u);
   ly = (int)(tile / p.tiles_x) * 4 + (int)(lane >> 3);
   return lx < p.crop_w && ly < p.crop_h;
-}
-
-// strict nearest-hit query, out of line: only reached when the gate rejects an optimistic BVH hit (a few rays
-// per 10^8, LrStats.gate_retraces)
-template <bool COUNT>
-__device__ __noinline__ void trace_strict(const DevScene& sc, F3 o, F3 d, float* t, int* id, TraceCounters* tc) {
-  trace<COUNT>(sc, o, d, *t, *id, *tc);
 }
 
 }  // namespace pk
@@ -136,8 +154,7 @@ render_persistent_kernel(const __grid_constant__ DevScene sc, const __grid_const
 
     // ================================================================ phase B
     // the suspended rays traverse the BVH together (one call site, one node and one triangle test per iteration:
-    // trav_step): optimistic accept, the nearest hit gated once at the end, strict re-trace in the rare case the gate
-    // rejects it
+    // trav_step)
 #pragma unroll 1
     for (int r = 0; TREE && r < NR; r++) {
       const bool on = r == 0 ? pend0 : pend1;
@@ -147,50 +164,31 @@ render_persistent_kernel(const __grid_constant__ DevScene sc, const __grid_const
         const F3 inv = f3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
         float t = r == 0 ? t0 : t1;
         int id = r == 0 ? id0 : id1;
-        bvh_traverse_unified<COUNT>(sc, o, d, inv, t, id, tc);
-        if (id >= 0 && id < sc.n_bvh_tris && !bvh_hit_is_gated(sc, o, inv, id)) {
-          trace_strict<COUNT>(sc, o, d, &t, &id, &tc);
-          n_retrace++;
-        }
+        finish_tree_query<COUNT>(sc, o, d, inv, t, id, tc, n_retrace);
         if (r == 0) { t0 = t; id0 = id; pend0 = false; } else { t1 = t; id1 = id; pend1 = false; }
       }
     }
     if (!__any_sync(kFull, alive)) break;
   }
 
-  // counters: warp reduce, one atomic per warp
-  n_rays = warp_sum_u(n_rays);
-  n_nonfinite = warp_sum_u(n_nonfinite);
-  n_retrace = warp_sum_u(n_retrace);
-  if (COUNT) {
-    tc.nodes = warp_sum_u(tc.nodes); tc.tris = warp_sum_u(tc.tris); tc.spheres = warp_sum_u(tc.spheres);
-    tc.flat_tris = warp_sum_u(tc.flat_tris); tc.flat_boxes = warp_sum_u(tc.flat_boxes);
-  }
-  if (lane == 0) {
-    if (n_rays) atomicAdd(counters + C_RAYS, (unsigned long long)n_rays);
-    if (n_nonfinite) atomicAdd(counters + C_NONFINITE, (unsigned long long)n_nonfinite);
-    if (n_retrace) atomicAdd(counters + C_RETRACE, (unsigned long long)n_retrace);
-    if (COUNT) {
-      atomicAdd(counters + C_NODES, (unsigned long long)tc.nodes);
-      atomicAdd(counters + C_TRIS, (unsigned long long)tc.tris);
-      atomicAdd(counters + C_SPHERES, (unsigned long long)tc.spheres);
-      atomicAdd(counters + C_FLAT_TRIS, (unsigned long long)tc.flat_tris);
-      atomicAdd(counters + C_FLAT_BOXES, (unsigned long long)tc.flat_boxes);
-    }
-  }
+  flush_counters<COUNT>(counters, lane, n_rays, n_nonfinite, n_retrace, tc);
 }
 
-// one launch = the whole sample range of every unit: a persistent grid that fills the SMs
+// One launch = the whole sample range of every unit: a persistent grid that fills the SMs.  Blocks for every unit at
+// units_per_block, at most as many as are resident at once (the occupancy query's blocks per SM, or `fallback` if it fails).
+inline unsigned int render_grid(const void* kernel, size_t smem, long long units_per_block, int fallback, const DevParams& p, int sm_count) {
+  int nb = 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, kBlockThreads, smem) != cudaSuccess || nb <= 0) nb = fallback;
+  const long long want = ((long long)render_units(p) + units_per_block - 1) / units_per_block;
+  return (unsigned int)std::max<long long>(1, std::min<long long>(want, (long long)nb * sm_count));
+}
+
 template <int INTEGRATOR, bool TREE, bool COUNT, int BUILD>
 cudaError_t launch_persistent_one(const DevScene& sc, const DevParams& p, float* out_sum, float* out_sumsq,
                                   unsigned long long* counters, unsigned int* next_unit, int sm_count, cudaStream_t stream) {
-  int nb = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, render_persistent_kernel<INTEGRATOR, TREE, COUNT, BUILD>, kBlockThreads, 0) !=
-          cudaSuccess || nb <= 0) nb = 4;
-  const long long units = render_units(p);
-  const long long want = (units + kBlockThreads - 1) / kBlockThreads;
-  const unsigned int blocks = (unsigned int)std::max<long long>(1, std::min<long long>(want, (long long)nb * sm_count));
-  render_persistent_kernel<INTEGRATOR, TREE, COUNT, BUILD><<<blocks, kBlockThreads, 0, stream>>>(sc, p, out_sum, out_sumsq, counters, next_unit);
+  auto kernel = render_persistent_kernel<INTEGRATOR, TREE, COUNT, BUILD>;
+  const unsigned int blocks = render_grid((const void*)kernel, 0, kBlockThreads, 4, p, sm_count);     // a lane serves one unit at a time
+  kernel<<<blocks, kBlockThreads, 0, stream>>>(sc, p, out_sum, out_sumsq, counters, next_unit);
   return cudaGetLastError();
 }
 

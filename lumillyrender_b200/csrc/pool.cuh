@@ -15,8 +15,6 @@
 // summed in its slot in sample order (main.rs:92-104) and its RNG stream is a function of (seed, pixel, sample), so
 // every sample — and the image — equals persistent.cuh's bit for bit, whichever lane ran which step.
 #pragma once
-#include <algorithm>
-
 #include "device_path.cuh"
 #include "kernels.h"
 #include "persistent.cuh"
@@ -253,8 +251,7 @@ render_pool_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ 
     } else {
       // ================================================================ phase B
       // a batch of up to 32 pending rays (extension or shadow) traverses the BVH: one loop that advances every lane by
-      // at most one inner node and one triangle test per iteration (trav_step), optimistic accept, the nearest hit gated
-      // once at the end, strict re-trace in the rare case the gate rejects it.  (Measured and dropped, each bit-exact: idle
+      // at most one inner node and one triangle test per iteration (trav_step).  (Measured and dropped, each bit-exact: idle
       // lanes refilled from the pending rays inside this loop — r01 and again r02 with pools of 64 / 96 slots: 14-22 % slower;
       // two rays per lane: 23 % slower; the tree collapsed to 4-wide nodes: 4 % slower; batches formed from one class of rays —
       // bounces off the mesh apart from rays that come from a wall or the camera: 2-6 % slower.  profiles/r02_{b,c,h}_ab.txt.)
@@ -269,11 +266,7 @@ render_pool_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ 
         const F3 inv = f3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
         float t = shadow ? SLF(W_T1) : SLF(W_T0);
         int id = shadow ? SLI(W_ID1) : SLI(W_ID0);
-        bvh_traverse_unified<COUNT>(sc, o, d, inv, t, id, tc);
-        if (id >= 0 && id < sc.n_bvh_tris && !bvh_hit_is_gated(sc, o, inv, id)) {
-          trace_strict<COUNT>(sc, o, d, &t, &id, &tc);
-          n_retrace++;
-        }
+        finish_tree_query<COUNT>(sc, o, d, inv, t, id, tc, n_retrace);
         if (shadow) { SLF(W_T1) = t; SLI(W_ID1) = id; } else { SLF(W_T0) = t; SLI(W_ID0) = id; }
       }
     }
@@ -282,29 +275,9 @@ render_pool_kernel(const __grid_constant__ DevScene sc, const __grid_constant__ 
 #undef SLF
 #undef SLI
 
-  // counters: warp reduce, one atomic per warp
-  n_rays = warp_sum_u(n_rays);
-  n_nonfinite = warp_sum_u(n_nonfinite);
-  n_retrace = warp_sum_u(n_retrace);
-  if (COUNT) {
-    tc.nodes = warp_sum_u(tc.nodes); tc.tris = warp_sum_u(tc.tris); tc.spheres = warp_sum_u(tc.spheres);
-    tc.flat_tris = warp_sum_u(tc.flat_tris); tc.flat_boxes = warp_sum_u(tc.flat_boxes);
-  }
-  if (lane == 0) {
-    if (n_rays) atomicAdd(counters + C_RAYS, (unsigned long long)n_rays);
-    if (n_nonfinite) atomicAdd(counters + C_NONFINITE, (unsigned long long)n_nonfinite);
-    if (n_retrace) atomicAdd(counters + C_RETRACE, (unsigned long long)n_retrace);
-    if (COUNT) {
-      atomicAdd(counters + C_NODES, (unsigned long long)tc.nodes);
-      atomicAdd(counters + C_TRIS, (unsigned long long)tc.tris);
-      atomicAdd(counters + C_SPHERES, (unsigned long long)tc.spheres);
-      atomicAdd(counters + C_FLAT_TRIS, (unsigned long long)tc.flat_tris);
-      atomicAdd(counters + C_FLAT_BOXES, (unsigned long long)tc.flat_boxes);
-    }
-  }
+  flush_counters<COUNT>(counters, lane, n_rays, n_nonfinite, n_retrace, tc);
 }
 
-// one launch = the whole sample range of every unit: a persistent grid that fills the SMs
 template <int INTEGRATOR, bool TREE, bool COUNT, int BUILD>
 cudaError_t launch_pool_one(const DevScene& sc, const DevParams& p, float* out_sum, float* out_sumsq, unsigned long long* counters,
                             unsigned int* next_unit, int sm_count, cudaStream_t stream) {
@@ -312,13 +285,8 @@ cudaError_t launch_pool_one(const DevScene& sc, const DevParams& p, float* out_s
   const size_t smem = (size_t)(kBlockThreads / 32) * pl::warp_words<INTEGRATOR>(out_sumsq != nullptr) * sizeof(float);
   cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  int nb = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, kBlockThreads, smem) != cudaSuccess || nb <= 0) nb = 2;
-  // a warp serves kSlots units at a time
-  const long long units = render_units(p);
-  const long long per_block = (long long)(kBlockThreads / 32) * pl::slots<INTEGRATOR>();
-  const long long want = (units + per_block - 1) / per_block;
-  const unsigned int blocks = (unsigned int)std::max<long long>(1, std::min<long long>(want, (long long)nb * sm_count));
+  // a warp serves as many units at a time as it has slots
+  const unsigned int blocks = render_grid((const void*)kernel, smem, (long long)(kBlockThreads / 32) * pl::slots<INTEGRATOR>(), 2, p, sm_count);
   kernel<<<blocks, kBlockThreads, smem, stream>>>(sc, p, out_sum, out_sumsq, counters, next_unit);
   return cudaGetLastError();
 }
