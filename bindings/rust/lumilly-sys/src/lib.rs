@@ -83,6 +83,13 @@ extern "C" {
     pub fn lr_multi_film_save(film: *const LrMultiFilm, path: *const c_char) -> c_int;
     pub fn lr_multi_film_load(ms: *mut LrMultiScene, path: *const c_char, out: *mut *mut LrMultiFilm) -> c_int;
     pub fn lr_multi_film_destroy(film: *mut LrMultiFilm);
+    /// adaptive sampling: spp_count more samples on the tiles whose relative standard error exceeds `threshold`, each from
+    /// its own count (max_spp > 0 caps a tile's samples); the per-pixel sample counts of either film
+    pub fn lr_film_render_adaptive(film: *mut LrFilm, spp_count: i32, threshold: f32, max_spp: i32, active_tiles: *mut i32, stats: *mut LrStats) -> c_int;
+    pub fn lr_film_spp_map(film: *const LrFilm, out: *mut i32) -> c_int;
+    pub fn lr_multi_film_render_adaptive(film: *mut LrMultiFilm, spp_count: i32, threshold: f32, max_spp: i32, active_tiles: *mut i32,
+                                         stats: *mut LrStats) -> c_int;
+    pub fn lr_multi_film_spp_map(film: *const LrMultiFilm, out: *mut i32) -> c_int;
     pub fn lr_trace_primary(scene: *const LrScene, u: f32, v: f32, ua: f32, va: f32, prim: *mut i32, t: *mut f32) -> c_int;
     pub fn lr_trace_rays(scene: *const LrScene, n: i64, origins: *const f32, directions: *const f32, prim: *mut i32, t: *mut f32, normal: *mut f32) -> c_int;
     pub fn lr_trace_rays_query(scene: *const LrScene, n: i64, origins: *const f32, directions: *const f32, query: i32, prim: *mut i32, t: *mut f32,

@@ -279,6 +279,25 @@ int lr_multi_film_save(const LrMultiFilm* film, const char* path);
 int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out);
 void lr_multi_film_destroy(LrMultiFilm* film);
 
+/* ---- adaptive sampling on either film: samples only where the image is still noisy.  Each 8x4 pixel tile of the crop holds
+ * its own sample count n.  A tile's error is the largest relative standard error of a pixel mean over its pixels and
+ * channels, sqrt(var / n) / max(mean, 1e-3) with var = max(0, (Q - S * mean) / (n - 1)), computed in double precision
+ * from the sums S and the sums of squares Q.  A tile is rendered when (n < 2 or (its S and Q are finite and its error >
+ * threshold)) and (max_spp == 0 or n < max_spp).  Every tile continues from its own count with one thread per pixel, so each
+ * pixel is bit for bit lr_render(splits = 1) at its tile's count, for any device count.  lr_film_render on a film whose
+ * tiles differ renders every tile from its own count; lr_film_info's spp_done is then the fewest samples any pixel holds,
+ * and lr_film_read divides every pixel by its tile's count.  A film whose tiles hold equal counts saves the LRFILM1
+ * checkpoint; otherwise save writes LRFILM2, the same followed by the tile counts (int32, row-major), and both handles load
+ * both. */
+/* Adds spp_count samples to every tile of the film whose noise exceeds `threshold` (the rule above), each tile from its own
+   sample count; tiles holding max_spp samples or more (max_spp > 0) are left alone, so a tile ends with fewer than
+   max_spp + spp_count.  Without a cap a tile whose estimates can be negative may never converge.  *active_tiles (nullable)
+   = tiles rendered; 0 means nothing was rendered.  Needs a film made with sums of squares; renders with splits = 1. */
+int lr_film_render_adaptive(LrFilm* film, int32_t spp_count, float threshold, int32_t max_spp, int32_t* active_tiles, LrStats* stats);
+int lr_film_spp_map(const LrFilm* film, int32_t* out /* crop_w*crop_h: samples held by each pixel */);
+int lr_multi_film_render_adaptive(LrMultiFilm* film, int32_t spp_count, float threshold, int32_t max_spp, int32_t* active_tiles, LrStats* stats);
+int lr_multi_film_spp_map(const LrMultiFilm* film, int32_t* out);
+
 /* ---- parity probe: nearest hit of the primary ray through every film pixel with the
  * sensor jitter fixed to (u,v) and the aperture sample fixed to (ua,va).
  * prim[i] = primitive id or -1, t[i] = Intersection.distance (bvh.rs:131-141).      */

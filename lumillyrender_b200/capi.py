@@ -119,6 +119,10 @@ SIGNATURES = {
     "lr_multi_film_save": (C.c_int, [_VP, C.c_char_p]),
     "lr_multi_film_load": (C.c_int, [_VP, C.c_char_p, C.POINTER(_VP)]),
     "lr_multi_film_destroy": (None, [_VP]),
+    "lr_film_render_adaptive": (C.c_int, [_VP, i32, f32, i32, _PI, C.POINTER(LrStats)]),
+    "lr_film_spp_map": (C.c_int, [_VP, _PI]),
+    "lr_multi_film_render_adaptive": (C.c_int, [_VP, i32, f32, i32, _PI, C.POINTER(LrStats)]),
+    "lr_multi_film_spp_map": (C.c_int, [_VP, _PI]),
     "lr_trace_primary": (C.c_int, [_VP, f32, f32, f32, f32, _PI, _PF]),
     "lr_trace_rays": (C.c_int, [_VP, i64, _PF, _PF, _PI, _PF, _PF]),
     "lr_trace_rays_query": (C.c_int, [_VP, i64, _PF, _PF, i32, _PI, _PF, _PF]),

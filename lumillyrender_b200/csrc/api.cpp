@@ -356,8 +356,15 @@ int lr_scene_bytes(const LrScene* s, uint64_t* h2d_bytes) {
 }
 
 // One shard of a sharded film (an LrMultiFilm): shard `index` of `count` (device_scene.h: shard_of_tile).  Such a
-// render always runs one thread per pixel, adding its samples in order (splits = 1), whatever LR_SPLITS says.
-struct FilmShard { int index, count; };
+// render always runs one thread per pixel, adding its samples in order (splits = 1), whatever LR_SPLITS says.  With a
+// tile_list (a film whose tiles hold different counts), the launch renders the `listed` tiles of that device list instead,
+// each from its own first sample index; they hold `pixels` pixels of the crop.
+struct FilmShard {
+  int index, count;
+  const int2* tile_list = nullptr;
+  int listed = 0;
+  uint64_t pixels = 0;
+};
 
 static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& dp, const FilmShard* shard = nullptr) {
   if (!s || !p) return fail(LR_ERR_INVALID, "null argument");
@@ -392,7 +399,8 @@ static int resolve_params(const LrScene* s, const LrRenderParams* p, DevParams& 
   dp.splits = splits;
   dp.shard = shard ? shard->index : 0;
   dp.n_shards = shard ? shard->count : 1;
-  dp.unit_tiles = shard_tile_count(dp.tiles_x * dp.tiles_y, dp.shard, dp.n_shards);
+  dp.unit_tiles = shard && shard->tile_list ? shard->listed : shard_tile_count(dp.tiles_x * dp.tiles_y, dp.shard, dp.n_shards);
+  dp.tile_list = shard ? shard->tile_list : nullptr;
   // kernel organisation knobs (development / profiling only; defaults are the measured best, DESIGN.md §4)
   const char* e_di = std::getenv("LR_DEFER_ITERS");
   const char* e_dt = std::getenv("LR_DEFER_THRESH");
@@ -467,7 +475,7 @@ static int accumulate(const LrScene* s, const LrRenderParams* p, float* d_sum, f
   }
   LR_CUDA(cudaEventRecord(s->ev1, st));
   s->ev_pending = true;
-  s->acc_samples += shard_pixels(dp) * (uint64_t)dp.spp_count;
+  s->acc_samples += (dp.tile_list ? shard->pixels : shard_pixels(dp)) * (uint64_t)dp.spp_count;
   s->last_splits = dp.splits;
   return LR_OK;
 }
@@ -898,19 +906,28 @@ int lr_trace_rays_query(const LrScene* s, int64_t n, const float* origins, const
 // ---------------------------------------------------------------- progressive / resumable rendering (main.rs:81-91)
 }  // extern "C"
 
-// A film: the per-pixel sums (and sums of squares) of a render in progress, and how many sample indices they hold.  It is a
-// list of parts, one per device, each with crop-sized buffers on its scene's device.  The crop's 8x4 tiles are dealt over
-// n_shards shards (device_scene.h: shard_of_tile), shard k renders on part shard_device(k, n_parts), and read / save gather
-// the crop on part 0's device, each pixel from the part that owns it.  Both C handles are this film; what differs is fixed
-// at creation (film_of): an LrFilm is one part on the scene's device and the legacy stream and renders as lr_render does,
-// params->splits included; an LrMultiFilm has a part per device of its LrMultiScene, each on that device's stream, and is
-// sharded: one thread per pixel adds the samples in order (splits = 1), so the bits do not depend on the device count.
+// A film: the per-pixel sums (and sums of squares) of a render in progress, and how many sample indices every 8x4 tile of
+// the crop holds.  It is a list of parts, one per device, each with crop-sized buffers on its scene's device.  The crop's
+// tiles are dealt over n_shards shards (device_scene.h: shard_of_tile), shard k renders on part shard_device(k, n_parts),
+// and read / save gather the crop on part 0's device, each pixel from the part that owns it.  Both C handles are this film;
+// what differs is fixed at creation (film_of): an LrFilm is one part on the scene's device and the legacy stream and renders
+// as lr_render does, params->splits included; an LrMultiFilm has a part per device of its LrMultiScene, each on that device's
+// stream, and is sharded: one thread per pixel adds the samples in order (splits = 1), so the bits do not depend on the
+// device count.  The host owns the tile counts.  While they are all equal a render adds the next sample indices to every
+// tile as lr_render does; once adaptive sampling has made them differ, every render launches a tile list (DevParams.tile_list)
+// so that each tile continues from its own count, one thread per pixel.
 struct Film {
   struct Part {
     const LrScene* scene = nullptr;
     cudaStream_t stream = nullptr;
     float* d_sum = nullptr;
     float* d_sumsq = nullptr;
+    // tile-list renders (made on first use): the film's tile counts, the lists of this part's shards (one segment each,
+    // shard_segments), the selection flags and the selected tile and pixel counts (two words per shard)
+    int* d_counts = nullptr;
+    int2* d_list = nullptr;
+    unsigned char* d_selected = nullptr;
+    unsigned long long* d_out = nullptr;
   };
   Part parts[kMaxPeers];
   int n_parts = 1;
@@ -918,20 +935,30 @@ struct Film {
   bool sharded = false;
   int n_shards = 1;
   LrRenderParams params{};               // spp_begin = first sample index of the film, spp_count unused
-  int32_t spp_done = 0;
   int32_t crop_w = 0, crop_h = 0;        // resolved window
+  int32_t tiles_x = 0, tiles_y = 0;      // its 8x4 tiles
+  std::vector<int32_t> tile_spp;         // samples every pixel of tile t (row-major over the crop's tiles) holds
   bool has_sumsq = false;
+
+  int n_tiles() const { return tiles_x * tiles_y; }
+  int32_t spp_min() const { return *std::min_element(tile_spp.begin(), tile_spp.end()); }
+  bool uniform() const { return std::all_of(tile_spp.begin(), tile_spp.end(), [&](int32_t n) { return n == tile_spp[0]; }); }
 
   Film() = default;
   Film(const Film&) = delete;
   Film& operator=(const Film&) = delete;
   ~Film() {
     for (int i = 0; i < n_parts; i++) {
-      if (!parts[i].d_sum && !parts[i].d_sumsq) continue;
-      const OnDevice on(parts[i].scene->device);
+      Part& p = parts[i];
+      if (!p.d_sum && !p.d_sumsq && !p.d_counts) continue;
+      const OnDevice on(p.scene->device);
       cudaDeviceSynchronize();
-      dev_free(parts[i].d_sum);
-      dev_free(parts[i].d_sumsq);
+      dev_free(p.d_sum);
+      dev_free(p.d_sumsq);
+      dev_free(p.d_counts);
+      dev_free(p.d_list);
+      dev_free(p.d_selected);
+      dev_free(p.d_out);
     }
   }
 };
@@ -939,7 +966,10 @@ struct LrFilm : Film {};
 struct LrMultiFilm : Film {};
 
 namespace {
+// LRFILM1: every tile holds spp_done samples.  LRFILM2 (tiles with different counts, adaptive sampling): the same header with
+// spp_done = the fewest samples any tile holds, the same data, then tiles_x * tiles_y int32 tile counts.
 constexpr char kFilmMagic[8] = {'L', 'R', 'F', 'I', 'L', 'M', '1', 0};
+constexpr char kFilmMagicTiles[8] = {'L', 'R', 'F', 'I', 'L', 'M', '2', 0};
 struct FilmHeader {                      // checkpoint file: this header, then crop_w*crop_h*3 floats (and again for the squares)
   char magic[8];
   int32_t film_w, film_h, crop_x, crop_y, crop_w, crop_h;
@@ -948,20 +978,28 @@ struct FilmHeader {                      // checkpoint file: this header, then c
 };
 
 // reads a checkpoint made for a film_w x film_h film: its header, its data (the raw sums, then the sums of squares if the
-// header says so) and the parameters to resume with
-int film_read(const char* path, int film_w, int film_h, FilmHeader* hp, std::vector<float>* data, LrRenderParams* params) {
+// header says so), the samples of every tile and the parameters to resume with
+int film_read(const char* path, int film_w, int film_h, FilmHeader* hp, std::vector<float>* data, std::vector<int32_t>* tile_spp,
+              LrRenderParams* params) {
   FILE* fp = std::fopen(path, "rb");
   if (!fp) return fail(LR_ERR_IO, std::string("File `") + path + "` is not found.");
   FilmHeader& h = *hp;
   int rc = LR_OK;
   do {
-    if (std::fread(&h, sizeof(h), 1, fp) != 1 || std::memcmp(h.magic, kFilmMagic, 8) != 0) { rc = fail(LR_ERR_PARSE, "not a film checkpoint"); break; }
+    if (std::fread(&h, sizeof(h), 1, fp) != 1) { rc = fail(LR_ERR_PARSE, "not a film checkpoint"); break; }
+    const bool tiles = std::memcmp(h.magic, kFilmMagicTiles, 8) == 0;
+    if (!tiles && std::memcmp(h.magic, kFilmMagic, 8) != 0) { rc = fail(LR_ERR_PARSE, "not a film checkpoint"); break; }
     if (h.film_w != film_w || h.film_h != film_h) { rc = fail(LR_ERR_INVALID, "the checkpoint was made for another film resolution"); break; }
     if (h.crop_w <= 0 || h.crop_h <= 0 || h.crop_x < 0 || h.crop_y < 0 || h.crop_x + h.crop_w > film_w || h.crop_y + h.crop_h > film_h ||
         h.spp_done < 0 || h.spp_begin < 0) { rc = fail(LR_ERR_PARSE, "corrupt film checkpoint header"); break; }
     const size_t n = (size_t)h.crop_w * h.crop_h * 3;
     data->resize(n * (h.has_sumsq ? 2 : 1));
     if (std::fread(data->data(), sizeof(float), data->size(), fp) != data->size()) { rc = fail(LR_ERR_PARSE, "truncated film checkpoint"); break; }
+    tile_spp->assign((size_t)((h.crop_w + 7) / 8) * ((h.crop_h + 3) / 4), h.spp_done);
+    if (tiles) {
+      if (std::fread(tile_spp->data(), sizeof(int32_t), tile_spp->size(), fp) != tile_spp->size()) { rc = fail(LR_ERR_PARSE, "truncated film checkpoint"); break; }
+      if (*std::min_element(tile_spp->begin(), tile_spp->end()) != h.spp_done) { rc = fail(LR_ERR_PARSE, "corrupt film checkpoint tile counts"); break; }
+    }
   } while (0);
   std::fclose(fp);
   if (rc != LR_OK) return rc;
@@ -1004,6 +1042,8 @@ int film_setup(Film* f, const LrRenderParams& p, int want_sumsq) {
   f->params = p; f->params.spp_count = 0;
   if (f->sharded) f->params.splits = 1;
   f->crop_w = dp.crop_w; f->crop_h = dp.crop_h; f->has_sumsq = want_sumsq != 0;
+  f->tiles_x = dp.tiles_x; f->tiles_y = dp.tiles_y;
+  f->tile_spp.assign((size_t)f->n_tiles(), 0);
   const size_t bytes = (size_t)dp.crop_w * dp.crop_h * 3 * sizeof(float);
   int rc = LR_OK;
   OnDevices on(rc);
@@ -1039,8 +1079,9 @@ int film_load(Owner* o, const char* path, Handle** out) {
   const Film::Part& p0 = f->parts[0];
   FilmHeader h;
   std::vector<float> host;
+  std::vector<int32_t> tile_spp;
   LrRenderParams p;
-  if (int rc = film_read(path, p0.scene->width, p0.scene->height, &h, &host, &p)) return rc;
+  if (int rc = film_read(path, p0.scene->width, p0.scene->height, &h, &host, &tile_spp, &p)) return rc;
   if (f->sharded && h.splits != 1) return fail(LR_ERR_INVALID, "the checkpoint was rendered with splits != 1; a multi-device film adds samples in order");
   if (int rc = film_setup(f.get(), p, h.has_sumsq)) return rc;
   // the sums go to part 0, and from there to every other part
@@ -1057,17 +1098,44 @@ int film_load(Owner* o, const char* path, Handle** out) {
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(p0.stream);
   if (e != cudaSuccess) return rc = fail(LR_ERR_CUDA, std::string("film load: ") + cudaGetErrorString(e));
-  f->spp_done = h.spp_done;
+  f->tile_spp = std::move(tile_spp);
   *out = f.release();
   return LR_OK;
 }
 
-int film_render(Film* f, int32_t spp_count, LrStats* stats) {
-  if (!f) return fail(LR_ERR_INVALID, "null argument");
-  if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
-  LrRenderParams q = f->params;
-  q.spp_begin = f->params.spp_begin + f->spp_done;
-  q.spp_count = spp_count;
+// Where shard k's tile list starts in the d_list of its part: the shards of a part own disjoint tiles, so their lists fit
+// one crop-sized buffer one after the other.
+std::vector<int> shard_segments(const Film* f) {
+  std::vector<int> at(f->n_shards), next(f->n_parts, 0);
+  for (int k = 0; k < f->n_shards; k++) {
+    int& n = next[shard_device(k, f->n_parts)];
+    at[k] = n;
+    n += shard_tile_count(f->n_tiles(), k, f->n_shards);
+  }
+  return at;
+}
+
+// the buffers of tile-list renders on every part, on first use
+int ensure_tile_lists(Film* f) {
+  int rc = LR_OK;
+  OnDevices on(rc);
+  for (int i = 0; i < f->n_parts && rc == LR_OK; i++) {
+    Film::Part& part = f->parts[i];
+    if (part.d_counts) continue;
+    if ((rc = on.use(part.scene->device)) != LR_OK) break;
+    const size_t n = (size_t)f->n_tiles();
+    cudaError_t e = dev_alloc((void**)&part.d_counts, n * sizeof(int));
+    if (e == cudaSuccess) e = dev_alloc((void**)&part.d_list, n * sizeof(int2));
+    if (e == cudaSuccess) e = dev_alloc((void**)&part.d_selected, n);
+    if (e == cudaSuccess) e = dev_alloc((void**)&part.d_out, 2 * (size_t)f->n_shards * sizeof(unsigned long long));
+    if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("film tile lists: ") + cudaGetErrorString(e));
+  }
+  return rc;
+}
+
+// Renders spp_count samples: shard k of `shards` on its part (honour_splits: an LrFilm whose tiles hold equal counts, which
+// renders as lr_render does), every part at once, then waits for them.  Statistics are totals, kernel_ms the slowest device's.
+int film_launch(Film* f, const LrRenderParams& q, const std::vector<FilmShard>& shards, bool honour_splits, LrStats* stats) {
   LrStats total;
   std::memset(&total, 0, sizeof(total));
   int rc = LR_OK;
@@ -1080,42 +1148,143 @@ int film_render(Film* f, int32_t spp_count, LrStats* stats) {
   // them one after the other (disjoint pixels of the same buffer)
   for (int k = 0; k < f->n_shards && rc == LR_OK; k++) {
     const Film::Part& part = f->parts[shard_device(k, f->n_parts)];
-    const FilmShard shard{k, f->n_shards};
-    rc = accumulate(part.scene, &q, part.d_sum, part.d_sumsq, part.stream, f->sharded ? &shard : nullptr);
+    rc = accumulate(part.scene, &q, part.d_sum, part.d_sumsq, part.stream, honour_splits ? nullptr : &shards[k]);
   }
-  // wait for every part: the samples are in the film; statistics are totals, kernel_ms the slowest device's
+  // wait for every part: the samples are in the film
   for (int i = 0; i < f->n_parts && rc == LR_OK; i++) {
     LrStats st;
     if ((rc = lr_stats_fetch(f->parts[i].scene, f->parts[i].stream, &st)) == LR_OK) add_device_stats(total, st);
   }
   if (rc != LR_OK) return rc;
-  f->spp_done += spp_count;
   if (stats) *stats = total;
   return LR_OK;
 }
 
+// Lists, on every part's device, the tiles of each shard that get samples in this call (launch_select_tiles): the noisy ones
+// (adaptive sampling), or every tile (every_tile: a film whose counts differ continues each tile from its own count).  Shard
+// k's list is at d_list + at[k] of its part; (*out)[2k] and (*out)[2k + 1] are its tile count and their in-crop pixels.
+int film_list_tiles(Film* f, bool every_tile, float threshold, int32_t max_spp, const std::vector<int>& at, std::vector<unsigned long long>* out) {
+  if (int rc = ensure_tile_lists(f)) return rc;
+  out->assign(2 * (size_t)f->n_shards, 0);
+  int rc = LR_OK;
+  OnDevices on(rc);
+  cudaError_t e = cudaSuccess;
+  for (int i = 0; i < f->n_parts && e == cudaSuccess; i++) {
+    if ((rc = on.use(f->parts[i].scene->device)) != LR_OK) return rc;
+    e = cudaMemcpyAsync(f->parts[i].d_counts, f->tile_spp.data(), f->tile_spp.size() * sizeof(int32_t), cudaMemcpyHostToDevice, f->parts[i].stream);
+  }
+  for (int k = 0; k < f->n_shards && e == cudaSuccess; k++) {
+    const Film::Part& part = f->parts[shard_device(k, f->n_parts)];
+    if ((rc = on.use(part.scene->device)) != LR_OK) return rc;
+    e = launch_select_tiles(part.d_sum, part.d_sumsq, part.d_counts, f->crop_w, f->crop_h, k, f->n_shards,
+                            shard_tile_count(f->n_tiles(), k, f->n_shards), threshold, max_spp, f->params.spp_begin,
+                            part.d_selected + at[k], part.d_list + at[k], every_tile, part.d_out + 2 * k, part.stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out->data() + 2 * k, part.d_out + 2 * k, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, part.stream);
+  }
+  for (int i = 0; i < f->n_parts && e == cudaSuccess; i++) {
+    if ((rc = on.use(f->parts[i].scene->device)) != LR_OK) return rc;
+    e = cudaStreamSynchronize(f->parts[i].stream);
+  }
+  if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("film tile list: ") + cudaGetErrorString(e));
+  return rc;
+}
+
+// Renders spp_count samples on the tiles film_list_tiles listed, each from its own first sample index.
+int film_launch_lists(Film* f, int32_t spp_count, const std::vector<int>& at, const std::vector<unsigned long long>& out, LrStats* stats) {
+  std::vector<FilmShard> shards(f->n_shards);
+  for (int k = 0; k < f->n_shards; k++)
+    shards[k] = FilmShard{k, f->n_shards, f->parts[shard_device(k, f->n_parts)].d_list + at[k], (int)out[2 * k], out[2 * k + 1]};
+  LrRenderParams q = f->params;
+  q.spp_count = spp_count;
+  return film_launch(f, q, shards, false, stats);
+}
+
+int film_render(Film* f, int32_t spp_count, LrStats* stats) {
+  if (!f) return fail(LR_ERR_INVALID, "null argument");
+  if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
+  if (!f->uniform()) {
+    const std::vector<int> at = shard_segments(f);
+    std::vector<unsigned long long> out;
+    if (int rc = film_list_tiles(f, true, 0.0f, 0, at, &out)) return rc;
+    if (int rc = film_launch_lists(f, spp_count, at, out, stats)) return rc;
+  } else {
+    LrRenderParams q = f->params;
+    q.spp_begin = f->params.spp_begin + f->tile_spp[0];
+    q.spp_count = spp_count;
+    std::vector<FilmShard> shards(f->n_shards);
+    for (int k = 0; k < f->n_shards; k++) shards[k] = FilmShard{k, f->n_shards};
+    if (int rc = film_launch(f, q, shards, !f->sharded, stats)) return rc;
+  }
+  for (int32_t& n : f->tile_spp) n += spp_count;
+  return LR_OK;
+}
+
+// Adaptive sampling: every shard selects its noisy tiles on its own device (select_tiles_kernel) and renders that list; the
+// host, which owns the counts, reads the lists back to advance the counts of the tiles they name.
+int film_render_adaptive(Film* f, int32_t spp_count, float threshold, int32_t max_spp, int32_t* active_tiles, LrStats* stats) {
+  if (!f) return fail(LR_ERR_INVALID, "null argument");
+  if (spp_count <= 0) return fail(LR_ERR_INVALID, "spp_count must be positive");
+  if (!(threshold >= 0.0f)) return fail(LR_ERR_INVALID, "threshold must be >= 0");
+  if (max_spp < 0) return fail(LR_ERR_INVALID, "max_spp must be >= 0");
+  if (!f->has_sumsq) return fail(LR_ERR_INVALID, "adaptive sampling needs a film made with sums of squares");
+  const std::vector<int> at = shard_segments(f);
+  std::vector<unsigned long long> out;
+  if (int rc = film_list_tiles(f, false, threshold, max_spp, at, &out)) return rc;
+  std::vector<std::vector<int2>> lists(f->n_shards);
+  int32_t active = 0;
+  {
+    int rc = LR_OK;
+    OnDevices on(rc);
+    cudaError_t e = cudaSuccess;
+    for (int k = 0; k < f->n_shards && e == cudaSuccess; k++) {
+      const Film::Part& part = f->parts[shard_device(k, f->n_parts)];
+      lists[k].resize(out[2 * k]);
+      active += (int32_t)out[2 * k];
+      if (lists[k].empty()) continue;
+      if ((rc = on.use(part.scene->device)) != LR_OK) return rc;
+      e = cudaMemcpyAsync(lists[k].data(), part.d_list + at[k], lists[k].size() * sizeof(int2), cudaMemcpyDeviceToHost, part.stream);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(part.stream);
+    }
+    if (e != cudaSuccess) return rc = fail(LR_ERR_CUDA, std::string("film tile list: ") + cudaGetErrorString(e));
+  }
+  if (active_tiles) *active_tiles = active;
+  if (active == 0) {
+    if (stats) std::memset(stats, 0, sizeof(*stats));
+    return LR_OK;
+  }
+  if (int rc = film_launch_lists(f, spp_count, at, out, stats)) return rc;
+  for (const std::vector<int2>& l : lists)
+    for (const int2& e : l) f->tile_spp[e.x] += spp_count;
+  return LR_OK;
+}
+
 // The crop gathered on part 0's device, each pixel from the part that owns it (read over NVLink where that device maps the
-// part's device, from a staged copy where it does not), to host memory: the sums divided by `divisor` if it is > 0, and
-// the sums of squares too if out_sumsq is not null.
-int film_download(const Film* f, float divisor, float* out, float* out_sumsq) {
+// part's device, from a staged copy where it does not), to host memory: the sums divided by their tile's count if `mean`,
+// and the sums of squares too if out_sumsq is not null.
+int film_download(const Film* f, bool mean, float* out, float* out_sumsq) {
   const Film::Part& p0 = f->parts[0];
   const size_t n = (size_t)f->crop_w * f->crop_h * 3;
   int rc = LR_OK;
   OnDevices on(rc);
   if ((rc = on.use(p0.scene->device)) != LR_OK) return rc;
+  std::vector<float> div(f->tile_spp.begin(), f->tile_spp.end());      // main.rs:104: `/ spp as f32`
   float* d_tmp = nullptr;
+  float* d_div = nullptr;
   cudaError_t e = dev_alloc((void**)&d_tmp, n * sizeof(float));
+  if (e == cudaSuccess && mean) e = dev_alloc((void**)&d_div, div.size() * sizeof(float));
+  if (e == cudaSuccess && mean) e = cudaMemcpyAsync(d_div, div.data(), div.size() * sizeof(float), cudaMemcpyHostToDevice, p0.stream);
   for (int sq = 0; sq < (out_sumsq ? 2 : 1) && e == cudaSuccess; sq++) {
     float* bufs[kMaxPeers];
     for (int i = 0; i < f->n_parts; i++) bufs[i] = sq ? f->parts[i].d_sumsq : f->parts[i].d_sum;
     PeerBuffers src;
     e = peer_buffers(f->ms, f->n_parts, bufs, n, p0.stream, &src);
-    if (e == cudaSuccess) e = launch_gather_shards(d_tmp, src, f->crop_w, f->crop_h, f->n_shards, sq ? 0.0f : divisor, p0.stream);
+    if (e == cudaSuccess) e = launch_gather_shards(d_tmp, src, f->crop_w, f->crop_h, f->n_shards, sq ? nullptr : d_div, p0.stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(sq ? out_sumsq : out, d_tmp, n * sizeof(float), cudaMemcpyDeviceToHost, p0.stream);
   }
   const cudaError_t done = cudaStreamSynchronize(p0.stream);   // before d_tmp goes back to the pool, on failure too
   if (e == cudaSuccess) e = done;
   dev_free(d_tmp);
+  dev_free(d_div);
   if (e != cudaSuccess) rc = fail(LR_ERR_CUDA, std::string("film read: ") + cudaGetErrorString(e));
   return rc;
 }
@@ -1123,8 +1292,8 @@ int film_download(const Film* f, float divisor, float* out, float* out_sumsq) {
 int film_read_mean(const Film* f, float* out_rgb, float* out_sumsq) {
   if (!f || !out_rgb) return fail(LR_ERR_INVALID, "null argument");
   if (out_sumsq && !f->has_sumsq) return fail(LR_ERR_INVALID, "the film was created without sums of squares");
-  if (f->spp_done <= 0) return fail(LR_ERR_INVALID, "the film holds no samples yet");
-  return film_download(f, (float)f->spp_done, out_rgb, out_sumsq);   // main.rs:104
+  if (f->spp_min() <= 0) return fail(LR_ERR_INVALID, "the film holds no samples yet");
+  return film_download(f, true, out_rgb, out_sumsq);
 }
 
 // The checkpoint: a film saves the same bytes for the same state through either handle, and each handle loads the other's.
@@ -1132,21 +1301,23 @@ int film_save(const Film* f, const char* path) {
   if (!f || !path) return fail(LR_ERR_INVALID, "null argument");
   const size_t n = (size_t)f->crop_w * f->crop_h * 3;
   std::vector<float> data(n * (f->has_sumsq ? 2 : 1));
-  if (int rc = film_download(f, 0.0f, data.data(), f->has_sumsq ? data.data() + n : nullptr)) return rc;
+  if (int rc = film_download(f, false, data.data(), f->has_sumsq ? data.data() + n : nullptr)) return rc;
+  const bool uniform = f->uniform();
   const LrScene* s0 = f->parts[0].scene;
   const LrRenderParams& p = f->params;
   FilmHeader h;
   std::memset(&h, 0, sizeof(h));
-  std::memcpy(h.magic, kFilmMagic, 8);
+  std::memcpy(h.magic, uniform ? kFilmMagic : kFilmMagicTiles, 8);
   h.film_w = s0->width; h.film_h = s0->height;
   h.crop_x = p.crop_w > 0 ? p.crop_x : 0; h.crop_y = p.crop_w > 0 ? p.crop_y : 0; h.crop_w = f->crop_w; h.crop_h = f->crop_h;
   h.integrator = p.integrator; h.depth = p.depth; h.depth_limit = p.depth_limit; h.no_direct_emitter = p.no_direct_emitter;
-  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = f->spp_done; h.has_sumsq = f->has_sumsq ? 1 : 0; h.seed = p.seed;
+  h.splits = p.splits; h.spp_begin = p.spp_begin; h.spp_done = f->spp_min(); h.has_sumsq = f->has_sumsq ? 1 : 0; h.seed = p.seed;
   // written next to the target and renamed: a crash mid-write never leaves a torn checkpoint under `path`
   const std::string tmp = std::string(path) + ".part";
   FILE* fp = std::fopen(tmp.c_str(), "wb");
   if (!fp) return fail(LR_ERR_IO, std::string("cannot write `") + tmp + "`");
-  const bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(data.data(), sizeof(float), data.size(), fp) == data.size();
+  bool ok = std::fwrite(&h, sizeof(h), 1, fp) == 1 && std::fwrite(data.data(), sizeof(float), data.size(), fp) == data.size();
+  if (ok && !uniform) ok = std::fwrite(f->tile_spp.data(), sizeof(int32_t), f->tile_spp.size(), fp) == f->tile_spp.size();
   const bool closed = std::fclose(fp) == 0;
   if (!ok || !closed || std::rename(tmp.c_str(), path) != 0) { std::remove(tmp.c_str()); return fail(LR_ERR_IO, std::string("cannot write `") + path + "`"); }
   return LR_OK;
@@ -1154,10 +1325,17 @@ int film_save(const Film* f, const char* path) {
 
 int film_info(const Film* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) {
   if (!f) return fail(LR_ERR_INVALID, "null argument");
-  if (spp_done) *spp_done = f->spp_done;
+  if (spp_done) *spp_done = f->spp_min();
   if (crop_w) *crop_w = f->crop_w;
   if (crop_h) *crop_h = f->crop_h;
   if (has_sumsq) *has_sumsq = f->has_sumsq ? 1 : 0;
+  return LR_OK;
+}
+
+int film_spp_map(const Film* f, int32_t* out) {
+  if (!f || !out) return fail(LR_ERR_INVALID, "null argument");
+  for (int y = 0; y < f->crop_h; y++)
+    for (int x = 0; x < f->crop_w; x++) out[(size_t)y * f->crop_w + x] = f->tile_spp[(size_t)(y >> 2) * f->tiles_x + (x >> 3)];
   return LR_OK;
 }
 }  // namespace
@@ -1166,7 +1344,11 @@ extern "C" {
 
 int lr_film_create(const LrScene* s, const LrRenderParams* p, int32_t want_sumsq, LrFilm** out) { LR_GUARDED(film_create(s, p, want_sumsq, out)); }
 int lr_film_render(LrFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(film_render(f, spp_count, stats)); }
+int lr_film_render_adaptive(LrFilm* f, int32_t spp_count, float threshold, int32_t max_spp, int32_t* active_tiles, LrStats* stats) {
+  LR_GUARDED(film_render_adaptive(f, spp_count, threshold, max_spp, active_tiles, stats));
+}
 int lr_film_info(const LrFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) { return film_info(f, spp_done, crop_w, crop_h, has_sumsq); }
+int lr_film_spp_map(const LrFilm* f, int32_t* out) { return film_spp_map(f, out); }
 int lr_film_read(const LrFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(film_read_mean(f, out_rgb, out_sumsq)); }
 int lr_film_save(const LrFilm* f, const char* path) { LR_GUARDED(film_save(f, path)); }
 int lr_film_load(const LrScene* s, const char* path, LrFilm** out) { LR_GUARDED(film_load(s, path, out)); }
@@ -1174,7 +1356,11 @@ void lr_film_destroy(LrFilm* f) { delete f; }
 
 int lr_multi_film_create(LrMultiScene* ms, const LrRenderParams* p, int32_t want_sumsq, LrMultiFilm** out) { LR_GUARDED(film_create(ms, p, want_sumsq, out)); }
 int lr_multi_film_render(LrMultiFilm* f, int32_t spp_count, LrStats* stats) { LR_GUARDED(film_render(f, spp_count, stats)); }
+int lr_multi_film_render_adaptive(LrMultiFilm* f, int32_t spp_count, float threshold, int32_t max_spp, int32_t* active_tiles, LrStats* stats) {
+  LR_GUARDED(film_render_adaptive(f, spp_count, threshold, max_spp, active_tiles, stats));
+}
 int lr_multi_film_info(const LrMultiFilm* f, int32_t* spp_done, int32_t* crop_w, int32_t* crop_h, int32_t* has_sumsq) { return film_info(f, spp_done, crop_w, crop_h, has_sumsq); }
+int lr_multi_film_spp_map(const LrMultiFilm* f, int32_t* out) { return film_spp_map(f, out); }
 int lr_multi_film_read(const LrMultiFilm* f, float* out_rgb, float* out_sumsq) { LR_GUARDED(film_read_mean(f, out_rgb, out_sumsq)); }
 int lr_multi_film_save(const LrMultiFilm* f, const char* path) { LR_GUARDED(film_save(f, path)); }
 int lr_multi_film_load(LrMultiScene* ms, const char* path, LrMultiFilm** out) { LR_GUARDED(film_load(ms, path, out)); }

@@ -12,9 +12,13 @@
 //   commented out)  --checkpoint FILE (with --progress: the film is saved after every chunk, and an existing FILE is
 //   resumed — bit for bit the image of an uninterrupted run)  --aov normal|depth (Scene::normal / Scene::depth,
 //   scene.rs:48-62, instead of the radiance; depth is written normalised to its maximum)
+//   --adaptive E (with --progress N: adaptive sampling.  Rounds of N samples go to the 8x4 tiles whose relative standard error
+//   is above E, until a round selects none; a tile holding the scene's spp or more gets no further round, so a tile ends
+//   with less than spp + N samples.  --checkpoint resumes it like any film)
 #include <sys/stat.h>
 
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -45,6 +49,7 @@ int main(int argc, char** argv) {
   const char* assets = nullptr;
   const char* checkpoint = nullptr;
   const char* aov = nullptr;
+  const char* adaptive = nullptr;
   int spp = -1, ow = 0, oh = 0, device = 0, gpus = 1, progress = 0;
   unsigned long long seed = 0;
   for (int i = 1; i < argc; i++) {
@@ -62,12 +67,22 @@ int main(int argc, char** argv) {
     else if (a == "--progress") progress = std::atoi(need("--progress"));
     else if (a == "--checkpoint") checkpoint = need("--checkpoint");
     else if (a == "--aov") aov = need("--aov");
+    else if (a == "--adaptive") adaptive = need("--adaptive");
     else if (!scene_path) scene_path = argv[i];
     else { std::fprintf(stderr, "error: unexpected argument `%s`\n", argv[i]); return 2; }
   }
   if (!scene_path) { std::fprintf(stderr, "Path for .toml must be specified.\n"); return 2; }   // main.rs:47-49
   if (aov && std::strcmp(aov, "normal") != 0 && std::strcmp(aov, "depth") != 0) { std::fprintf(stderr, "error: --aov normal|depth\n"); return 2; }
   if (checkpoint && progress <= 0) { std::fprintf(stderr, "error: --checkpoint needs --progress N\n"); return 2; }
+  float threshold = 0.0f;
+  if (adaptive) {
+    char* end = nullptr;
+    const double e = std::strtod(adaptive, &end);
+    if (end == adaptive || *end != 0 || !(e >= 0.0) || !std::isfinite(e)) { std::fprintf(stderr, "error: --adaptive takes a relative error >= 0\n"); return 2; }
+    if (progress <= 0) { std::fprintf(stderr, "error: --adaptive needs --progress N\n"); return 2; }
+    if (aov) { std::fprintf(stderr, "error: --adaptive renders the radiance, not an AOV\n"); return 2; }
+    threshold = (float)e;
+  }
   if (gpus > 8) { std::fprintf(stderr, "error: --gpus takes 1..8\n"); return 2; }
   if (aov && gpus > 1) { std::fprintf(stderr, "error: --aov renders on one GPU\n"); return 2; }
   std::printf("loading: %s\n", scene_path);
@@ -125,12 +140,30 @@ int main(int argc, char** argv) {
     struct stat sb;
     if (checkpoint && stat(checkpoint, &sb) == 0) {
       if (lr_multi_film_load(ms, checkpoint, &mfilm) != LR_OK) return die("resuming the checkpoint");
-    } else if (lr_multi_film_create(ms, &p, 0, &mfilm) != LR_OK) return die("creating the film");
+    } else if (lr_multi_film_create(ms, &p, adaptive ? 1 : 0, &mfilm) != LR_OK) return die("creating the film");
     int32_t done = 0;
     lr_multi_film_info(mfilm, &done, nullptr, nullptr, nullptr);
     if (done > 0) std::printf("resuming: %d of %d spp are in %s\n", done, cfg.samples, checkpoint);
     std::memset(&st, 0, sizeof(st));
-    while (done < cfg.samples) {
+    for (int round = 1; adaptive; round++) {
+      // adaptive: rounds of `progress` samples on the noisy tiles, until none is left; a tile holding the scene's spp gets no more
+      LrStats part;
+      int32_t active = 0;
+      if (lr_multi_film_render_adaptive(mfilm, progress, threshold, cfg.samples, &active, &part) != LR_OK) return die("rendering");
+      if (active == 0) break;
+      st.kernel_ms += part.kernel_ms; st.samples += part.samples; st.rays += part.rays; st.nonfinite_samples += part.nonfinite_samples;
+      if (checkpoint && lr_multi_film_save(mfilm, checkpoint) != LR_OK) return die("writing the checkpoint");
+      std::printf("adaptive round %d: %d tiles, %llu samples\n", round, active, (unsigned long long)part.samples);
+      std::fflush(stdout);
+    }
+    if (adaptive) {
+      std::vector<int32_t> spp_map((size_t)cfg.width * cfg.height);
+      lr_multi_film_spp_map(mfilm, spp_map.data());
+      double total = 0.0;
+      for (int32_t n : spp_map) total += n;
+      std::printf("adaptive: mean %.2f spp (threshold %g, at most %d)\n", total / spp_map.size(), threshold, cfg.samples);
+    }
+    while (!adaptive && done < cfg.samples) {
       const int n = cfg.samples - done < progress ? cfg.samples - done : progress;
       LrStats part;
       if (lr_multi_film_render(mfilm, n, &part) != LR_OK) return die("rendering");

@@ -56,6 +56,8 @@ struct DevParams {
   int unit_tiles;                        // how many tiles that is: shard_tile_count(tiles_x * tiles_y, ...), set once on the host
   int defer_iters, defer_thresh;         // path vertices per phase A; suspended lanes that end it early (persistent.cuh)
   int organisation;                      // BVH scenes only: 1 = one path per lane (persistent.cuh), otherwise the pool (pool.cuh)
+  const int2* tile_list;                 // null: the shard's tiles from spp_begin; else the j-th tile is {global tile, first
+                                         // sample index} = tile_list[j], j < unit_tiles (a film whose tiles hold different counts)
 };
 
 // Pixel sharding of a film over several devices (lr_multi_film_*): the crop's 8x4 tiles are dealt round-robin, shard k of
@@ -75,6 +77,22 @@ struct SampleRange { int begin, count; };
 __host__ __device__ inline SampleRange range_part(int begin, int count, int part, int n_parts) {
   const int per = count / n_parts, rem = count % n_parts;
   return {begin + part * per + (part < rem ? part : rem), per + (part < rem ? 1 : 0)};
+}
+// Adaptive sampling of a film (lr_film_render_adaptive): which 8x4 tiles get more samples.  A tile holding n samples of each
+// of its pixels, with per-pixel sums S and sums of squares Q, has the error max over its in-crop pixels and channels of
+//   sqrt(var / n) / max(m, kAdaptiveFloor),   m = S / n,   var = max(0, (Q - S m) / (n - 1))
+// (the relative standard error of the pixel mean), all in fp64 without contraction (kernels.cu is built with -fmad=false), so
+// a numpy float64 restatement decides the same.  The floor keeps black pixels from asking for samples forever.
+constexpr double kAdaptiveFloor = 1e-3;
+__host__ __device__ inline double adaptive_error(double s, double q, double n) {
+  const double m = s / n;
+  const double var = fmax(0.0, (q - s * m) / (n - 1.0));
+  return sqrt(var / n) / fmax(m, kAdaptiveFloor);
+}
+// Fewer than two samples say nothing about the noise; a tile with a non-finite sum is left alone once it has two (more samples
+// cannot make its sum finite again); max_spp > 0 caps the samples a tile gets.
+__host__ __device__ inline bool adaptive_selects(int n, bool finite, double error, float threshold, int max_spp) {
+  return (n < 2 || (finite && error > (double)threshold)) && (max_spp == 0 || n < max_spp);
 }
 // work items of one render launch: one per (split, pixel slot of the shard's tiles)
 __host__ __device__ inline unsigned int render_units(const DevParams& p) { return (unsigned int)p.unit_tiles * 32u * (unsigned int)p.splits; }

@@ -38,16 +38,91 @@ __global__ void reduce_peers_kernel(float* __restrict__ dst, PeerBuffers src, si
 
 // The image of a pixel-sharded film (lr_multi_film_*), on the first device: every device's buffer spans the whole crop but
 // holds only the pixels of its own shards (stale values or zeros elsewhere), so each pixel is taken from the device that
-// owns its tile, never summed across devices.  Divided by the sample count with the expression of scale_kernel, so the
-// bits equal lr_film_read's; divisor <= 0: the raw sums (sums of squares, checkpoints).
-__global__ void gather_shards_kernel(float* __restrict__ dst, const __grid_constant__ PeerBuffers src, int crop_w, int crop_h, int n_shards, float divisor) {
+// owns its tile, never summed across devices.  Divided by its tile's sample count (tile_div, one float per tile) with the
+// expression of scale_kernel, so the bits of a film whose tiles hold the same count equal lr_render's; tile_div null: the
+// raw sums (sums of squares, checkpoints).
+__global__ void gather_shards_kernel(float* __restrict__ dst, const __grid_constant__ PeerBuffers src, int crop_w, int crop_h, int n_shards,
+                                     const float* __restrict__ tile_div) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (size_t)crop_w * crop_h * 3) return;
   const int px = (int)(i / 3), lx = px % crop_w, ly = px / crop_w;
   const int tiles_x = (crop_w + 7) / 8;
-  const int shard = shard_of_tile((ly >> 2) * tiles_x + (lx >> 3), n_shards);
-  const float v = src.p[shard_device(shard, src.count)][i];
-  dst[i] = divisor > 0.0f ? v / divisor : v;
+  const int tile = (ly >> 2) * tiles_x + (lx >> 3);
+  const float v = src.p[shard_device(shard_of_tile(tile, n_shards), src.count)][i];
+  dst[i] = tile_div ? v / tile_div[tile] : v;
+}
+
+// Adaptive sampling, step 1: does the j-th tile of the shard get samples in this call (adaptive_selects, device_scene.h)?  One
+// warp per tile, one lane per pixel.  counts[t] = the samples every pixel of global tile t holds.
+__global__ void select_tiles_kernel(const float* __restrict__ sum, const float* __restrict__ sumsq, const int* __restrict__ counts,
+                                    int crop_w, int crop_h, int shard, int n_shards, int unit_tiles, float threshold, int max_spp,
+                                    unsigned char* __restrict__ selected) {
+  const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int j = (int)(gid >> 5), lane = (int)(gid & 31);
+  if (j >= unit_tiles) return;                          // warp-uniform
+  const int tiles_x = (crop_w + 7) / 8;
+  const int tile = shard_tile(j, shard, n_shards), n = counts[tile];
+  const int lx = (tile % tiles_x) * 8 + (lane & 7), ly = (tile / tiles_x) * 4 + (lane >> 3);
+  bool finite = true;
+  double err = 0.0;
+  if (lx < crop_w && ly < crop_h) {
+    const size_t i = 3 * ((size_t)ly * crop_w + lx);
+    for (int c = 0; c < 3; c++) {
+      const float s = sum[i + c], q = sumsq[i + c];
+      finite = finite && isfinite(s) && isfinite(q);
+      if (n >= 2) err = fmax(err, adaptive_error((double)s, (double)q, (double)n));
+    }
+  }
+  finite = __all_sync(0xffffffffu, finite);
+  for (int off = 16; off > 0; off >>= 1) err = fmax(err, __shfl_xor_sync(0xffffffffu, err, off));
+  if (lane == 0) selected[j] = adaptive_selects(n, finite, err, threshold, max_spp) ? 1 : 0;
+}
+
+// Adaptive sampling, step 2: the selected tiles of the shard as a list in ascending tile order, {global tile, spp_begin +
+// counts[tile]} (what decode_unit reads), by ballot and scan in one block, so the launch order does not depend on timing.
+// out[0] = tiles listed, out[1] = their pixels inside the crop.
+__global__ void __launch_bounds__(1024) compact_tiles_kernel(const unsigned char* __restrict__ selected, const int* __restrict__ counts,
+                                                             int crop_w, int crop_h, int shard, int n_shards, int unit_tiles, int spp_begin,
+                                                             int2* __restrict__ list, unsigned long long* __restrict__ out) {
+  __shared__ int warp_base[32];
+  __shared__ int total;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int tiles_x = (crop_w + 7) / 8;
+  if (threadIdx.x == 0) total = 0;
+  unsigned long long pixels = 0;
+  __syncthreads();
+  for (int j0 = 0; j0 < unit_tiles; j0 += 1024) {
+    const int j = j0 + (int)threadIdx.x;
+    const bool take = j < unit_tiles && selected[j];
+    const unsigned m = __ballot_sync(0xffffffffu, take);
+    if (lane == 0) warp_base[warp] = __popc(m);
+    __syncthreads();
+    if (warp == 0) {                                     // exclusive scan of the 32 warp counts
+      const int c = warp_base[lane];
+      int incl = c;
+      for (int off = 1; off < 32; off <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, off); if (lane >= off) incl += v; }
+      warp_base[lane] = total + incl - c;
+    }
+    __syncthreads();
+    if (take) {
+      const int tile = shard_tile(j, shard, n_shards), tx = tile % tiles_x, ty = tile / tiles_x;
+      list[warp_base[warp] + __popc(m & ((1u << lane) - 1u))] = make_int2(tile, spp_begin + counts[tile]);
+      pixels += (unsigned long long)(min(8, crop_w - 8 * tx) * min(4, crop_h - 4 * ty));
+    }
+    __syncthreads();
+    if (threadIdx.x == 1023) total = warp_base[31] + __popc(m);
+    __syncthreads();
+  }
+  __shared__ unsigned long long warp_pixels[32];
+  pixels = __reduce_add_sync(0xffffffffu, (unsigned int)pixels);   // < 2^32: 32 pixels a tile, < 2^26 tiles a crop
+  if (lane == 0) warp_pixels[warp] = pixels;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned long long all = 0;
+    for (int w = 0; w < 32; w++) all += warp_pixels[w];
+    out[0] = (unsigned long long)total;
+    out[1] = all;
+  }
 }
 
 // parity probe: nearest hit of the primary ray of every film pixel with fixed random numbers
@@ -196,9 +271,24 @@ cudaError_t launch_reduce_peers(float* dst, const PeerBuffers& src, size_t n, fl
   return cudaGetLastError();
 }
 
-cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, float divisor, cudaStream_t stream) {
+cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, const float* tile_div, cudaStream_t stream) {
   const size_t n = (size_t)crop_w * crop_h * 3;
-  gather_shards_kernel<<<(unsigned int)((n + 255) / 256), 256, 0, stream>>>(dst, src, crop_w, crop_h, n_shards, divisor);
+  gather_shards_kernel<<<(unsigned int)((n + 255) / 256), 256, 0, stream>>>(dst, src, crop_w, crop_h, n_shards, tile_div);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_select_tiles(const float* sum, const float* sumsq, const int* counts, int crop_w, int crop_h, int shard, int n_shards,
+                                int unit_tiles, float threshold, int max_spp, int spp_begin, unsigned char* selected, int2* list,
+                                bool every_tile, unsigned long long* out, cudaStream_t stream) {
+  if (every_tile) {
+    const cudaError_t e = cudaMemsetAsync(selected, 1, (size_t)unit_tiles, stream);
+    if (e != cudaSuccess) return e;
+  } else if (unit_tiles > 0) {
+    const long long threads = (long long)unit_tiles * 32;
+    select_tiles_kernel<<<(unsigned int)((threads + 255) / 256), 256, 0, stream>>>(sum, sumsq, counts, crop_w, crop_h, shard, n_shards, unit_tiles,
+                                                                                 threshold, max_spp, selected);
+  }
+  compact_tiles_kernel<<<1, 1024, 0, stream>>>(selected, counts, crop_w, crop_h, shard, n_shards, unit_tiles, spp_begin, list, out);
   return cudaGetLastError();
 }
 

@@ -21,8 +21,16 @@ cudaError_t launch_scale(float* dst, size_t n, float divisor, cudaStream_t strea
 constexpr int kMaxPeers = 8;
 struct PeerBuffers { const float* p[kMaxPeers]; int count; };
 cudaError_t launch_reduce_peers(float* dst, const PeerBuffers& src, size_t n, float divisor, cudaStream_t stream);
-// lr_multi_film: each pixel from the buffer of the device that owns its tile (shard_of_tile / shard_device), / divisor if > 0
-cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, float divisor, cudaStream_t stream);
+// a film: each pixel from the buffer of the device that owns its tile (shard_of_tile / shard_device), / tile_div[its tile]
+// if tile_div is not null
+cudaError_t launch_gather_shards(float* dst, const PeerBuffers& src, int crop_w, int crop_h, int n_shards, const float* tile_div, cudaStream_t stream);
+// the tile list of a film's shard: the tiles that adaptive_selects (device_scene.h) picks, or every tile of the shard if
+// every_tile, as {global tile, spp_begin + counts[tile]} in ascending tile order into list[0, out[0]); out[1] = their pixels
+// inside the crop.  selected: unit_tiles bytes of scratch.  sum / sumsq / counts are the film's buffers on the device the
+// stream belongs to (sum / sumsq are not read if every_tile).
+cudaError_t launch_select_tiles(const float* sum, const float* sumsq, const int* counts, int crop_w, int crop_h, int shard, int n_shards,
+                                int unit_tiles, float threshold, int max_spp, int spp_begin, unsigned char* selected, int2* list,
+                                bool every_tile, unsigned long long* out, cudaStream_t stream);
 cudaError_t launch_primary(const DevScene& sc, float u, float v, float ua, float va, int* prim, float* t, cudaStream_t stream);
 cudaError_t launch_aov(const DevScene& sc, const DevParams& p, int kind, float* out, cudaStream_t stream);
 cudaError_t launch_rays(const DevScene& sc, long long n, const float* org, const float* dir, int* prim, float* t, float* nout,

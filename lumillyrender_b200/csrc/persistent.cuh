@@ -60,12 +60,20 @@ LR_DEV void flush_counters(unsigned long long* counters, int lane, unsigned int&
   }
 }
 
-// unit -> (split, crop-relative pixel): the shard's 8x4 pixel tiles lane by lane, so a warp starts on one tile
-LR_DEV bool decode_unit(const DevParams& p, unsigned int u, int& lx, int& ly, int& split) {
+// unit -> (split, crop-relative pixel, first sample index): the shard's 8x4 pixel tiles (or those of p.tile_list) lane by
+// lane, so a warp starts on one tile
+LR_DEV bool decode_unit(const DevParams& p, unsigned int u, int& lx, int& ly, int& split, int& begin) {
   const unsigned int per_split = (unsigned int)p.unit_tiles * 32u;
   split = (int)(u / per_split);
   const unsigned int r = u % per_split;
-  const unsigned int tile = (unsigned int)shard_tile((int)(r >> 5), p.shard, p.n_shards), lane = r & 31u;
+  unsigned int tile = (unsigned int)shard_tile((int)(r >> 5), p.shard, p.n_shards);
+  begin = p.spp_begin;
+  if (p.tile_list) {
+    const int2 e = __ldg(p.tile_list + (r >> 5));
+    tile = (unsigned int)e.x;
+    begin = e.y;
+  }
+  const unsigned int lane = r & 31u;
   lx = (int)(tile % p.tiles_x) * 8 + (int)(lane & 7u);
   ly = (int)(tile / p.tiles_x) * 4 + (int)(lane >> 3);
   return lx < p.crop_w && ly < p.crop_h;

@@ -259,7 +259,8 @@ class _FilmBase:
 
     def __init__(self, owner, params=None, sumsq=False, path=None):
         self._lib = capi.load_library()
-        self._fn = {n: getattr(self._lib, "%s_%s" % (self._API, n)) for n in ("create", "load", "render", "info", "read", "save", "destroy")}
+        self._fn = {n: getattr(self._lib, "%s_%s" % (self._API, n))
+                    for n in ("create", "load", "render", "render_adaptive", "info", "spp_map", "read", "save", "destroy")}
         self._f = C.c_void_p()
         if path is not None:
             check(self._fn["load"](owner, str(path).encode(), C.byref(self._f)))
@@ -281,6 +282,23 @@ class _FilmBase:
         st = LrStats()
         check(self._fn["render"](self._f, int(spp), C.byref(st)))
         return st.as_dict()
+
+    def render_adaptive(self, spp, threshold, max_spp=0):
+        """Adds `spp` samples to every 8x4 tile whose relative standard error exceeds `threshold`, each tile from its own
+        count; tiles holding `max_spp` samples (if > 0) are left alone.  Needs a film made with sumsq=True.  Returns the
+        stats dict plus `active_tiles`, the tiles rendered (0: the film has converged)."""
+        st = LrStats()
+        active = C.c_int32()
+        check(self._fn["render_adaptive"](self._f, int(spp), float(threshold), int(max_spp), C.byref(active), C.byref(st)))
+        d = st.as_dict()
+        d["active_tiles"] = active.value
+        return d
+
+    def spp_map(self):
+        """The samples every pixel of the crop holds, (h, w) int32."""
+        out = np.empty(self._shape[:2], dtype=np.int32)
+        check(self._fn["spp_map"](self._f, _iptr(out)))
+        return out
 
     def read(self, sumsq=False):
         img = np.empty(self._shape, dtype=np.float32)
